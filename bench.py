@@ -40,6 +40,7 @@ import torch  # noqa: E402
 
 UNIT = "edges/s"
 L2_BYTES = 126 * 1024 * 1024
+DUMP_BYTES = 64 * 1000 * 1000
 METRICS = {
     "pose": "GripNet fwd+bwd edges/sec per epoch (pose-0 shape)",
     "pose2": "GripNet fwd+bwd edges/sec per epoch (pose-2 shape, R=1097)",
@@ -245,6 +246,27 @@ def timed_steps(step, n, flush):
     return [a.elapsed_time(b) for a, b in evs]
 
 
+def dump_outputs(out_dir, named):
+    """Write each (name, tensor) of `named` to out_dir/<name>.npy as float32, DUMP_BYTES in all at most.  The
+    budget is shared out smallest array first; an array larger than its share is replaced by a sample of its
+    rows: a sorted choice without replacement from numpy's default_rng(0) that depends on the row count only,
+    so two builds of the project dump the same rows."""
+    os.makedirs(out_dir, exist_ok=True)
+    named = sorted(named, key=lambda kv: kv[1].numel())
+    left = DUMP_BYTES
+    for i, (name, t) in enumerate(named):
+        share = left // (len(named) - i)
+        t = t.detach()
+        if t.dim() > 0 and t.numel() * 4 + 256 > share:
+            row_bytes = 4 * (t.numel() // max(t.size(0), 1))
+            k = max(0, (share - 256) // row_bytes)
+            rows = np.sort(np.random.default_rng(0).choice(t.size(0), size=k, replace=False))
+            t = t[torch.from_numpy(rows).to(t.device)]
+        path = os.path.join(out_dir, name + ".npy")
+        np.save(path, t.float().cpu().numpy())
+        left -= os.path.getsize(path)
+
+
 def e2e_pipelined(io, step, n_steps, flush):
     """End-to-end steps with the PCIe copies double-buffered: the host->device copy of step i+1's inputs (copy
     stream 1, pinned host -> device staging slot) and the device->host read of step i-1's results (copy stream 2,
@@ -387,6 +409,7 @@ def build_pose(args, world, rank, dev, dctx, workload="pose"):
         return probes
 
     return dict(model=model, data=data, graph=g, fwd=fwd, dynamic=[neg_static], edges=e_epoch, io=io,
+                output_names=("loss", "z", "pos_score", "neg_score"),
                 host_loss=host_loss, loss_of=loss_of, h2d_bytes=int(neg_static.numel() * 8),
                 d2h_bytes=int(4 + 2 * e_loc * 4), kernels=kernels,
                 row_partitioned=("gg.embedding", "gd.target_feat") if dctx is not None else (),
@@ -434,6 +457,7 @@ def build_nc(args, world, rank, dev, dctx, workload):
                  lambda: ops.spmm(pp.fwd, ops.M(x), ops.M(out), F, bias=bias, relu=True))]
 
     return dict(model=model, data=data, graph=g, fwd=fwd, dynamic=[], edges=e_epoch, io=io, host_loss=host_loss,
+                output_names=("loss", "z", "score"),
                 loss_of=lambda outs: outs[0].detach().view(1), h2d_bytes=int(n_lab * 8),
                 d2h_bytes=int(4 + n_lab * n_class * 4), kernels=kernels, row_partitioned=(),
                 e2e_note="labels from pinned host memory each step; loss and class scores read back")
@@ -485,6 +509,7 @@ def build_chain(args, world, rank, dev, dctx, workload="scaled"):
                  lambda: ops.spmm(aa.fwd, ops.M(x), ops.M(out), F, bias=bias, relu=True))]
 
     return dict(model=model, data=data, graph=None, fwd=fwd, dynamic=[], edges=e_epoch, io=io, host_loss=host_loss,
+                output_names=("loss", "z", "score"),
                 loss_of=loss_of, h2d_bytes=int(n_lab * 8), d2h_bytes=int(4 + n_lab * n_class * 4), kernels=kernels,
                 row_partitioned=("aa.embedding", "ab.target_feat", "bc.target_feat") if dctx is not None else (),
                 e2e_note="labels from pinned host memory each step; loss and class scores read back")
@@ -567,8 +592,9 @@ def kernel_rooflines(w, step_ms, workload, flush, peaks, peak_src):
     return top, rows
 
 
-def time_workload(args, workload, world, rank, dev, dctx, steps, flush, with_e2e=True):
-    """Build, capture and time one workload.  Returns (record, w, step)."""
+def time_workload(args, workload, world, rank, dev, dctx, steps, flush, with_e2e=True, dump_dir=None):
+    """Build, capture and time one workload; with `dump_dir`, rank 0 writes what the last timed step computed
+    (the model's outputs and every parameter gradient) there.  Returns (record, w, step)."""
     import torch.distributed as dist
     import gripnet_b200 as gb  # noqa: F401
     w = build_workload(args, workload, world, rank, dev, dctx)
@@ -589,6 +615,10 @@ def time_workload(args, workload, world, rank, dev, dctx, steps, flush, with_e2e
         t_wall = time.perf_counter() - t_wall0
     dev_ms = sum(times)
     loss_dev = float(w["loss_of"](step.outputs).cpu()[0])
+    if dump_dir is not None and rank == 0:
+        outs = [w["loss_of"](step.outputs)] + list(step.outputs[1:])
+        grads = [("grad." + k, p.grad) for k, p in w["model"].named_parameters() if p.grad is not None]
+        dump_outputs(dump_dir, list(zip(w["output_names"], outs)) + grads)
 
     io = w["io"]
     e2e_mode, e2e_ms = "pipelined", None
@@ -775,7 +805,8 @@ def run_cuda(args):
     flush = torch.empty(2 * L2_BYTES, dtype=torch.uint8, device=dev)
     peaks, peak_src = measured_peaks()
 
-    rec, w, step = time_workload(args, workload, world, rank, dev, dctx, args.steps, flush)
+    rec, w, step = time_workload(args, workload, world, rank, dev, dctx, args.steps, flush,
+                                 dump_dir=args.dump_outputs)
     model, e_epoch = w["model"], w["edges"]
     dev_ms, e2e_ms = rec["dev_ms"], rec["e2e_ms"]
     value = e_epoch * args.steps / (dev_ms * 1e-3)
@@ -912,7 +943,13 @@ def main():
     ap.add_argument("--check-config5", action="store_true",
                     help="also replay config 5 on rank 0 alone and compare the loss (tens of seconds, ~40 GB)")
     ap.add_argument("--eager", action="store_true", help="do not capture the step into a CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (loss, embeddings, scores and every "
+                         "parameter gradient; rank 0's in a multi-GPU run) as DIR/<name>.npy in float32, 64 MB in all "
+                         "at most; an array over its share holds a fixed seeded sample of its rows")
     args = ap.parse_args()
+    if args.impl == "reference" and args.dump_outputs is not None:
+        ap.error("--dump-outputs applies to the CUDA arm (--impl cuda) only")
     if args.impl == "reference":
         return run_reference(args)
     return run_cuda(args)

@@ -265,6 +265,7 @@ def variants():
 if __name__ == "__main__":
     torch.set_num_threads(1)          # sequential index_add order -> reproducible fixtures
     torch.manual_seed(20261017)       # default initialisers of the reference modules draw from the global RNG
+    # tests/test_init_distributions.py replays every module construction below, in this order, with this seed
     norm_cases()
     g = synth.pose_small()
     pose_case("pose_small", g, synth.pose_params(g))
