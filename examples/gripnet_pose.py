@@ -3,6 +3,7 @@
 
     python examples/gripnet_pose.py EPOCHS datasets/pose/pose-0.pt [--out out/pose-0]
     python examples/gripnet_pose.py EPOCHS --synthetic            # pose-0-shaped synthetic supergraph
+    python examples/gripnet_pose.py EPOCHS --synthetic --rank     # + filtered test MRR / Hits@10 every epoch
 
 Same model (``GripNet-pose.py:86-99``), optimiser (Adam, lr 0.01, ``:104``), per-epoch negative sampling
 (``:131``), loss (``:140-142``) and per-relation AUPRC / AUROC / AP@all records (``:148-164``, ``:174-199``) —
@@ -26,9 +27,12 @@ def main():
     ap.add_argument("--out", default="out/pose")
     ap.add_argument("--lr", type=float, default=0.01)
     ap.add_argument("--seed", type=int, default=1111)
+    ap.add_argument("--rank", action="store_true",
+                    help="also print the filtered test MRR and Hits@10 (all drugs as candidate tails, train + test "
+                         "positives filtered), macro-averaged over relations")
     args = ap.parse_args()
 
-    from gripnet_b200 import data as gd, metrics, utils
+    from gripnet_b200 import data as gd, metrics, ranking, utils
     from gripnet_b200.pipelines import PoseModel, to_device
     from gripnet_b200.training import PoseTrainer
     dev = torch.device("cuda:0")
@@ -51,6 +55,12 @@ def main():
     train_rec = torch.empty(args.epochs, 3, n_rel, dtype=torch.float64, device=dev)
     test_rec = torch.empty(args.epochs, 3, n_rel, dtype=torch.float64, device=dev)
     losses = torch.empty(args.epochs, device=dev)
+    ranker = None
+    if args.rank:                                           # built once; one filtered ranking pass per epoch
+        pos = [(train["dd_edge_index"], train["dd_edge_type"]), (test["dd_edge_index"], test["dd_edge_type"])]
+        filt = ranking.EdgeFilter(pos, test["n_d"], n_rel)
+        ranker = ranking.LinkRanker(test["dd_edge_index"], test["dd_edge_type"], test["n_d"], n_rel, filter=filt)
+        rank_rec = torch.empty(args.epochs, 2, n_rel, dtype=torch.float64, device=dev)
     for epoch in range(args.epochs):
         t0 = time.time()
         losses[epoch] = trainer.train_epoch().detach()
@@ -60,12 +70,20 @@ def main():
             pos = model.dmt(z, test["dd_edge_index"], test["dd_edge_type"])
             neg = model.dmt(z, test_neg, test["dd_edge_type"])
             metrics.lp_metrics(pos, neg, test["dd_range_list"], out=test_rec[epoch])
+            if ranker is not None:
+                ranker.metrics(z, model.dmt.weight, hits=(10,), out=rank_rec[epoch])
         tr, te = train_rec[epoch].nanmean(dim=1).tolist(), test_rec[epoch].nanmean(dim=1).tolist()   # one sync per epoch
-        print("{:3d}   loss:{:0.4f}   train auprc:{:0.4f} auroc:{:0.4f} ap:{:0.4f}   test auprc:{:0.4f} auroc:{:0.4f} "
-              "ap:{:0.4f}   time:{:0.3f}".format(epoch, float(losses[epoch].detach()), *tr, *te, time.time() - t0))
+        line = "{:3d}   loss:{:0.4f}   train auprc:{:0.4f} auroc:{:0.4f} ap:{:0.4f}   test auprc:{:0.4f} auroc:{:0.4f} " \
+               "ap:{:0.4f}".format(epoch, float(losses[epoch].detach()), *tr, *te)
+        if ranker is not None:
+            line += "   test mrr:{:0.4f} hits@10:{:0.4f}".format(*rank_rec[epoch].nanmean(dim=1).tolist())
+        print(line + "   time:{:0.3f}".format(time.time() - t0))
     os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
     torch.save({k: v.cpu() for k, v in model.state_dict().items()}, args.out + "-model.pt")
-    torch.save({"train_record": train_rec.cpu(), "test_record": test_rec.cpu(), "loss": losses.cpu()}, args.out + "-record.pt")
+    rec = {"train_record": train_rec.cpu(), "test_record": test_rec.cpu(), "loss": losses.cpu()}
+    if ranker is not None:
+        rec["test_rank_record"] = rank_rec.cpu()             # [epochs, 2 (mrr, hits@10), R]
+    torch.save(rec, args.out + "-record.pt")
 
 
 if __name__ == "__main__":

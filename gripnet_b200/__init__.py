@@ -25,10 +25,11 @@ def _require_library():
 
 _require_library()          # fail loudly at import if libgripnet_b200.so is missing
 
-from . import graph, ops, parallel, layers, decoder, encoder, losses, utils, metrics, optim  # noqa: E402,F401
+from . import graph, ops, parallel, layers, decoder, encoder, losses, utils, metrics, optim, ranking  # noqa: E402,F401
 from .layers import myGCN, myRGCN, homoGraph, interGraph  # noqa: E402,F401
 from .decoder import multiRelaInnerProductDecoder, multiClassInnerProductDecoder  # noqa: E402,F401
 from .losses import link_prediction_loss, node_classification_loss  # noqa: E402,F401
+from .ranking import EdgeFilter, LinkRanker  # noqa: E402,F401
 
 
 def install_as_gripnet():

@@ -1,0 +1,403 @@
+// K16: filtered candidate ranking (OGB rank rule, per-relation MRR / Hits@k) and top-k link prediction of the
+// DistMult decoder.  Every candidate tail c of a query (s, r) is scored as one row of S = Q . z^T with
+// Q[g] = z[s_g] .* w[r_g]; the product itself is the existing dense GEMM (gn_sgemm / gn_tc_gemm).  This file holds
+// what sits around it: the (src, rel)-grouped edge structure, the query rows, the filtered rank count, the
+// per-relation reduction and the per-query top-k selection.
+#include "sortkit.cuh"
+
+namespace gn {
+
+constexpr int kRankMaxHits = 8;
+constexpr int kTopkThreads = 256;
+constexpr int kTopkMax = 256;                  // largest k: one selected key per thread of the sort
+constexpr uint32_t kMaskedBits = 0xffffffffu;  // NaN payload no arithmetic produces: "filtered" in a top-k row
+
+// ---------------------------------------------------------------------------------------------------------------
+// grouped edge structure: rows s*R + r, entries (dst, edge id) sorted by dst inside a row (two stable counting
+// sorts: by dst, then by row), and the compacted list of non-empty rows
+// ---------------------------------------------------------------------------------------------------------------
+__global__ void rank_dst_keys_kernel(const int64_t* __restrict__ dst, int64_t n, int32_t* __restrict__ key) {
+  const int64_t e = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (e < n) key[e] = int32_t(dst[e]);
+}
+
+__global__ void rank_row_keys_kernel(const int64_t* __restrict__ src, const int64_t* __restrict__ etype,
+                                     const int32_t* __restrict__ perm, int64_t n, int32_t n_rel,
+                                     int32_t* __restrict__ key) {
+  const int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const int32_t e = perm[i];
+  key[i] = int32_t(src[e]) * n_rel + int32_t(etype[e]);
+}
+
+__global__ void rank_fill_kernel(const int64_t* __restrict__ dst, const int32_t* __restrict__ eid, int64_t n,
+                                 int32_t* __restrict__ ent_dst) {
+  const int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (i < n) ent_dst[i] = int32_t(dst[eid[i]]);
+}
+
+__global__ void rank_row_flags_kernel(const int32_t* __restrict__ rowptr, int32_t n_rows, int32_t* __restrict__ flag) {
+  const int r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r < n_rows) flag[r] = rowptr[r + 1] > rowptr[r] ? 1 : 0;
+}
+
+__global__ void rank_groups_kernel(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ pos, int32_t n_rows,
+                                   int32_t* __restrict__ group_row) {
+  const int r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r < n_rows && rowptr[r + 1] > rowptr[r]) group_row[pos[r]] = r;
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// query rows Q[i, :] = z[s_i, :] .* w[r_i, :]; (s, r) from a group row id s*R + r or from two index lists
+// ---------------------------------------------------------------------------------------------------------------
+__global__ void rank_query_rows_kernel(const float* __restrict__ z, int64_t ldz, int D, const float* __restrict__ w,
+                                       int32_t n_rel, const int32_t* __restrict__ group_row,
+                                       const int64_t* __restrict__ node, const int64_t* __restrict__ rel,
+                                       int64_t count, float* __restrict__ q, int64_t ldq) {
+  const int64_t t = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (t >= count * D) return;
+  const int64_t i = t / D;
+  const int f = int(t - i * D);
+  int64_t s, r;
+  if (group_row != nullptr) {
+    const int32_t g = group_row[i];
+    s = g / n_rel;
+    r = g - s * n_rel;
+  } else {
+    s = node[i];
+    r = rel[i];
+  }
+  q[i * ldq + f] = z[s * ldz + f] * w[r * D + f];
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// filtered rank: one warp per group (a row of S), the group's targets in turn.  opt / pess count the candidates
+// c != t above / at-or-above S(t) over the whole row, then the distinct filtered candidates other than t that met
+// the same comparisons are taken back out.  S(t) is read from the same row as every S(c).
+// ---------------------------------------------------------------------------------------------------------------
+constexpr int kCountWarps = 8;
+
+__global__ void __launch_bounds__(kCountWarps * 32) rank_count_kernel(
+    const float* __restrict__ S, int64_t lds, int32_t n, const int32_t* __restrict__ group_row, int32_t n_groups,
+    const int32_t* __restrict__ q_rowptr, const int32_t* __restrict__ q_dst, const int32_t* __restrict__ q_eid,
+    const int32_t* __restrict__ f_rowptr, const int32_t* __restrict__ f_dst, float* __restrict__ rank) {
+  const int lane = threadIdx.x & 31;
+  const int g = blockIdx.x * kCountWarps + (threadIdx.x >> 5);
+  if (g >= n_groups) return;
+  const int32_t row = group_row[g];
+  const float* srow = S + int64_t(g) * lds;
+  const int f0 = f_rowptr ? f_rowptr[row] : 0, f1 = f_rowptr ? f_rowptr[row + 1] : 0;
+  for (int j = q_rowptr[row]; j < q_rowptr[row + 1]; ++j) {
+    const int t = q_dst[j];
+    const float st = srow[t];
+    int opt = 0, pess = 0;
+    for (int c = lane; c < n; c += 32) {
+      const float v = srow[c];
+      opt += (c != t) & (v > st);
+      pess += (c != t) & (v >= st);
+    }
+    for (int k = f0 + lane; k < f1; k += 32) {
+      const int c = f_dst[k];
+      if (c == t || (k > f0 && f_dst[k - 1] == c)) continue;   // the target itself; duplicates count once
+      const float v = srow[c];
+      opt -= v > st;
+      pess -= v >= st;
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      opt += __shfl_xor_sync(kFull, opt, o);
+      pess += __shfl_xor_sync(kFull, pess, o);
+    }
+    if (lane == 0) rank[q_eid[j]] = 1.0f + 0.5f * float(opt + pess);
+  }
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// per-relation MRR / Hits@k: one block per relation, a fixed entry -> thread assignment and a fixed tree (float64)
+// ---------------------------------------------------------------------------------------------------------------
+struct HitsK {
+  int32_t k[kRankMaxHits];
+};
+
+constexpr int kMetricThreads = 256;
+
+__global__ void __launch_bounds__(kMetricThreads) rank_metrics_kernel(const float* __restrict__ rank,
+                                                                      const int32_t* __restrict__ rel_rowptr,
+                                                                      const int32_t* __restrict__ rel_perm,
+                                                                      int32_t n_rel, HitsK hk, int n_hits,
+                                                                      double* __restrict__ out) {
+  __shared__ double red[kMetricThreads];
+  __shared__ int hred[kRankMaxHits][kMetricThreads];
+  const int r = blockIdx.x;
+  const int b = rel_rowptr[r], e = rel_rowptr[r + 1];
+  double s = 0.0;
+  int h[kRankMaxHits];
+#pragma unroll
+  for (int i = 0; i < kRankMaxHits; ++i) h[i] = 0;
+  for (int i = b + threadIdx.x; i < e; i += kMetricThreads) {
+    const float rk = rank[rel_perm[i]];
+    s += 1.0 / double(rk);
+#pragma unroll
+    for (int m = 0; m < kRankMaxHits; ++m) h[m] += (m < n_hits && rk <= float(hk.k[m])) ? 1 : 0;
+  }
+  red[threadIdx.x] = s;
+#pragma unroll
+  for (int m = 0; m < kRankMaxHits; ++m) hred[m][threadIdx.x] = h[m];
+  __syncthreads();
+  for (int w = kMetricThreads / 2; w > 0; w >>= 1) {
+    if (threadIdx.x < w) {
+      red[threadIdx.x] += red[threadIdx.x + w];
+#pragma unroll
+      for (int m = 0; m < kRankMaxHits; ++m) hred[m][threadIdx.x] += hred[m][threadIdx.x + w];
+    }
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) {
+    const int cnt = e - b;
+    const double nan = __longlong_as_double(0x7ff8000000000000ll);
+    out[r] = cnt ? red[0] / double(cnt) : nan;
+    for (int m = 0; m < n_hits; ++m) out[int64_t(1 + m) * n_rel + r] = cnt ? double(hred[m][0]) / double(cnt) : nan;
+  }
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// top-k: one block per query row.  A candidate's key is (order-preserving bits of its score) << 32 | ~id, so keys
+// are distinct, a larger key is a higher score and, among equal scores, a smaller id; a filtered candidate (its S
+// entry overwritten with kMaskedBits first) has key 0.  The k-th largest key is found by an MSB-first radix select
+// (8 passes of 8 bits over the row, read from L1 / L2), the keys at or above it are gathered and bitonic-sorted.
+// ---------------------------------------------------------------------------------------------------------------
+__device__ __forceinline__ uint64_t topk_key(const float* srow, int c) {
+  const uint32_t b = __float_as_uint(srow[c]);
+  if (b == kMaskedBits) return 0ull;
+  const uint32_t u = (b & 0x80000000u) ? ~b : (b | 0x80000000u);
+  return (uint64_t(u) << 32) | uint64_t(~uint32_t(c));
+}
+
+__device__ __forceinline__ float topk_score(uint64_t key) {
+  const uint32_t u = uint32_t(key >> 32);
+  return __uint_as_float((u & 0x80000000u) ? (u & 0x7fffffffu) : ~u);
+}
+
+__global__ void __launch_bounds__(kTopkThreads) rank_topk_kernel(float* __restrict__ S, int64_t lds, int32_t n,
+                                                                 int32_t n_rel, const int64_t* __restrict__ node,
+                                                                 const int64_t* __restrict__ rel,
+                                                                 const int32_t* __restrict__ f_rowptr,
+                                                                 const int32_t* __restrict__ f_dst, int k, int sigmoid,
+                                                                 float* __restrict__ out_score,
+                                                                 int64_t* __restrict__ out_id) {
+  __shared__ int hist[256];
+  __shared__ uint64_t sel[kTopkMax];
+  __shared__ int warp_cnt[kTopkThreads / 32];
+  __shared__ uint64_t prefix_s;
+  __shared__ int remaining_s, n_sel;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int64_t qi = blockIdx.x;
+  float* srow = S + qi * lds;
+  if (f_rowptr != nullptr) {
+    const int64_t row = node[qi] * n_rel + rel[qi];
+    for (int j = f_rowptr[row] + tid; j < f_rowptr[row + 1]; j += kTopkThreads) srow[f_dst[j]] = __uint_as_float(kMaskedBits);
+  }
+  __syncthreads();
+  // admissible candidates
+  int a = 0;
+  for (int c = tid; c < n; c += kTopkThreads) a += topk_key(srow, c) != 0ull;
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) a += __shfl_xor_sync(kFull, a, o);
+  if (lane == 0) warp_cnt[warp] = a;
+  __syncthreads();
+  int admissible = 0;
+#pragma unroll
+  for (int w = 0; w < kTopkThreads / 32; ++w) admissible += warp_cnt[w];
+  uint64_t thresh = 1ull;                      // fewer than k admissible: every admissible key
+  if (admissible > k) {
+    if (tid == 0) {
+      prefix_s = 0ull;
+      remaining_s = k;
+    }
+    uint64_t mask = 0ull;
+    for (int shift = 56; shift >= 0; shift -= 8) {
+      hist[tid] = 0;
+      __syncthreads();
+      const uint64_t prefix = prefix_s;
+      for (int c = tid; c < n; c += kTopkThreads) {
+        const uint64_t key = topk_key(srow, c);
+        if (key != 0ull && (key & mask) == prefix) atomicAdd(&hist[int(key >> shift) & 255], 1);
+      }
+      __syncthreads();
+      if (warp == 0) {
+        // lane l owns digits 255-8l .. 248-8l (descending); find the digit at which the running count from the
+        // top reaches `remaining`
+        int cnt[8], tot = 0;
+#pragma unroll
+        for (int i = 0; i < 8; ++i) {
+          cnt[i] = hist[255 - 8 * lane - i];
+          tot += cnt[i];
+        }
+        int incl = tot;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+          const int t = __shfl_up_sync(kFull, incl, o);
+          if (lane >= o) incl += t;
+        }
+        const int rem = remaining_s;
+        const unsigned hit = __ballot_sync(kFull, incl >= rem);
+        const int owner = __ffs(hit) - 1;
+        if (lane == owner) {
+          int run = incl - tot;
+#pragma unroll
+          for (int i = 0; i < 8; ++i) {
+            if (run + cnt[i] >= rem) {
+              prefix_s = prefix | (uint64_t(255 - 8 * lane - i) << shift);
+              remaining_s = rem - run;
+              break;
+            }
+            run += cnt[i];
+          }
+        }
+      }
+      mask |= 0xffull << shift;
+      __syncthreads();
+    }
+    thresh = prefix_s;
+  }
+  if (tid == 0) n_sel = 0;
+  sel[tid] = 0ull;
+  __syncthreads();
+  for (int c = tid; c < n; c += kTopkThreads) {
+    const uint64_t key = topk_key(srow, c);
+    if (key != 0ull && key >= thresh) {
+      const int at = atomicAdd(&n_sel, 1);
+      if (at < kTopkMax) sel[at] = key;
+    }
+  }
+  __syncthreads();
+  // bitonic sort of the 256 slots, descending
+  for (int size = 2; size <= kTopkMax; size <<= 1) {
+    for (int stride = size >> 1; stride > 0; stride >>= 1) {
+      const int partner = tid ^ stride;
+      if (partner > tid) {
+        const uint64_t x = sel[tid], y = sel[partner];
+        const bool desc = (tid & size) == 0;
+        if (desc ? (x < y) : (x > y)) {
+          sel[tid] = y;
+          sel[partner] = x;
+        }
+      }
+      __syncthreads();
+    }
+  }
+  if (tid < k) {
+    const uint64_t key = sel[tid];
+    float v = __uint_as_float(0x7fc00000u);
+    int64_t id = -1;
+    if (key != 0ull) {
+      v = topk_score(key);
+      if (sigmoid) v = 1.0f / (1.0f + expf(-v));
+      id = int64_t(~uint32_t(key));
+    }
+    out_score[qi * k + tid] = v;
+    out_id[qi * k + tid] = id;
+  }
+}
+
+}  // namespace gn
+
+using namespace gn;
+
+extern "C" {
+
+size_t gn_rank_csr_workspace_bytes(int64_t n_edges, int32_t n_nodes, int32_t n_rel) {
+  const size_t E = size_t(n_edges > 0 ? n_edges : 1);
+  const int64_t rows = int64_t(n_nodes > 0 ? n_nodes : 1) * (n_rel > 0 ? n_rel : 1);
+  return 4 * align_up(E * 4) + sort_ws_bytes(n_edges) + 2 * align_up(size_t(rows) * 4) + scan_ws_bytes(rows) + 4096;
+}
+
+int gn_rank_csr(const int64_t* src, const int64_t* dst, const int64_t* etype, int64_t n_edges, int32_t n_nodes,
+                int32_t n_rel, int32_t* rowptr, int32_t* ent_dst, int32_t* ent_eid, int32_t* group_row,
+                int32_t* n_groups, void* ws, size_t ws_bytes, void* stream) {
+  if (n_edges < 0 || n_nodes <= 0 || n_rel <= 0 || !rowptr) return GN_ERR_ARG;
+  if (n_edges > 0 && (!src || !dst || !etype || !ent_dst || !ent_eid)) return GN_ERR_ARG;
+  if ((group_row == nullptr) != (n_groups == nullptr)) return GN_ERR_ARG;
+  if (n_edges >= (int64_t(1) << 31) || int64_t(n_nodes) * n_rel >= (int64_t(1) << 31)) return GN_ERR_RANGE;
+  cudaStream_t st = as_stream(stream);
+  const int32_t n_rows = n_nodes * n_rel;
+  const size_t Ea = size_t(n_edges > 0 ? n_edges : 1);
+  Arena a(ws, ws_bytes);
+  int32_t* key1 = a.take<int32_t>(Ea);
+  int32_t* sorted1 = a.take<int32_t>(Ea);
+  int32_t* perm1 = a.take<int32_t>(Ea);
+  int32_t* key2 = a.take<int32_t>(Ea);
+  int32_t* flag = a.take<int32_t>(size_t(n_rows));
+  int32_t* pos = a.take<int32_t>(size_t(n_rows));
+  if (!a.ok()) return GN_ERR_WORKSPACE;
+  void* rest = a.base + a.off;
+  const size_t rest_bytes = a.cap - a.off;
+  int32_t* sorted2 = sorted1;                        // free once key2 is formed
+  if (n_edges > 0) {
+    const unsigned ge = (unsigned)ceil_div(n_edges, 256);
+    GN_LAUNCH(rank_dst_keys_kernel, ge, 256, 0, st, dst, n_edges, key1);
+    GN_CHECK(sort_pairs(key1, nullptr, sorted1, perm1, n_edges, bits_for(n_nodes > 1 ? n_nodes : 2), rest,
+                        rest_bytes, st));
+    GN_LAUNCH(rank_row_keys_kernel, ge, 256, 0, st, src, etype, (const int32_t*)perm1, n_edges, n_rel, key2);
+    GN_CHECK(sort_pairs(key2, perm1, sorted2, ent_eid, n_edges, bits_for(n_rows > 1 ? n_rows : 2), rest, rest_bytes,
+                        st));
+    GN_LAUNCH(rank_fill_kernel, ge, 256, 0, st, dst, (const int32_t*)ent_eid, n_edges, ent_dst);
+  }
+  GN_CHECK(rowptr_from_sorted(sorted2, n_edges, n_rows, rowptr, st));
+  if (group_row != nullptr) {
+    const unsigned gr = (unsigned)ceil_div(n_rows, 256);
+    GN_LAUNCH(rank_row_flags_kernel, gr, 256, 0, st, (const int32_t*)rowptr, n_rows, flag);
+    GN_CHECK(exclusive_scan_i32(flag, pos, n_rows, n_groups, rest, rest_bytes, st));
+    GN_LAUNCH(rank_groups_kernel, gr, 256, 0, st, (const int32_t*)rowptr, (const int32_t*)pos, n_rows, group_row);
+  }
+  return GN_OK;
+}
+
+int gn_rank_query_rows(const float* z, int64_t ldz, int32_t D, const float* w, int32_t n_rel, const int32_t* group_row,
+                       const int64_t* node, const int64_t* rel, int64_t count, float* q, int64_t ldq, void* stream) {
+  if (count < 0 || D <= 0 || n_rel <= 0 || ldq < D) return GN_ERR_ARG;
+  if (count == 0) return GN_OK;
+  if (!z || !w || !q || (!group_row && (!node || !rel))) return GN_ERR_ARG;
+  GN_LAUNCH(rank_query_rows_kernel, (unsigned)ceil_div(count * D, 256), 256, 0, as_stream(stream), z, ldz, D, w, n_rel,
+            group_row, node, rel, count, q, ldq);
+  return GN_OK;
+}
+
+int gn_rank_count(const float* S, int64_t lds, int32_t n_nodes, const int32_t* group_row, int32_t n_groups,
+                  const int32_t* q_rowptr, const int32_t* q_dst, const int32_t* q_eid, const int32_t* f_rowptr,
+                  const int32_t* f_dst, float* rank, void* stream) {
+  if (n_groups < 0 || n_nodes <= 0 || lds < n_nodes) return GN_ERR_ARG;
+  if (n_groups == 0) return GN_OK;
+  if (!S || !group_row || !q_rowptr || !q_dst || !q_eid || !rank || (f_rowptr && !f_dst)) return GN_ERR_ARG;
+  GN_LAUNCH(rank_count_kernel, (unsigned)ceil_div(n_groups, kCountWarps), kCountWarps * 32, 0, as_stream(stream), S,
+            lds, n_nodes, group_row, n_groups, q_rowptr, q_dst, q_eid, f_rowptr, f_dst, rank);
+  return GN_OK;
+}
+
+int gn_rank_max_hits(void) { return kRankMaxHits; }
+
+int gn_rank_metrics(const float* rank, const int32_t* rel_rowptr, const int32_t* rel_perm, int32_t n_rel,
+                    const int32_t* hits_k, int32_t n_hits, double* out, void* stream) {
+  if (n_rel < 0 || n_hits < 0 || n_hits > kRankMaxHits || (n_hits > 0 && !hits_k)) return GN_ERR_ARG;
+  if (n_rel == 0) return GN_OK;
+  if (!rel_rowptr || !out) return GN_ERR_ARG;
+  HitsK hk{};
+  for (int i = 0; i < n_hits; ++i) hk.k[i] = hits_k[i];
+  GN_LAUNCH(rank_metrics_kernel, (unsigned)n_rel, kMetricThreads, 0, as_stream(stream), rank, rel_rowptr, rel_perm,
+            n_rel, hk, n_hits, out);
+  return GN_OK;
+}
+
+int gn_rank_topk(float* S, int64_t lds, int32_t n_nodes, int32_t n_rel, const int64_t* node, const int64_t* rel,
+                 int64_t count, const int32_t* f_rowptr, const int32_t* f_dst, int32_t k, int sigmoid,
+                 float* out_score, int64_t* out_id, void* stream) {
+  if (count < 0 || n_nodes <= 0 || n_rel <= 0 || lds < n_nodes || k < 1 || k > kTopkMax) return GN_ERR_ARG;
+  if (count == 0) return GN_OK;
+  if (count >= (int64_t(1) << 31)) return GN_ERR_RANGE;
+  if (!S || !node || !rel || !out_score || !out_id || (f_rowptr && !f_dst)) return GN_ERR_ARG;
+  GN_LAUNCH(rank_topk_kernel, (unsigned)count, kTopkThreads, 0, as_stream(stream), S, lds, n_nodes, n_rel, node, rel,
+            f_rowptr, f_dst, k, sigmoid, out_score, out_id);
+  return GN_OK;
+}
+
+}  // extern "C"

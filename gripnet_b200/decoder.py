@@ -4,7 +4,7 @@ import math
 import torch
 from torch.nn import Module, Parameter
 
-from . import ops
+from . import ops, ranking
 from .parallel import replicated
 
 
@@ -35,6 +35,12 @@ class multiRelaInnerProductDecoder(Module):
         started the build of the backward's (node, relation) structures; the decoder's backward joins it."""
         return ops.DistMultPair.apply(z, replicated(self.weight, self.dist_ctx), pos_edge_index, neg_edge_index,
                                       edge_type, bool(sigmoid), int(rel_lo), n_rel_local, struct_branch)
+
+    def topk(self, z, node, rel, k, filter=None, sigmoid=True):
+        """The ``k`` most likely tails of every query ``(node[i], rel[i])`` under this decoder's weight, skipping the
+        known positives of ``filter`` (a ``ranking.EdgeFilter``): ``(scores [Q, k], ids int64 [Q, k])`` —
+        ``ranking.topk``.  No gradient flows through it."""
+        return ranking.topk(z, self.weight, node, rel, k, filter=filter, sigmoid=sigmoid)
 
     def reset_parameters(self):
         with torch.no_grad():

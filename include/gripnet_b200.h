@@ -383,6 +383,50 @@ size_t gn_nc_metrics_workspace_bytes(int32_t C);
 int gn_nc_metrics(const int64_t* target, const int64_t* pred, int64_t n, int32_t C, double* out,
                   void* ws, size_t ws_bytes, void* stream);
 
+/* ---- K16: filtered candidate ranking and top-k of the DistMult decoder --------------------------- */
+/* New capability (the reference evaluates each positive against ONE sampled negative, GripNet-pose.py:148-164).
+ * Every candidate tail c in [0, n) of a query (s, r), c == s included, is scored with the PRE-sigmoid DistMult
+ * score S(c) = sum_k z[s,k] w[r,k] z[c,k], evaluated as one row of S = Q . z^T with Q[g] = z[s_g] .* w[r_g]
+ * (gn_rank_query_rows, then the dense product gn_sgemm / gn_tc_gemm with transB = 1).  Only tail queries
+ * (s, r, ?) are ranked: lists holding both directions of every pair rank the head through the mirrored edge.
+ *
+ * gn_rank_csr: one-sided grouped structure of an edge list — rowptr [n_nodes*n_rel + 1] (row s*n_rel + r), entries
+ *   ent_dst / ent_eid [E] (candidate, edge id) sorted by candidate inside a row (two stable counting sorts).  A
+ *   FILTER (the set of directed known positives (s, r, c), e.g. train + test) is the structure of the concatenated
+ *   filter lists; duplicates stay stored and are skipped where they are read.  group_row / n_groups (both or
+ *   neither): the ids of the non-empty rows in ascending order ("groups", capacity n_nodes*n_rel) and their count
+ *   (device int32).
+ * gn_rank_query_rows: q[i, 0:D] = z[s_i] .* w[r_i], with (s_i, r_i) taken from group_row[i] = s*n_rel + r, or, when
+ *   group_row is NULL, from node[i] / rel[i].
+ * gn_rank_count: filtered rank of every target of groups [0, n_groups) whose score rows are S[g] (leading dimension
+ *   lds >= n_nodes; group_row points at the first group of the chunk).  OGB rule: with the negatives
+ *   N = {c != t : (s, r, c) not in the filter}, opt = #{c in N : S(c) > S(t)}, pess = #{c in N : S(c) >= S(t)},
+ *   rank[edge id] = 1 + (opt + pess) / 2 (float32).  S(t) is read from the same row as every S(c).  f_rowptr ==
+ *   NULL: no filter.
+ * gn_rank_metrics: out (DEVICE double [1 + n_hits, n_rel]) = MRR = mean(1/rank) and Hits@k = mean(rank <= k) per
+ *   relation over the edges rel_perm[rel_rowptr[r] : rel_rowptr[r+1]] (gn_index_prep of the edge types); NaN for a
+ *   relation without edges.  hits_k is a HOST array of at most gn_rank_max_hits() entries (it travels in the
+ *   kernel-parameter block: capturable).  Fixed-order float64 sums: repeated calls are bit-identical.
+ * gn_rank_topk: the k (1 <= k <= 256) highest-scoring candidates c with (node[i], rel[i], c) not in the filter, for
+ *   every query row i of S (overwritten: filtered entries are marked in place).  Order: descending pre-sigmoid
+ *   score, ties by smaller id.  out_score / out_id [count, k]: score (sigmoid applied when `sigmoid`) and id; id -1
+ *   and score NaN pad a query with fewer than k admissible candidates. */
+size_t gn_rank_csr_workspace_bytes(int64_t n_edges, int32_t n_nodes, int32_t n_rel);
+int gn_rank_csr(const int64_t* src, const int64_t* dst, const int64_t* etype, int64_t n_edges, int32_t n_nodes,
+                int32_t n_rel, int32_t* rowptr, int32_t* ent_dst, int32_t* ent_eid, int32_t* group_row /*or NULL*/,
+                int32_t* n_groups /*or NULL*/, void* ws, size_t ws_bytes, void* stream);
+int gn_rank_query_rows(const float* z, int64_t ldz, int32_t D, const float* w, int32_t n_rel, const int32_t* group_row,
+                       const int64_t* node, const int64_t* rel, int64_t count, float* q, int64_t ldq, void* stream);
+int gn_rank_count(const float* S, int64_t lds, int32_t n_nodes, const int32_t* group_row, int32_t n_groups,
+                  const int32_t* q_rowptr, const int32_t* q_dst, const int32_t* q_eid,
+                  const int32_t* f_rowptr /*or NULL*/, const int32_t* f_dst, float* rank, void* stream);
+int gn_rank_max_hits(void);
+int gn_rank_metrics(const float* rank, const int32_t* rel_rowptr, const int32_t* rel_perm, int32_t n_rel,
+                    const int32_t* hits_k /*host*/, int32_t n_hits, double* out, void* stream);
+int gn_rank_topk(float* S, int64_t lds, int32_t n_nodes, int32_t n_rel, const int64_t* node, const int64_t* rel,
+                 int64_t count, const int32_t* f_rowptr /*or NULL*/, const int32_t* f_dst, int32_t k, int sigmoid,
+                 float* out_score, int64_t* out_id, void* stream);
+
 /* ---- K12: slot all-gather over NVLink peer memory (multi-GPU exchange step) ------------------ */
 /* New design (the reference is single-device, SURVEY.md §8e).  Every rank of the node maps one
  * symmetric arena of identical layout; `arena_base` (HOST array, `world + 1` entries) holds every rank's
