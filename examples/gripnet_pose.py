@@ -29,7 +29,8 @@ def main():
     ap.add_argument("--seed", type=int, default=1111)
     ap.add_argument("--rank", action="store_true",
                     help="also print the filtered test MRR and Hits@10 (all drugs as candidate tails, train + test "
-                         "positives filtered), macro-averaged over relations")
+                         "positives filtered) and the filtered test relation MRR and Hits@10 (all side effects as "
+                         "candidates of each drug pair), macro-averaged over relations")
     args = ap.parse_args()
 
     from gripnet_b200 import data as gd, metrics, ranking, utils
@@ -60,7 +61,10 @@ def main():
         pos = [(train["dd_edge_index"], train["dd_edge_type"]), (test["dd_edge_index"], test["dd_edge_type"])]
         filt = ranking.EdgeFilter(pos, test["n_d"], n_rel)
         ranker = ranking.LinkRanker(test["dd_edge_index"], test["dd_edge_type"], test["n_d"], n_rel, filter=filt)
+        rel_ranker = ranking.RelationRanker(test["dd_edge_index"], test["dd_edge_type"], test["n_d"], n_rel,
+                                            filter=filt)
         rank_rec = torch.empty(args.epochs, 2, n_rel, dtype=torch.float64, device=dev)
+        rel_rank_rec = torch.empty(args.epochs, 2, n_rel, dtype=torch.float64, device=dev)
     for epoch in range(args.epochs):
         t0 = time.time()
         losses[epoch] = trainer.train_epoch().detach()
@@ -72,17 +76,20 @@ def main():
             metrics.lp_metrics(pos, neg, test["dd_range_list"], out=test_rec[epoch])
             if ranker is not None:
                 ranker.metrics(z, model.dmt.weight, hits=(10,), out=rank_rec[epoch])
+                rel_ranker.metrics(z, model.dmt.weight, hits=(10,), out=rel_rank_rec[epoch])
         tr, te = train_rec[epoch].nanmean(dim=1).tolist(), test_rec[epoch].nanmean(dim=1).tolist()   # one sync per epoch
         line = "{:3d}   loss:{:0.4f}   train auprc:{:0.4f} auroc:{:0.4f} ap:{:0.4f}   test auprc:{:0.4f} auroc:{:0.4f} " \
                "ap:{:0.4f}".format(epoch, float(losses[epoch].detach()), *tr, *te)
         if ranker is not None:
             line += "   test mrr:{:0.4f} hits@10:{:0.4f}".format(*rank_rec[epoch].nanmean(dim=1).tolist())
+            line += "   test relation mrr:{:0.4f} hits@10:{:0.4f}".format(*rel_rank_rec[epoch].nanmean(dim=1).tolist())
         print(line + "   time:{:0.3f}".format(time.time() - t0))
     os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
     torch.save({k: v.cpu() for k, v in model.state_dict().items()}, args.out + "-model.pt")
     rec = {"train_record": train_rec.cpu(), "test_record": test_rec.cpu(), "loss": losses.cpu()}
     if ranker is not None:
         rec["test_rank_record"] = rank_rec.cpu()             # [epochs, 2 (mrr, hits@10), R]
+        rec["test_relation_rank_record"] = rel_rank_rec.cpu()   # [epochs, 2 (mrr, hits@10), R]
     torch.save(rec, args.out + "-record.pt")
 
 

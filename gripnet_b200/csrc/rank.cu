@@ -3,6 +3,9 @@
 // Q[g] = z[s_g] .* w[r_g]; the product itself is the existing dense GEMM (gn_sgemm / gn_tc_gemm).  This file holds
 // what sits around it: the (src, rel)-grouped edge structure, the query rows, the filtered rank count, the
 // per-relation reduction and the per-query top-k selection.
+// Relation queries (s, ?, t) of a directed pair score every relation r' as one row of S = P . W^T with
+// P[g] = z[s_g] .* z[t_g]; they share the count and top-k kernels, templated on how a row finds its filter row, and
+// add a pair-grouped structure (rows = distinct directed pairs, sorted by (src, dst)) and a pair lookup.
 #include "sortkit.cuh"
 
 namespace gn {
@@ -48,45 +51,148 @@ __global__ void rank_groups_kernel(const int32_t* __restrict__ rowptr, const int
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-// query rows Q[i, :] = z[s_i, :] .* w[r_i, :]; (s, r) from a group row id s*R + r or from two index lists
+// pair-grouped structure: entries ordered by (src, dst, rel) with three stable counting sorts (by rel, by dst, by
+// src), rows = the distinct directed pairs in that order, entries (rel, edge id) sorted by rel inside a row.  Rows
+// are compacted pairs, not s*n + t: n^2 does not fit int32 for general n.
 // ---------------------------------------------------------------------------------------------------------------
-__global__ void rank_query_rows_kernel(const float* __restrict__ z, int64_t ldz, int D, const float* __restrict__ w,
-                                       int32_t n_rel, const int32_t* __restrict__ group_row,
-                                       const int64_t* __restrict__ node, const int64_t* __restrict__ rel,
-                                       int64_t count, float* __restrict__ q, int64_t ldq) {
+__global__ void rank_gather_keys_kernel(const int64_t* __restrict__ v, const int32_t* __restrict__ perm, int64_t n,
+                                        int32_t* __restrict__ key) {
+  const int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (i < n) key[i] = int32_t(v[perm ? perm[i] : int32_t(i)]);
+}
+
+__global__ void rank_pair_heads_kernel(const int64_t* __restrict__ src, const int64_t* __restrict__ dst,
+                                       const int32_t* __restrict__ eid, int64_t n, int32_t* __restrict__ flag) {
+  const int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const int32_t e = eid[i];
+  flag[i] = i == 0 || src[e] != src[eid[i - 1]] || dst[e] != dst[eid[i - 1]] ? 1 : 0;
+}
+
+__global__ void rank_pair_fill_kernel(const int64_t* __restrict__ src, const int64_t* __restrict__ dst,
+                                      const int64_t* __restrict__ etype, const int32_t* __restrict__ eid,
+                                      const int32_t* __restrict__ flag, const int32_t* __restrict__ pos, int64_t n,
+                                      int32_t* __restrict__ rowptr, int32_t* __restrict__ pair_src,
+                                      int32_t* __restrict__ pair_dst, int32_t* __restrict__ ent_rel) {
+  const int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const int32_t e = eid[i];
+  ent_rel[i] = int32_t(etype[e]);
+  if (flag[i]) {
+    const int32_t p = pos[i];
+    rowptr[p] = int32_t(i);
+    pair_src[p] = int32_t(src[e]);
+    pair_dst[p] = int32_t(dst[e]);
+  }
+  if (i == n - 1) rowptr[pos[i] + flag[i]] = int32_t(n);
+}
+
+// row of the filter's pair (s, t) by binary search over its (src, dst)-sorted pairs, or -1
+__global__ void rank_pair_lookup_kernel(const int32_t* __restrict__ f_src, const int32_t* __restrict__ f_dst,
+                                        int32_t n_fpairs, const int32_t* __restrict__ pair_src,
+                                        const int32_t* __restrict__ pair_dst, const int64_t* __restrict__ src,
+                                        const int64_t* __restrict__ dst, int64_t count, int32_t* __restrict__ row) {
+  const int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (i >= count) return;
+  const int32_t s = pair_src ? pair_src[i] : int32_t(src[i]);
+  const int32_t t = pair_src ? pair_dst[i] : int32_t(dst[i]);
+  int lo = 0, hi = n_fpairs;
+  while (lo < hi) {
+    const int mid = lo + ((hi - lo) >> 1);
+    const int32_t ms = f_src[mid];
+    if (ms < s || (ms == s && f_dst[mid] < t)) lo = mid + 1;
+    else hi = mid;
+  }
+  row[i] = (lo < n_fpairs && f_src[lo] == s && f_dst[lo] == t) ? lo : -1;
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// query rows q[i, :] = a_i .* b_i.  Tail queries: a = z[s], b = w[r], (s, r) from a group row id s*R + r or from two
+// index lists.  Relation queries: a = z[s], b = z[t], (s, t) from a pair-grouped structure or from two index lists.
+// ---------------------------------------------------------------------------------------------------------------
+struct TailOperands {
+  const float* z;
+  int64_t ldz;
+  const float* w;
+  int D;
+  int32_t n_rel;
+  const int32_t* group_row;
+  const int64_t* node;
+  const int64_t* rel;
+  __device__ __forceinline__ void at(int64_t i, const float*& a, const float*& b) const {
+    int64_t s, r;
+    if (group_row != nullptr) {
+      const int32_t g = group_row[i];
+      s = g / n_rel;
+      r = g - s * n_rel;
+    } else {
+      s = node[i];
+      r = rel[i];
+    }
+    a = z + s * ldz;
+    b = w + r * D;
+  }
+};
+
+struct PairOperands {
+  const float* z;
+  int64_t ldz;
+  const int32_t* pair_src;    // group pairs, or nullptr: the index lists
+  const int32_t* pair_dst;
+  const int64_t* src;
+  const int64_t* dst;
+  __device__ __forceinline__ void at(int64_t i, const float*& a, const float*& b) const {
+    const int64_t s = pair_src ? int64_t(pair_src[i]) : src[i];
+    const int64_t t = pair_src ? int64_t(pair_dst[i]) : dst[i];
+    a = z + s * ldz;
+    b = z + t * ldz;
+  }
+};
+
+template <class Operands>
+__global__ void rank_query_rows_kernel(const Operands ops, int D, int64_t count, float* __restrict__ q, int64_t ldq) {
   const int64_t t = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
   if (t >= count * D) return;
   const int64_t i = t / D;
   const int f = int(t - i * D);
-  int64_t s, r;
-  if (group_row != nullptr) {
-    const int32_t g = group_row[i];
-    s = g / n_rel;
-    r = g - s * n_rel;
-  } else {
-    s = node[i];
-    r = rel[i];
-  }
-  q[i * ldq + f] = z[s * ldz + f] * w[r * D + f];
+  const float *a, *b;
+  ops.at(i, a, b);
+  q[i * ldq + f] = a[f] * b[f];
 }
 
 // ---------------------------------------------------------------------------------------------------------------
 // filtered rank: one warp per group (a row of S), the group's targets in turn.  opt / pess count the candidates
 // c != t above / at-or-above S(t) over the whole row, then the distinct filtered candidates other than t that met
-// the same comparisons are taken back out.  S(t) is read from the same row as every S(c).
+// the same comparisons are taken back out.  S(t) is read from the same row as every S(c).  Rows says where group g's
+// targets and filter entries are: tail groups use the row s*R + r of both structures, relation groups (pairs) their
+// own compacted row and the filter row found by gn_rank_pair_lookup (-1: the pair has no filtered triple).
 // ---------------------------------------------------------------------------------------------------------------
 constexpr int kCountWarps = 8;
 
+struct TailRows {
+  const int32_t* group_row;
+  bool filtered;
+  __device__ __forceinline__ int32_t query(int g) const { return group_row[g]; }
+  __device__ __forceinline__ int32_t filter(int g) const { return filtered ? group_row[g] : -1; }
+};
+
+struct PairRows {
+  const int32_t* f_row;       // nullptr: no filter
+  __device__ __forceinline__ int32_t query(int g) const { return g; }
+  __device__ __forceinline__ int32_t filter(int g) const { return f_row ? f_row[g] : -1; }
+};
+
+template <class Rows>
 __global__ void __launch_bounds__(kCountWarps * 32) rank_count_kernel(
-    const float* __restrict__ S, int64_t lds, int32_t n, const int32_t* __restrict__ group_row, int32_t n_groups,
+    const float* __restrict__ S, int64_t lds, int32_t n, const Rows rows, int32_t n_groups,
     const int32_t* __restrict__ q_rowptr, const int32_t* __restrict__ q_dst, const int32_t* __restrict__ q_eid,
     const int32_t* __restrict__ f_rowptr, const int32_t* __restrict__ f_dst, float* __restrict__ rank) {
   const int lane = threadIdx.x & 31;
   const int g = blockIdx.x * kCountWarps + (threadIdx.x >> 5);
   if (g >= n_groups) return;
-  const int32_t row = group_row[g];
+  const int32_t row = rows.query(g), frow = rows.filter(g);
   const float* srow = S + int64_t(g) * lds;
-  const int f0 = f_rowptr ? f_rowptr[row] : 0, f1 = f_rowptr ? f_rowptr[row + 1] : 0;
+  const int f0 = frow >= 0 ? f_rowptr[frow] : 0, f1 = frow >= 0 ? f_rowptr[frow + 1] : 0;
   for (int j = q_rowptr[row]; j < q_rowptr[row + 1]; ++j) {
     const int t = q_dst[j];
     const float st = srow[t];
@@ -178,9 +284,23 @@ __device__ __forceinline__ float topk_score(uint64_t key) {
   return __uint_as_float((u & 0x80000000u) ? (u & 0x7fffffffu) : ~u);
 }
 
+// the filter row of query row qi (-1: none): s*R + r of a tail query, the looked-up pair row of a relation query
+struct TailFilterRow {
+  const int64_t* node;
+  const int64_t* rel;
+  int32_t n_rel;
+  bool filtered;
+  __device__ __forceinline__ int64_t operator()(int64_t qi) const { return filtered ? node[qi] * n_rel + rel[qi] : -1; }
+};
+
+struct PairFilterRow {
+  const int32_t* f_row;       // nullptr: no filter
+  __device__ __forceinline__ int64_t operator()(int64_t qi) const { return f_row ? f_row[qi] : -1; }
+};
+
+template <class FilterRow>
 __global__ void __launch_bounds__(kTopkThreads) rank_topk_kernel(float* __restrict__ S, int64_t lds, int32_t n,
-                                                                 int32_t n_rel, const int64_t* __restrict__ node,
-                                                                 const int64_t* __restrict__ rel,
+                                                                 const FilterRow filter_row,
                                                                  const int32_t* __restrict__ f_rowptr,
                                                                  const int32_t* __restrict__ f_dst, int k, int sigmoid,
                                                                  float* __restrict__ out_score,
@@ -193,8 +313,8 @@ __global__ void __launch_bounds__(kTopkThreads) rank_topk_kernel(float* __restri
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int64_t qi = blockIdx.x;
   float* srow = S + qi * lds;
-  if (f_rowptr != nullptr) {
-    const int64_t row = node[qi] * n_rel + rel[qi];
+  const int64_t row = filter_row(qi);
+  if (row >= 0) {
     for (int j = f_rowptr[row] + tid; j < f_rowptr[row + 1]; j += kTopkThreads) srow[f_dst[j]] = __uint_as_float(kMaskedBits);
   }
   __syncthreads();
@@ -358,8 +478,9 @@ int gn_rank_query_rows(const float* z, int64_t ldz, int32_t D, const float* w, i
   if (count < 0 || D <= 0 || n_rel <= 0 || ldq < D) return GN_ERR_ARG;
   if (count == 0) return GN_OK;
   if (!z || !w || !q || (!group_row && (!node || !rel))) return GN_ERR_ARG;
-  GN_LAUNCH(rank_query_rows_kernel, (unsigned)ceil_div(count * D, 256), 256, 0, as_stream(stream), z, ldz, D, w, n_rel,
-            group_row, node, rel, count, q, ldq);
+  const TailOperands ops{z, ldz, w, D, n_rel, group_row, node, rel};
+  GN_LAUNCH(rank_query_rows_kernel<TailOperands>, (unsigned)ceil_div(count * D, 256), 256, 0, as_stream(stream), ops,
+            D, count, q, ldq);
   return GN_OK;
 }
 
@@ -369,8 +490,9 @@ int gn_rank_count(const float* S, int64_t lds, int32_t n_nodes, const int32_t* g
   if (n_groups < 0 || n_nodes <= 0 || lds < n_nodes) return GN_ERR_ARG;
   if (n_groups == 0) return GN_OK;
   if (!S || !group_row || !q_rowptr || !q_dst || !q_eid || !rank || (f_rowptr && !f_dst)) return GN_ERR_ARG;
-  GN_LAUNCH(rank_count_kernel, (unsigned)ceil_div(n_groups, kCountWarps), kCountWarps * 32, 0, as_stream(stream), S,
-            lds, n_nodes, group_row, n_groups, q_rowptr, q_dst, q_eid, f_rowptr, f_dst, rank);
+  const TailRows rows{group_row, f_rowptr != nullptr};
+  GN_LAUNCH(rank_count_kernel<TailRows>, (unsigned)ceil_div(n_groups, kCountWarps), kCountWarps * 32, 0,
+            as_stream(stream), S, lds, n_nodes, rows, n_groups, q_rowptr, q_dst, q_eid, f_rowptr, f_dst, rank);
   return GN_OK;
 }
 
@@ -395,8 +517,100 @@ int gn_rank_topk(float* S, int64_t lds, int32_t n_nodes, int32_t n_rel, const in
   if (count == 0) return GN_OK;
   if (count >= (int64_t(1) << 31)) return GN_ERR_RANGE;
   if (!S || !node || !rel || !out_score || !out_id || (f_rowptr && !f_dst)) return GN_ERR_ARG;
-  GN_LAUNCH(rank_topk_kernel, (unsigned)count, kTopkThreads, 0, as_stream(stream), S, lds, n_nodes, n_rel, node, rel,
-            f_rowptr, f_dst, k, sigmoid, out_score, out_id);
+  const TailFilterRow frow{node, rel, n_rel, f_rowptr != nullptr};
+  GN_LAUNCH(rank_topk_kernel<TailFilterRow>, (unsigned)count, kTopkThreads, 0, as_stream(stream), S, lds, n_nodes,
+            frow, f_rowptr, f_dst, k, sigmoid, out_score, out_id);
+  return GN_OK;
+}
+
+size_t gn_rank_pair_csr_workspace_bytes(int64_t n_edges) {
+  const size_t E = size_t(n_edges > 0 ? n_edges : 1);
+  return 4 * align_up(E * 4) + sort_ws_bytes(n_edges) + scan_ws_bytes(n_edges) + 4096;
+}
+
+int gn_rank_pair_csr(const int64_t* src, const int64_t* dst, const int64_t* etype, int64_t n_edges, int32_t n_nodes,
+                     int32_t n_rel, int32_t* rowptr, int32_t* pair_src, int32_t* pair_dst, int32_t* ent_rel,
+                     int32_t* ent_eid, int32_t* n_pairs, void* ws, size_t ws_bytes, void* stream) {
+  if (n_edges < 0 || n_nodes <= 0 || n_rel <= 0 || !rowptr || !n_pairs) return GN_ERR_ARG;
+  if (n_edges > 0 && (!src || !dst || !etype || !pair_src || !pair_dst || !ent_rel || !ent_eid)) return GN_ERR_ARG;
+  if (n_edges >= (int64_t(1) << 31)) return GN_ERR_RANGE;
+  cudaStream_t st = as_stream(stream);
+  if (n_edges == 0) {
+    if (cudaMemsetAsync(rowptr, 0, 4, st) != cudaSuccess || cudaMemsetAsync(n_pairs, 0, 4, st) != cudaSuccess)
+      return GN_ERR_CUDA;
+    return GN_OK;
+  }
+  Arena a(ws, ws_bytes);
+  int32_t* key = a.take<int32_t>(size_t(n_edges));
+  int32_t* sorted = a.take<int32_t>(size_t(n_edges));
+  int32_t* perm1 = a.take<int32_t>(size_t(n_edges));
+  int32_t* perm2 = a.take<int32_t>(size_t(n_edges));
+  if (!a.ok()) return GN_ERR_WORKSPACE;
+  void* rest = a.base + a.off;
+  const size_t rest_bytes = a.cap - a.off;
+  const unsigned ge = (unsigned)ceil_div(n_edges, 256);
+  const int node_bits = bits_for(n_nodes > 1 ? n_nodes : 2);
+  // stable passes by rel, then dst, then src: entries in (src, dst, rel) order
+  GN_LAUNCH(rank_gather_keys_kernel, ge, 256, 0, st, etype, (const int32_t*)nullptr, n_edges, key);
+  GN_CHECK(sort_pairs(key, nullptr, sorted, perm1, n_edges, bits_for(n_rel > 1 ? n_rel : 2), rest, rest_bytes, st));
+  GN_LAUNCH(rank_gather_keys_kernel, ge, 256, 0, st, dst, (const int32_t*)perm1, n_edges, key);
+  GN_CHECK(sort_pairs(key, perm1, sorted, perm2, n_edges, node_bits, rest, rest_bytes, st));
+  GN_LAUNCH(rank_gather_keys_kernel, ge, 256, 0, st, src, (const int32_t*)perm2, n_edges, key);
+  GN_CHECK(sort_pairs(key, perm2, sorted, ent_eid, n_edges, node_bits, rest, rest_bytes, st));
+  // run heads -> compacted pair rows
+  int32_t* flag = key;
+  int32_t* pos = sorted;
+  GN_LAUNCH(rank_pair_heads_kernel, ge, 256, 0, st, src, dst, (const int32_t*)ent_eid, n_edges, flag);
+  GN_CHECK(exclusive_scan_i32(flag, pos, n_edges, n_pairs, rest, rest_bytes, st));
+  GN_LAUNCH(rank_pair_fill_kernel, ge, 256, 0, st, src, dst, etype, (const int32_t*)ent_eid, (const int32_t*)flag,
+            (const int32_t*)pos, n_edges, rowptr, pair_src, pair_dst, ent_rel);
+  return GN_OK;
+}
+
+int gn_rank_pair_lookup(const int32_t* f_src, const int32_t* f_dst, int32_t n_fpairs, const int32_t* pair_src,
+                        const int32_t* pair_dst, const int64_t* src, const int64_t* dst, int64_t count, int32_t* row,
+                        void* stream) {
+  if (count < 0 || n_fpairs < 0) return GN_ERR_ARG;
+  if (count == 0) return GN_OK;
+  if (!row || (n_fpairs > 0 && (!f_src || !f_dst)) || (pair_src ? !pair_dst : (!src || !dst))) return GN_ERR_ARG;
+  GN_LAUNCH(rank_pair_lookup_kernel, (unsigned)ceil_div(count, 256), 256, 0, as_stream(stream), f_src, f_dst,
+            n_fpairs, pair_src, pair_dst, src, dst, count, row);
+  return GN_OK;
+}
+
+int gn_rank_pair_rows(const float* z, int64_t ldz, int32_t D, const int32_t* pair_src, const int32_t* pair_dst,
+                      const int64_t* src, const int64_t* dst, int64_t count, float* p, int64_t ldp, void* stream) {
+  if (count < 0 || D <= 0 || ldp < D) return GN_ERR_ARG;
+  if (count == 0) return GN_OK;
+  if (!z || !p || (pair_src ? !pair_dst : (!src || !dst))) return GN_ERR_ARG;
+  const PairOperands ops{z, ldz, pair_src, pair_dst, src, dst};
+  GN_LAUNCH(rank_query_rows_kernel<PairOperands>, (unsigned)ceil_div(count * D, 256), 256, 0, as_stream(stream), ops,
+            D, count, p, ldp);
+  return GN_OK;
+}
+
+int gn_rank_pair_count(const float* S, int64_t lds, int32_t n_rel, int32_t n_pairs, const int32_t* q_rowptr,
+                       const int32_t* q_rel, const int32_t* q_eid, const int32_t* f_row, const int32_t* f_rowptr,
+                       const int32_t* f_rel, float* rank, void* stream) {
+  if (n_pairs < 0 || n_rel <= 0 || lds < n_rel) return GN_ERR_ARG;
+  if (n_pairs == 0) return GN_OK;
+  if (!S || !q_rowptr || !q_rel || !q_eid || !rank || (f_row && (!f_rowptr || !f_rel))) return GN_ERR_ARG;
+  const PairRows rows{f_row};
+  GN_LAUNCH(rank_count_kernel<PairRows>, (unsigned)ceil_div(n_pairs, kCountWarps), kCountWarps * 32, 0,
+            as_stream(stream), S, lds, n_rel, rows, n_pairs, q_rowptr, q_rel, q_eid, f_rowptr, f_rel, rank);
+  return GN_OK;
+}
+
+int gn_rank_pair_topk(float* S, int64_t lds, int32_t n_rel, int64_t count, const int32_t* f_row,
+                      const int32_t* f_rowptr, const int32_t* f_rel, int32_t k, int sigmoid, float* out_score,
+                      int64_t* out_id, void* stream) {
+  if (count < 0 || n_rel <= 0 || lds < n_rel || k < 1 || k > kTopkMax) return GN_ERR_ARG;
+  if (count == 0) return GN_OK;
+  if (count >= (int64_t(1) << 31)) return GN_ERR_RANGE;
+  if (!S || !out_score || !out_id || (f_row && (!f_rowptr || !f_rel))) return GN_ERR_ARG;
+  const PairFilterRow frow{f_row};
+  GN_LAUNCH(rank_topk_kernel<PairFilterRow>, (unsigned)count, kTopkThreads, 0, as_stream(stream), S, lds, n_rel, frow,
+            f_rowptr, f_rel, k, sigmoid, out_score, out_id);
   return GN_OK;
 }
 

@@ -42,6 +42,12 @@ class multiRelaInnerProductDecoder(Module):
         ``ranking.topk``.  No gradient flows through it."""
         return ranking.topk(z, self.weight, node, rel, k, filter=filter, sigmoid=sigmoid)
 
+    def topk_relations(self, z, src, dst, k, filter=None, sigmoid=True):
+        """The ``k`` most likely relations of every directed pair ``(src[i], dst[i])`` under this decoder's weight,
+        skipping the known triples of ``filter``: ``(scores [Q, k], relation ids int64 [Q, k])`` —
+        ``ranking.topk_relations``.  No gradient flows through it."""
+        return ranking.topk_relations(z, self.weight, src, dst, k, filter=filter, sigmoid=sigmoid)
+
     def reset_parameters(self):
         with torch.no_grad():
             self.weight.normal_(std=1.0 / math.sqrt(self.in_dim))          # decoder.py:25-26

@@ -427,6 +427,47 @@ int gn_rank_topk(float* S, int64_t lds, int32_t n_nodes, int32_t n_rel, const in
                  int64_t count, const int32_t* f_rowptr /*or NULL*/, const int32_t* f_dst, int32_t k, int sigmoid,
                  float* out_score, int64_t* out_id, void* stream);
 
+/* Relation queries (s, ?, t) of a directed pair: every relation r' in [0, n_rel) is a candidate, scored with the
+ * PRE-sigmoid S(r') = sum_k z[s,k] z[t,k] w[r',k], one row of S = P . W^T with P[g] = z[s_g] .* z[t_g]
+ * (gn_rank_pair_rows, then gn_sgemm / gn_tc_gemm with transB = 1; W the decoder weight [n_rel, D]).  P is bitwise
+ * symmetric (fp32 products commute), so (s, t) and (t, s) give identical rows when both take the same product path.
+ * Filter: the same set of directed known triples (s, r', t), duplicates counted once.  For a query triple (s, r, t):
+ * N = {r' != r : (s, r', t) not in the filter}, opt = #{r' in N : S(r') > S(r)}, pess = #{r' in N : S(r') >= S(r)},
+ * rank = 1 + (opt + pess) / 2, S(r) read from the same row as every S(r').  Metrics: gn_index_prep of the query
+ * triples' relations, then gn_rank_metrics.
+ *
+ * gn_rank_pair_csr: pair-grouped structure of an edge list.  Three stable counting sorts (by rel, by dst, by src)
+ *   order the entries by (src, dst, rel); rows are the distinct directed pairs in (src, dst) order, compacted (not
+ *   s*n + t, which does not fit int32 for general n): rowptr [capacity n_edges + 1], pair_src / pair_dst [capacity
+ *   n_edges], entries ent_rel / ent_eid [n_edges] (relation, edge id) sorted by relation inside a row; n_pairs
+ *   (device int32) the row count.
+ * gn_rank_pair_lookup: row[i] = the row of pair (s_i, t_i) in a pair-grouped filter of n_fpairs rows (binary search
+ *   over its sorted pairs), or -1 when the filter holds no triple of that pair.  (s_i, t_i) from pair_src / pair_dst
+ *   (int32, e.g. a query structure's pairs) or, when pair_src is NULL, from src / dst (int64).
+ * gn_rank_pair_rows: p[i, 0:D] = z[s_i] .* z[t_i], (s_i, t_i) taken as in gn_rank_pair_lookup.
+ * gn_rank_pair_count: filtered relation rank of every entry of pairs [0, n_pairs) whose score rows are S[g] (lds >=
+ *   n_rel; q_rowptr and f_row point at the first pair of the chunk); f_row[g] is the filter row of pair g (from
+ *   gn_rank_pair_lookup), f_row == NULL: no filter.  rank[edge id] as in gn_rank_count.
+ * gn_rank_pair_topk: the k (1 <= k <= 256; k > n_rel is padded) highest-scoring relations r' with (s_i, r', t_i)
+ *   not in the filter, for every row i of S (overwritten: filtered entries are marked in place); f_row[i] the
+ *   filter row of query i, or f_row == NULL.  Order, padding and sigmoid as in gn_rank_topk. */
+size_t gn_rank_pair_csr_workspace_bytes(int64_t n_edges);
+int gn_rank_pair_csr(const int64_t* src, const int64_t* dst, const int64_t* etype, int64_t n_edges, int32_t n_nodes,
+                     int32_t n_rel, int32_t* rowptr, int32_t* pair_src, int32_t* pair_dst, int32_t* ent_rel,
+                     int32_t* ent_eid, int32_t* n_pairs, void* ws, size_t ws_bytes, void* stream);
+int gn_rank_pair_lookup(const int32_t* f_src, const int32_t* f_dst, int32_t n_fpairs,
+                        const int32_t* pair_src /*or NULL*/, const int32_t* pair_dst, const int64_t* src,
+                        const int64_t* dst, int64_t count, int32_t* row, void* stream);
+int gn_rank_pair_rows(const float* z, int64_t ldz, int32_t D, const int32_t* pair_src /*or NULL*/,
+                      const int32_t* pair_dst, const int64_t* src, const int64_t* dst, int64_t count, float* p,
+                      int64_t ldp, void* stream);
+int gn_rank_pair_count(const float* S, int64_t lds, int32_t n_rel, int32_t n_pairs, const int32_t* q_rowptr,
+                       const int32_t* q_rel, const int32_t* q_eid, const int32_t* f_row /*or NULL*/,
+                       const int32_t* f_rowptr, const int32_t* f_rel, float* rank, void* stream);
+int gn_rank_pair_topk(float* S, int64_t lds, int32_t n_rel, int64_t count, const int32_t* f_row /*or NULL*/,
+                      const int32_t* f_rowptr, const int32_t* f_rel, int32_t k, int sigmoid, float* out_score,
+                      int64_t* out_id, void* stream);
+
 /* ---- K12: slot all-gather over NVLink peer memory (multi-GPU exchange step) ------------------ */
 /* New design (the reference is single-device, SURVEY.md §8e).  Every rank of the node maps one
  * symmetric arena of identical layout; `arena_base` (HOST array, `world + 1` entries) holds every rank's
