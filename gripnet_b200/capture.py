@@ -29,7 +29,7 @@ class CapturedStep:
         cur = torch.cuda.current_stream()
         # warm-up and capture run on ONE high-priority stream: the chain's kernels keep that priority in the graph,
         # the background branches (streams.Branch(background=True)) stay below it
-        side = torch.cuda.Stream(priority=streams.chain_priority())
+        side = torch.cuda.Stream(priority=streams.CHAIN_PRIORITY)
         side.wait_stream(cur)
         with torch.cuda.stream(side):
             for _ in range(max(int(warmup), 1)):      # builds and caches every static graph structure

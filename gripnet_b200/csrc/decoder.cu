@@ -1,8 +1,6 @@
 // K9/K10/K11: DistMult link decoder (fused gather-multiply-reduce), its
 // deterministic backward, and the softmax pieces of the multi-class decoder.
 // Reference arithmetic restated: gripnet/decoder.py:19-23, :38-45.
-#include <cstdlib>
-
 #include "rowsplit.cuh"
 #include "sortkit.cuh"
 
@@ -583,14 +581,9 @@ struct WidthPlan {
 };
 
 // lanes-per-entry and vectors-per-lane for a D-wide row (at most kMaxNV vectors per lane)
-inline WidthPlan plan_width(int D, bool can_vec4, bool wide = false) {
+inline WidthPlan plan_width(int D, bool can_vec4) {
   WidthPlan p{can_vec4 ? 4 : 1, 0, 0, true};
   const int units = (D + p.vec - 1) / p.vec;
-  if (wide && can_vec4 && units > 8 && units <= 24) {   // 8 lanes x 3 vectors: fewer registers, more warps per SM
-    p.lpe = 8;
-    p.nv = 3;
-    return p;
-  }
   if (units <= 4 * kMaxNV) p.lpe = 4;
   else if (units <= 32 * kMaxNV) p.lpe = 32;
   else p.ok = false;
@@ -599,12 +592,6 @@ inline WidthPlan plan_width(int D, bool can_vec4, bool wide = false) {
     p.nv = need <= 1 ? 1 : need <= 2 ? 2 : need <= 4 ? 4 : need <= 5 ? 5 : kMaxNV;
   }
   return p;
-}
-
-// GRIPNET_B200_DECODER_KERNELS=legacy keeps the per-edge / per-entry forms (A/B measurements, parity tests of both)
-static bool legacy_decoder_kernels() {
-  const char* e = std::getenv("GRIPNET_B200_DECODER_KERNELS");
-  return e && e[0] == 'l';
 }
 
 }  // namespace gn
@@ -619,8 +606,11 @@ int gn_distmult_fwd(const float* z, int64_t ldz, int32_t D, const float* w, cons
   if (n_edges == 0) return GN_OK;
   if (!z || !w || !src || !dst || !etype || !out) return GN_ERR_ARG;
   cudaStream_t st = as_stream(stream);
-  const bool v4 = (D % 4 == 0) && (ldz % 4 == 0) && aligned16(z) && aligned16(w);
-  if (v4 && D <= 128 && ldz < (int64_t(1) << 30) && !legacy_decoder_kernels()) {
+  // float4 rows.  Up to D = 128 they take the batch form, which steps rows with a 32-bit byte stride, so there a z row
+  // stride of 2^30 floats or more takes the scalar per-edge form.
+  const bool v4 = (D % 4 == 0) && (ldz % 4 == 0) && aligned16(z) && aligned16(w) &&
+                  (D > 128 || ldz < (int64_t(1) << 30));
+  if (v4 && D <= 128) {
     const int nv = (D / 4 + 7) / 8;
     int64_t nwarps = ceil_div(n_edges, 32);
     const int64_t cap = int64_t(148) * 4 * 8;                // one wave of resident warps; each walks its batches
@@ -649,7 +639,6 @@ int gn_distmult_fwd(const float* z, int64_t ldz, int32_t D, const float* w, cons
     GN_LAUNCH((distmult_fwd_kernel<L, V>), grid, 256, 0, st, z, ldz, D, w, src, dst, etype, n_edges, sigmoid, out); \
     return GN_OK;                                                                                                   \
   }
-  GN_FWD_CASE(4, 4)
   GN_FWD_CASE(8, 4)
   GN_FWD_CASE(32, 4)
   GN_FWD_CASE(4, 1)
@@ -726,12 +715,14 @@ int gn_distmult_bwd_pairs(const gn_csr* pair_csr, const int32_t* ent_other, cons
   const gn_csr& csr = *pair_csr;
   if (csr.n_rows == 0 || csr.n_chunks == 0) return GN_OK;
   if (csr.n_chunks > csr.n_rows && !partial) return GN_ERR_ARG;
-  const bool v4 = (D % 4 == 0) && (ldz % 4 == 0) && aligned16(z) && aligned16(T) && (!partial || aligned16(partial));
-  const WidthPlan p = plan_width(D, v4, true);
+  // float4 rows: the batch form up to D = 128, where (as in gn_distmult_fwd) the z row stride must stay below 2^30
+  const bool v4 = (D % 4 == 0) && (ldz % 4 == 0) && aligned16(z) && aligned16(T) && (!partial || aligned16(partial)) &&
+                  (D > 128 || ldz < (int64_t(1) << 30));
+  const WidthPlan p = plan_width(D, v4);
   if (!p.ok) return GN_ERR_ARG;
   cudaStream_t st = as_stream(stream);
   const unsigned grid = (unsigned)ceil_div(csr.n_chunks, 8);
-  if (v4 && D <= 128 && ldz < (int64_t(1) << 30) && !legacy_decoder_kernels()) {
+  if (v4 && D <= 128) {
     const int nv = (D / 4 + 7) / 8;
 #define GN_PWB_CASE(N)                                                                                        \
   if (nv == N) {                                                                                              \
@@ -751,11 +742,11 @@ int gn_distmult_bwd_pairs(const gn_csr* pair_csr, const int32_t* ent_other, cons
               partial);                                                                                      \
     return GN_OK;                                                                                            \
   }
-#define GN_PW_CASES(L, V) GN_PW_CASE(L, V, 1) GN_PW_CASE(L, V, 2) GN_PW_CASE(L, V, 4) GN_PW_CASE(L, V, 5) \
-  GN_PW_CASE(L, V, 8)
-  GN_PW_CASES(4, 4)
-  GN_PW_CASE(8, 4, 3)
+// the per-entry form serves float4 rows only past D = 128, and 32 lanes per entry only past 32 units per row
+// (so at least two vectors per lane)
+#define GN_PW_CASES(L, V) GN_PW_CASE(L, V, 2) GN_PW_CASE(L, V, 4) GN_PW_CASE(L, V, 5) GN_PW_CASE(L, V, 8)
   GN_PW_CASES(32, 4)
+  GN_PW_CASE(4, 1, 1)
   GN_PW_CASES(4, 1)
   GN_PW_CASES(32, 1)
 #undef GN_PW_CASES

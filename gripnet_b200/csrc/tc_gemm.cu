@@ -476,12 +476,6 @@ static int tc_set_smem_attr() {
 
 // CTAs along M: persistent over the M tiles — as many CTAs as can be resident (two per SM when shared memory and
 // TMEM allow it), each walking its tiles with a stride of the grid
-// GRIPNET_B200_TC_PREFETCH=1 keeps the shallow loader everywhere (A/B measurements)
-static bool tc_shallow_only() {
-  const char* e = std::getenv("GRIPNET_B200_TC_PREFETCH");
-  return e && e[0] == '1';
-}
-
 static int tc_ctas_per_sm(const tc::Plan& pl) {
   return (2 * pl.smem_bytes <= 220 * 1024 && 2 * pl.tmem_cols <= 512) ? 2 : 1;
 }
@@ -496,7 +490,7 @@ static unsigned tc_grid_x(int M, const tc::Plan& pl) {
 
 // deep prefetch when one CTA owns an SM and walks several M tiles (a long stream of A); PF = 1 otherwise
 static int tc_launch(const tc::Plan& pl, int M, dim3 grid, const tc::Params& p, cudaStream_t st) {
-  const bool deep = tc_ctas_per_sm(pl) == 1 && ceil_div(M, tc::BM) > int64_t(grid.x) && !tc_shallow_only();
+  const bool deep = tc_ctas_per_sm(pl) == 1 && ceil_div(M, tc::BM) > int64_t(grid.x);
   if (deep) {
     GN_LAUNCH(tc::tc_gemm_kernel<3>, grid, tc::kThreads, pl.smem_bytes, st, p);
   } else {

@@ -15,7 +15,6 @@ import torch
 from . import _lib, streams
 
 _SM_COUNT = 148
-ROW_IS_CHUNK = os.environ.get("GRIPNET_B200_ROW_IS_CHUNK", "1") != "0"
 
 
 def _stream():
@@ -32,13 +31,6 @@ def _host_int(t):
     if s is not None:
         s.synchronize()
     return int(t.item())
-
-
-def _host_bool(t):
-    s = streams.override()
-    if s is not None:
-        s.synchronize()
-    return bool(t.item())
 
 
 def _ptr(t):
@@ -94,24 +86,11 @@ class Csr:
         else:
             self.n_chunks = cap - 1 if self.n_rows > 0 else 0
         # every row fits one chunk (known exactly): kernels read the row bounds straight from rowptr
-        self.flags = _lib.CSR_ROW_IS_CHUNK if (exact and ROW_IS_CHUNK and self.n_chunks == self.n_rows) else 0
+        self.flags = _lib.CSR_ROW_IS_CHUNK if (exact and self.n_chunks == self.n_rows) else 0
         self.c = _lib.GnCsr(self.n_rows, self.n_cols, self.nnz, self.chunk_len, self.n_chunks, self.flags,
                             _ptr(rowptr), _ptr(col), _ptr(val), _ptr(self.chunk_ptr), _ptr(self.chunk_row),
                             _ptr(self.chunk_beg), _ptr(self.row_counter))
         self.ref = C.byref(self.c)
-        self._alt = None
-
-    def alt_ref(self):
-        """The same CSR with a second set of row-arrival counters, so that two kernels may walk it
-        concurrently on different streams (``ops.DistMultPair``: dw of the positive and of the negative
-        edges share the relation CSR)."""
-        if self._alt is None:
-            rc = torch.zeros(max(self.n_rows, 1), dtype=torch.int32, device=self.rowptr.device)
-            c = _lib.GnCsr(self.n_rows, self.n_cols, self.nnz, self.chunk_len, self.n_chunks, self.flags,
-                           _ptr(self.rowptr), _ptr(self.col), _ptr(self.val), _ptr(self.chunk_ptr),
-                           _ptr(self.chunk_row), _ptr(self.chunk_beg), _ptr(rc))
-            self._alt = (c, C.byref(c), rc)
-        return self._alt[1]
 
     @property
     def extra_chunks(self):
@@ -527,11 +506,6 @@ class IndexStruct:
         _lib.check(lib.gn_index_prep(_ptr(idx) if n else None, n, n_nodes, _ptr(rowptr), _ptr(self.perm), _ptr(ws),
                                      ws.numel(), _stream()), "gn_index_prep")
         self.csr = Csr(rowptr, self.perm, None, n_nodes, max(n, 1), n, exact=exact)
-        # a non-decreasing index list (relation-major edge types) sorts to itself: consumers may then walk
-        # the list in place instead of through `perm`.  Known only for structures built outside a capture
-        # (one host read at build time); structures built inside a captured graph keep the general path.
-        self.identity = bool(exact and n > 0 and _host_bool(
-            (self.perm[:n] == torch.arange(n, dtype=torch.int32, device=dev)).all()))
 
 
 # --------------------------------------------------------------------------

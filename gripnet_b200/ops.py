@@ -9,7 +9,6 @@ gradients are fused into the producing kernels' epilogues.
 PyTorch is used for device memory (``torch.empty``) and streams only; every
 arithmetic step is a kernel of ``libgripnet_b200.so``.
 """
-import os
 import weakref
 
 import torch
@@ -100,16 +99,15 @@ def spmm(csr, x, out, F, row_scale=None, bias=None, addend=None, relu=False):
                            int(relu), out.ptr, out.ld, _ptr(partial), _stream()), "gn_spmm")
 
 
-# dense-transform dispatch: "auto" sends tall products (M >= _TC_MIN_M) to the tcgen05 3xTF32 kernel,
-# "ffma" keeps everything on the CUDA-core kernel, "tc" forces the tensor path whenever it is legal
-GEMM_PATH = os.environ.get("GRIPNET_B200_GEMM", "auto")
+# dense-transform dispatch: tall products (M >= _TC_MIN_M) go to the tcgen05 3xTF32 kernel, the rest to the
+# CUDA-core kernel
 _TC_MIN_M = 4096
 
 
 def _tc_eligible(ta, m, n, k, a_ptr, lda, c_ptr, ldc, batch, alpha, accumulate, addend, mask, a_rows):
-    if GEMM_PATH == "ffma" or ta or batch != 1 or a_rows is not None or accumulate or alpha != 1.0:
+    if ta or batch != 1 or a_rows is not None or accumulate or alpha != 1.0:
         return False
-    if GEMM_PATH != "tc" and (m < _TC_MIN_M or k < 16):
+    if m < _TC_MIN_M or k < 16:
         return False
     if k % 4 or lda % 4 or ldc % 4 or a_ptr % 16 or c_ptr % 16 or k > 4096:
         return False
@@ -150,9 +148,8 @@ def sgemm(ta, tb, m, n, k, a_ptr, lda, b_ptr, ldb, c_ptr, ldc, device, batch=1, 
 
 
 # relation transform Y[:, r, :] = X W[r]: tensor cores whenever the 3xTF32 kernel's alignment rules hold
-# ("ffma" keeps it on the CUDA cores — the A/B switch of the config-4 measurements)
 def _rel_tc_ok(k, ldx, ldy, x_ptr, y_ptr):
-    return GEMM_PATH != "ffma" and k % 4 == 0 and ldx % 4 == 0 and ldy % 4 == 0 and x_ptr % 16 == 0 and y_ptr % 16 == 0
+    return k % 4 == 0 and ldx % 4 == 0 and ldy % 4 == 0 and x_ptr % 16 == 0 and y_ptr % 16 == 0
 
 
 def rel_transform(x, w, y, r, k, f, device, image=None):
@@ -207,7 +204,7 @@ class RelPrologue:
                 nb, k, f = basis.shape
                 r = att.size(0)
                 image = None
-                nbytes = int(lib.gn_tc_gemm_rel_workspace_bytes(n_rows, r, f, k)) if GEMM_PATH != "ffma" and k % 4 == 0 else 0
+                nbytes = int(lib.gn_tc_gemm_rel_workspace_bytes(n_rows, r, f, k)) if k % 4 == 0 else 0
                 if nbytes and n_rows > 0:
                     image = _ws(nbytes, basis.device)
                     _lib.check(lib.gn_tc_rel_image(n_rows, r, f, k, w.data_ptr(), _ptr(image), nbytes, _stream()),
@@ -244,8 +241,8 @@ def weight_grad(a, b, out, device, c_inner=0, c_stride=0, force_tc=False):
     not apply (the caller then runs its FFMA product)."""
     lib = _lib.load()
     n, mo, no = a.n, a.f, b.f
-    ok = GEMM_PATH != "ffma" and n > 0 and mo % 4 == 0 and no % 4 == 0 and a.ld % 4 == 0 and b.ld % 4 == 0 and \
-        a.ptr % 16 == 0 and b.ptr % 16 == 0 and (force_tc or GEMM_PATH == "tc" or n >= _TC_TN_MIN_ROWS)
+    ok = n > 0 and mo % 4 == 0 and no % 4 == 0 and a.ld % 4 == 0 and b.ld % 4 == 0 and \
+        a.ptr % 16 == 0 and b.ptr % 16 == 0 and (force_tc or n >= _TC_TN_MIN_ROWS)
     if not ok:
         return False
     nbytes = int(lib.gn_tc_tn_workspace_bytes(n, mo, no))

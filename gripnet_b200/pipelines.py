@@ -7,8 +7,6 @@ forward/loss part of its ``train()`` (``:117-142``); ``AminerModel`` =
 a ``state_dict`` saved by the reference scripts loads unchanged.
 Used by ``bench.py``, ``__graft_entry__.smoke()`` and the parity tests.
 """
-import os
-
 import torch
 from torch.nn import Module, Parameter
 
@@ -18,10 +16,6 @@ from . import graph as G
 from . import ops, streams
 from .layers import homoGraph, interGraph
 from .losses import link_prediction_loss, node_classification_loss
-
-
-PROLOGUE = os.environ.get("GRIPNET_B200_PROLOGUE", "1") != "0"
-PREP_AT = os.environ.get("GRIPNET_B200_PREP_AT", "top")
 
 
 class PoseModel(Module):
@@ -64,27 +58,20 @@ class PoseModel(Module):
         # the decoder backward's (node, relation) structures depend on the edge lists only — the negatives' one is
         # rebuilt every step (GripNet-pose.py:131 resamples them).  The build is forked BEFORE the first kernel of the
         # step on a background-priority stream: its ~15 small kernels are roots of the captured graph, fill SM slots
-        # the dependency chain leaves idle, and are joined where they are consumed (the decoder's backward).
-        # PREP_AT = "first" forks it behind the first supervertex instead: the chain alone starts the step, but the
-        # build then ends ~30 us after the loss is ready and the backward waits for it (profiles/r02_v19_*).
-        prep = streams.Branch(background=PREP_AT == "top")
-
-        def fork_prep():
-            if torch.is_grad_enabled():
-                with prep(pos, neg, et):
-                    G.pair_struct(neg, et, n_dec, self.dmt.num_et if dctx is None else rel_n)
-                    G.pair_struct(pos, et, n_dec, self.dmt.num_et if dctx is None else rel_n)
+        # the dependency chain leaves idle, and are joined where they are consumed (the decoder's backward).  Forked
+        # behind the first supervertex instead, the build ends ~30 us after the loss is ready and the backward waits
+        # for it (profiles/r02_v19_*).
+        prep = streams.Branch(background=True)
+        if torch.is_grad_enabled():
+            with prep(pos, neg, et):
+                G.pair_struct(neg, et, n_dec, self.dmt.num_et if dctx is None else rel_n)
+                G.pair_struct(pos, et, n_dec, self.dmt.num_et if dctx is None else rel_n)
 
         def after_first():
             # W[r] / image of the relational layer: needed ~30 us after the first supervertex, so they are forked
             # behind it (two fewer launches ahead of the chain's first kernel)
-            if PROLOGUE:
-                self.dd.prologue(n_dec)
-            if PREP_AT != "top":
-                fork_prep()
+            self.dd.prologue(n_dec)
 
-        if PREP_AT == "top":
-            fork_prep()
         z = self.embed(data, after_first=after_first)
         # `prep` is NOT joined here: only the decoder's backward reads the structures (it joins the branch)
         if dctx is None:

@@ -32,20 +32,15 @@ parameter-only work.  A branch that is dropped un-joined joins itself first (``_
 holds are never released under running side work.  ``background=True`` puts a branch on a default-priority stream,
 below the high-priority stream the step's dependency chain is captured on (``capture.CapturedStep``).
 """
-import os
 import threading
 
 import torch
 
-ENABLED = os.environ.get("GRIPNET_B200_STREAMS", "1") != "0"
-# parameter-gradient branches may stay un-joined until the END of the autograd backward pass (see
-# ``Branch.join(deferrable=True)``); "0" joins every branch where it was forked
-DEFER_JOINS = os.environ.get("GRIPNET_B200_DEFER_JOINS", "1") != "0"
 # Stream priorities: the kernels of the step's dependency chain (and the branches that are joined straight back into
 # it) run on high-priority streams, parameter-gradient / structure-build branches ("background") on default-priority
 # ones, so a chain kernel that becomes ready while a wide weight-gradient kernel is in flight gets the next free SM
-# slots.  A captured graph keeps the priority of the stream each kernel was captured on.  "0" = one priority.
-PRIORITIES = os.environ.get("GRIPNET_B200_PRIORITIES", "1") != "0"
+# slots.  A captured graph keeps the priority of the stream each kernel was captured on.
+CHAIN_PRIORITY = -1
 _N_SIDE = 8
 _tls = threading.local()
 _pools = {}
@@ -69,13 +64,9 @@ def keep(*tensors):
         b._keep.extend(t for t in tensors if t is not None)
 
 
-def chain_priority():
-    return -1 if PRIORITIES else 0
-
-
 def _next_side(device, avoid=None, background=False):
     idx = device.index if device.index is not None else torch.cuda.current_device()
-    prio = 0 if background else chain_priority()
+    prio = 0 if background else CHAIN_PRIORITY
     with _pool_lock:
         pool = _pools.get((idx, prio))
         if pool is None:
@@ -101,7 +92,7 @@ class Branch:
     def __init__(self, enabled=True, background=False):
         """``background``: work nothing on the step's dependency chain waits for soon (parameter gradients, index
         structures of the backward, weight images): default-priority stream, below the chain's."""
-        self.enabled = bool(enabled) and ENABLED
+        self.enabled = bool(enabled)
         self._keep = []
         self._dirty = False
         self._args = ()
@@ -137,7 +128,7 @@ class Branch:
         that nothing reads before the backward pass ends (the caller has checked that autograd will only STORE
         them): the join is postponed to an autograd-engine callback that runs when the whole backward pass is
         done, so the dependency chain of the step never waits for weight-gradient kernels."""
-        if deferrable and self.enabled and self._dirty and self._parent is None and DEFER_JOINS and _defer(self):
+        if deferrable and self.enabled and self._dirty and self._parent is None and _defer(self):
             return
         self._join_now()
 

@@ -172,22 +172,18 @@ def test_distmult_forward_backward():
             assert rel_err(wc.grad, wr.grad) < TOL, (D, sig)
 
 
-@pytest.mark.parametrize("kernels", ["batch", "legacy"])
+@pytest.mark.parametrize("D", [80, 160])
 @pytest.mark.parametrize("n", [645, 3000])
-def test_distmult_pose_sized_and_pair(n, kernels, monkeypatch):
+def test_distmult_pose_sized_and_pair(n, D):
     """Pose-sized decoder call (n = 645 drugs x D = 80, 400 k edges) and a larger table, against float64;
     the fused pos/neg pair against two single calls (scores bit-identical; the pair adds the two lists' T
     before the products with w / z, two single calls add afterwards: gradients agree to rounding).
-    Both kernel families: the batch forms (32 edges / entries per warp step, the default) and the per-edge forms
-    (``GRIPNET_B200_DECODER_KERNELS=legacy``, also the path of widths the batch forms do not cover)."""
+    Both kernel families: D = 80 takes the batch forms (32 edges / entries per warp step, every float4 width up
+    to 128), D = 160 the per-edge / per-entry forms."""
     from gripnet_b200 import ops
-    if kernels == "legacy":
-        monkeypatch.setenv("GRIPNET_B200_DECODER_KERNELS", "legacy")
-    else:
-        monkeypatch.delenv("GRIPNET_B200_DECODER_KERNELS", raising=False)
     rs = np.random.RandomState(n)
     d = _dev()
-    D, r, e = 80, 16, 400_000
+    r, e = 16, 400_000
     z = torch.randn(n, D, dtype=torch.float64) * 0.3
     w = torch.randn(r, D, dtype=torch.float64)
     ei = torch.from_numpy(rs.randint(0, n, (2, e)))
