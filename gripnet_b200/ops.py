@@ -57,20 +57,21 @@ class Slot:
     NCCL all-gather (gathered row index == global node id)."""
     __slots__ = ("m", "full", "dctx", "halo")
 
-    def __init__(self, n_local, f, like, dctx=None, block=None, halo=None):
+    def __init__(self, m, full=None, dctx=None, halo=None):
+        """``Slot(m)`` wraps an existing local matrix that needs no gather; ``alloc`` makes a new slot."""
+        self.m, self.full = m, m if full is None else full
         self.dctx, self.halo = dctx, halo
+
+    @classmethod
+    def alloc(cls, n_local, f, like, dctx=None, block=None, halo=None):
         if dctx is None:
-            t = _new(n_local, f, like)
-            self.m, self.full = M(t), M(t)
-        elif halo is not None:
+            return cls(M(_new(n_local, f, like)))
+        if halo is not None:
             # halo-packed operand (graph.HaloPlan): own rows first, then only the referenced rows of each peer
             buf = dctx.slot_buffer(halo.rows, f, like, uniform=False)
-            self.full = M(buf)
-            self.m = M(buf[:n_local])
-        else:
-            buf = dctx.slot_buffer(dctx.world * block, f, like)
-            self.full = M(buf)
-            self.m = M(buf[dctx.rank * block: dctx.rank * block + n_local])
+            return cls(M(buf[:n_local]), M(buf), dctx, halo)
+        buf = dctx.slot_buffer(dctx.world * block, f, like)
+        return cls(M(buf[dctx.rank * block: dctx.rank * block + n_local]), M(buf), dctx)
 
     def gather(self):
         if self.dctx is not None:
@@ -269,6 +270,122 @@ def colsum(x, out):
 
 
 # ----------------------------------------------------------------------------
+# layer stacks: one autograd node per stack of GCN / RGCN layers.  With ``catout`` every H_l (H_0 = x) is a column
+# slice of one [n, sum(dims)] buffer, the stack's output; without it each H_l is a tensor of its own and H_L is the
+# output.
+# ----------------------------------------------------------------------------
+def _views(dims, catout, ts):
+    """M views of H_0 .. H_L, or of their gradients: the column slices of ``ts[0]`` with ``catout``, else ``ts``."""
+    if catout:
+        offs = [sum(dims[:i]) for i in range(len(dims))]
+        return [M(ts[0], offs[i], dims[i]) for i in range(len(dims))]
+    return [M(t) for t in ts]
+
+
+def _stack_input(x0, n_rows, nodes, catout, out_dims):
+    """``(x0, dims, buf, outs)``: the checked input, the widths of H_0 .. H_L, the catout buffer (or None) and the
+    views of the H_l that exist yet: all of them with ``catout``, else H_0 alone (the layer loop appends the rest)."""
+    x0 = _as_rows(x0, "x")
+    if x0.size(0) != n_rows:
+        raise RuntimeError(f"x has {x0.size(0)} rows but the graph has {n_rows} {nodes}")
+    dims = [x0.size(1)] + out_dims
+    if not catout:
+        return x0, dims, None, [M(x0)]
+    buf = _new(n_rows, sum(dims), x0)
+    return x0, dims, buf, _views(dims, True, [buf])
+
+
+def _stack_save(ctx, graph, relu_flags, catout, dims, params, n_per, buf, outs, saved):
+    """Keeps what ``_stack_backward`` reads (``saved``: the same number of tensors for every layer, layer by layer)
+    and returns the stack's output.  ``n_per``: parameters per layer, the bias last."""
+    ctx.graph, ctx.relu_flags, ctx.catout, ctx.dims = graph, relu_flags, catout, dims
+    ctx.has_bias = [b is not None for b in params[n_per - 1::n_per]]
+    ctx.param_refs = [None if p is None else weakref.ref(p) for p in params]
+    # outputs/intermediates go through save_for_backward (no ctx <-> output reference cycle)
+    acts = [buf] if catout else [o.t for o in outs]
+    ctx.n_acts = len(acts)
+    ctx.save_for_backward(*acts, *saved)
+    return buf if catout else outs[-1].t
+
+
+def _stack_backward(ctx, grad_out, n_per, n_dst, n_src, block, halo, layer_bwd):
+    """Backward of a layer stack, layer L down to 1, with ``n_per`` parameters per layer (the bias last).
+
+    Decided here for both stacks: which dZ_l lives in a gatherable slot, the bias gradient, and the slot dH_{l-1} is
+    produced into (``n_dst`` / ``n_src`` local rows, ``block`` rows per rank, halo plan ``halo``) together with the
+    concat-slice ``addend`` and the ReLU ``mask`` of layer l-1 applied to it.
+    ``layer_bwd(saved, need, dz, h_prev, dprev, addend, mask, br)`` launches the rest of one layer: the SpMM backward
+    from the slot ``dz``; the other parameter gradients flagged in ``need`` on the branch ``br``, returned in
+    parameter order; and, when ``dprev`` is not None, dH_{l-1} into ``dprev.m``.  ``saved``: the layer's tensors
+    kept by ``_stack_save``; ``h_prev``: the view of H_{l-1}."""
+    graph, relu_flags, catout, dims = ctx.graph, ctx.relu_flags, ctx.catout, ctx.dims
+    n_layers = len(relu_flags)
+    saved = ctx.saved_tensors
+    outs, per_layer = _views(dims, catout, saved[: ctx.n_acts]), saved[ctx.n_acts:]
+    g = _as_rows(grad_out, "grad")
+    dev = g.device
+    dctx = getattr(graph, "ctx", None)
+    gs = _views(dims, catout, [g])
+    dh = gs[-1]
+    grads = [None] * (n_per * n_layers)
+    need_db = [ctx.has_bias[i] and ctx.needs_input_grad[4 + n_per * i + n_per - 1] for i in range(n_layers)]
+    dz_slot = None            # set when `dh` already is a masked dZ living in a gatherable slot
+    dx0 = None
+    # bias / weight gradients leave the dependency chain dZ -> dY -> dH_{l-1}: side stream (a partitioned
+    # run all-reduces them on the caller's stream right away unless the reduction is deferred)
+    side = dctx is None or dctx.defer_grad_reduce
+    br = streams.Branch(enabled=side, background=True)
+    # bias sums on a branch of their own: ready before the SpMM, never queued behind a weight GEMM
+    br_b = streams.Branch(enabled=side, background=True) if any(need_db) else None
+    for l in range(n_layers, 0, -1):
+        f, k = dims[l], dims[l - 1]
+        p = n_per * (l - 1)                   # the layer's first parameter
+        h_prev = outs[l - 1]
+        if dz_slot is not None:
+            dz = dz_slot
+        elif relu_flags[l - 1]:
+            dz = Slot.alloc(n_dst, f, g, dctx, block, halo)
+            relu_bwd(dh, outs[l], dz.m)
+        elif dctx is not None:
+            dz = Slot.alloc(n_dst, f, g, dctx, block, halo)
+            map2d(_lib.EW_COPY, dh, dz.m)
+        else:
+            dz = Slot(dh)
+        if need_db[l - 1]:
+            db = torch.empty(f, dtype=torch.float32, device=dev)
+            with br_b(dz.m.t):
+                colsum(dz.m, db)
+            grads[p + n_per - 1] = _reduce(dctx, db)
+        dprev = addend = mask = None
+        if l > 1 or ctx.needs_input_grad[0]:
+            addend = gs[l - 1] if catout else None
+            mask = h_prev if (l > 1 and relu_flags[l - 2]) else None
+            # when dH_{l-1} is the next layer's dZ it is produced straight into that layer's gather slot
+            dprev = Slot.alloc(n_src, k, g, dctx if mask is not None else None, block, halo)
+        s = len(per_layer) // n_layers
+        grads[p: p + n_per - 1] = layer_bwd(per_layer[s * (l - 1): s * l], ctx.needs_input_grad[4 + p: 3 + p + n_per],
+                                            dz, h_prev, dprev, addend, mask, br)
+        dz_slot = dprev if mask is not None else None
+        if dprev is not None:
+            dh = dprev.m
+            if l == 1:
+                dx0 = dprev.m.t
+    defer = _only_stored(ctx, dctx)
+    if br_b is not None:
+        br_b.join(deferrable=defer)
+    br.join(deferrable=defer)
+    return (dx0, None, None, None) + tuple(grads)
+
+
+def _only_stored(ctx, dctx):
+    """May the parameter-gradient branch of this backward stay un-joined until the backward pass ends?"""
+    if dctx is not None and not dctx.defer_grad_reduce:
+        return False                      # the gradients are all-reduced right away
+    params = [None if r is None else r() for r in ctx.param_refs]
+    return streams.grads_only_stored(params, ctx.needs_input_grad[4:])
+
+
+# ----------------------------------------------------------------------------
 # GCN stack:  H_l = act_l( A_hat (H_{l-1} W_l) + b_l ),  optional concat of all H_l
 #   reference: myGCN.forward (layers.py:71-100) inside homoGraph.forward (:252-318)
 #   and interGraph.forward (:362-370, rectangular A_hat)
@@ -279,12 +396,9 @@ class GcnStack(torch.autograd.Function):
         n_layers = len(relu_flags)
         weights = [params[2 * l] for l in range(n_layers)]
         biases = [params[2 * l + 1] for l in range(n_layers)]
-        x0 = _as_rows(x0, "x")
-        if x0.size(0) != graph.n_src:
-            raise RuntimeError(f"x has {x0.size(0)} rows but the graph has {graph.n_src} source nodes")
         if catout and graph.n_src != graph.n_dst:
             raise RuntimeError("if_catout needs a square graph")
-        dims = [x0.size(1)] + [w.size(1) for w in weights]
+        x0, dims, buf, outs = _stack_input(x0, graph.n_src, "source nodes", catout, [w.size(1) for w in weights])
         for l, w in enumerate(weights):
             require_cuda(w, "weight", torch.float32)
             if w.size(0) != dims[l]:
@@ -292,130 +406,51 @@ class GcnStack(torch.autograd.Function):
         dev = x0.device
         dctx = getattr(graph, "ctx", None)
         b_src = graph.b_src if dctx is not None else None
-        outs = []      # M views of H_0 .. H_L
         br = streams.Branch()                  # no collective is ever issued inside a branch
-        if catout:
-            buf = _new(graph.n_dst, sum(dims), x0)
-            offs = [sum(dims[:i]) for i in range(len(dims))]
-            h0 = M(buf, offs[0], dims[0])
-            outs.append(h0)
-        else:
-            buf = None
-            outs.append(M(x0))
         for l in range(n_layers):
             w = weights[l].contiguous()
             k, f = dims[l], dims[l + 1]
-            y = Slot(graph.n_src, f, x0, dctx, b_src, getattr(graph, "fwd_halo", None))
+            y = Slot.alloc(graph.n_src, f, x0, dctx, b_src, getattr(graph, "fwd_halo", None))
             xin = M(x0) if l == 0 else outs[l]
             sgemm(False, False, graph.n_src, f, k, xin.ptr, xin.ld, w.data_ptr(), f, y.m.ptr, y.m.ld, dev)
             if l == 0 and catout:
                 with br(x0):                     # the concat copy of H_0 is off the chain (layer 0 reads x0 itself);
-                    map2d(_lib.EW_COPY, M(x0), h0)   # forked behind the first transform: the chain starts first
-            if catout:
-                hl = M(buf, offs[l + 1], f)
-            else:
-                hl = M(_new(graph.n_dst, f, x0))
+                    map2d(_lib.EW_COPY, M(x0), outs[0])   # forked behind the first transform: the chain starts first
+            if not catout:
+                outs.append(M(_new(graph.n_dst, f, x0)))
             b = biases[l].contiguous() if biases[l] is not None else None
-            spmm(graph.fwd, y.gather(), hl, f, bias=b, relu=relu_flags[l])
-            outs.append(hl)
+            spmm(graph.fwd, y.gather(), outs[l + 1], f, bias=b, relu=relu_flags[l])
         br.join()
-        ctx.graph, ctx.relu_flags, ctx.catout, ctx.dims = graph, relu_flags, catout, dims
-        ctx.has_bias = [b is not None for b in biases]
-        ctx.param_refs = [None if p is None else weakref.ref(p) for p in params]
-        ws = [w.contiguous() for w in weights]
-        # outputs/intermediates go through save_for_backward (no ctx <-> output reference cycle)
-        acts = [buf] if catout else [o.t for o in outs]
-        ctx.n_acts = len(acts)
-        ctx.save_for_backward(*acts, *ws)
-        return buf if catout else outs[-1].t
+        return _stack_save(ctx, graph, relu_flags, catout, dims, params, 2, buf, outs,
+                           [w.contiguous() for w in weights])
 
     @staticmethod
     def backward(ctx, grad_out):
-        graph, relu_flags, catout, dims = ctx.graph, ctx.relu_flags, ctx.catout, ctx.dims
-        n_layers = len(relu_flags)
-        saved = ctx.saved_tensors
-        acts, weights = saved[: ctx.n_acts], saved[ctx.n_acts:]
-        if catout:
-            offs0 = [sum(dims[:i]) for i in range(len(dims))]
-            outs = [M(acts[0], offs0[i], dims[i]) for i in range(len(dims))]
-        else:
-            outs = [M(a) for a in acts]
-        g = _as_rows(grad_out, "grad")
-        dev = g.device
+        graph = ctx.graph
         dctx = getattr(graph, "ctx", None)
-        b_dst = graph.b_dst if dctx is not None else None
-        bwd_halo = getattr(graph, "bwd_halo", None)
-        if catout:
-            offs = [sum(dims[:i]) for i in range(len(dims))]
-            gs = [M(g, offs[i], dims[i]) for i in range(len(dims))]
-            dh = gs[n_layers]
-        else:
-            gs = None
-            dh = M(g)
-        grads = [None] * (2 * n_layers)
-        dz_slot = None            # set when `dh` already is a masked dZ living in a gatherable slot
-        dx0 = None
-        # bias / weight gradients leave the dependency chain dZ -> dY -> dH_{l-1}: side stream (a partitioned
-        # run all-reduces them on the caller's stream right away unless the reduction is deferred)
-        br = streams.Branch(enabled=dctx is None or dctx.defer_grad_reduce, background=True)
-        br_b = streams.Branch(enabled=dctx is None or dctx.defer_grad_reduce, background=True)   # bias sums: ready before the SpMM,
-        for l in range(n_layers, 0, -1):                                        # never queued behind a weight GEMM
-            f, k = dims[l], dims[l - 1]
-            h_l, h_prev = outs[l], outs[l - 1]
-            if dz_slot is not None:
-                dz = dz_slot
-            elif relu_flags[l - 1]:
-                dz = Slot(graph.n_dst, f, g, dctx, b_dst, bwd_halo)
-                relu_bwd(dh, h_l, dz.m)
-            elif dctx is not None:
-                dz = Slot(graph.n_dst, f, g, dctx, b_dst, bwd_halo)
-                map2d(_lib.EW_COPY, dh, dz.m)
-            else:
-                dz = Slot.__new__(Slot)
-                dz.m, dz.full, dz.dctx = dh, dh, None
-            if ctx.has_bias[l - 1] and ctx.needs_input_grad[4 + 2 * (l - 1) + 1]:
-                db = torch.empty(f, dtype=torch.float32, device=dev)
-                with br_b(dz.m.t):
-                    colsum(dz.m, db)
-                grads[2 * (l - 1) + 1] = _reduce(dctx, db)
-            dy = M(_new(graph.n_src, f, g))
+
+        def layer(saved, need, dz, h_prev, dprev, addend, mask, br):
+            (w,) = saved
+            k, f, dev = h_prev.f, dz.m.f, dz.m.t.device
+            dy = M(_new(graph.n_src, f, dz.m.t))
             spmm(graph.bwd, dz.gather(), dy, f)
-            if ctx.needs_input_grad[4 + 2 * (l - 1)]:
+            dw = None
+            if need[0]:
                 dw = torch.empty((k, f), dtype=torch.float32, device=dev)
                 # dW = H_{l-1}^T dY : reduction over the node dimension -> deterministic split-K
                 with br(dy.t, h_prev.t):
                     if not weight_grad(h_prev, dy, dw, dev):
                         sgemm(True, False, k, f, graph.n_src, h_prev.ptr, h_prev.ld, dy.ptr, dy.ld, dw.data_ptr(),
                               f, dev)
-                grads[2 * (l - 1)] = _reduce(dctx, dw)
-            need_prev = (l > 1) or ctx.needs_input_grad[0]
-            dz_slot = None
-            if need_prev:
-                w = weights[l - 1]
-                addend = gs[l - 1] if catout else None
-                mask = h_prev if (l > 1 and relu_flags[l - 2]) else None
-                # dH_{l-1} = dY W^T (+ concat-slice grad) (masked by ReLU of layer l-1); when it is the
-                # next layer's dZ it is produced straight into that layer's gather slot
-                dprev = Slot(graph.n_src, k, g, dctx if mask is not None else None, b_dst, bwd_halo)
+                dw = _reduce(dctx, dw)
+            if dprev is not None:
+                # dH_{l-1} = dY W^T (+ concat-slice grad) (masked by ReLU of layer l-1)
                 sgemm(False, True, graph.n_src, k, f, dy.ptr, dy.ld, w.data_ptr(), f, dprev.m.ptr, dprev.m.ld, dev,
                       addend=addend, mask=mask)
-                dh = dprev.m
-                if mask is not None:
-                    dz_slot = dprev
-                if l == 1:
-                    dx0 = dprev.m.t
-        defer = _only_stored(ctx, dctx)
-        br_b.join(deferrable=defer)
-        br.join(deferrable=defer)
-        return (dx0, None, None, None) + tuple(grads)
+            return (dw,)
 
-
-def _only_stored(ctx, dctx):
-    """May the parameter-gradient branch of this backward stay un-joined until the backward pass ends?"""
-    if dctx is not None and not dctx.defer_grad_reduce:
-        return False                      # the gradients are all-reduced right away
-    params = [None if r is None else r() for r in ctx.param_refs]
-    return streams.grads_only_stored(params, ctx.needs_input_grad[4:])
+        return _stack_backward(ctx, grad_out, 2, graph.n_dst, graph.n_src, graph.b_dst if dctx is not None else None,
+                               getattr(graph, "bwd_halo", None), layer)
 
 
 # ----------------------------------------------------------------------------
@@ -430,29 +465,18 @@ class RgcnStack(torch.autograd.Function):
         att = [params[4 * l + 1] for l in range(n_layers)]
         root = [params[4 * l + 2] for l in range(n_layers)]
         bias = [params[4 * l + 3] for l in range(n_layers)]
-        x0 = _as_rows(x0, "x")
         n, r = graph.n_nodes, graph.n_rel
-        if x0.size(0) != n:
-            raise RuntimeError(f"x has {x0.size(0)} rows but the graph has {n} nodes")
-        dims = [x0.size(1)] + [rt.size(1) for rt in root]
+        x0, dims, buf, outs = _stack_input(x0, n, "nodes", catout, [rt.size(1) for rt in root])
         dev = x0.device
         dctx = getattr(graph, "ctx", None)
         blk = graph.b if dctx is not None else None
-        outs, ws_list = [], []
+        saved = []                             # (w, basis, att, root) of every layer
         br = streams.Branch()                  # no collective is ever issued inside a branch
         if catout:
-            buf = _new(n, sum(dims), x0)
-            offs = [sum(dims[:i]) for i in range(len(dims))]
-            h0 = M(buf, offs[0], dims[0])
             with br(x0):
-                map2d(_lib.EW_COPY, M(x0), h0)
-            outs.append(h0)
-        else:
-            buf = None
-            outs.append(M(x0))
+                map2d(_lib.EW_COPY, M(x0), outs[0])
         for l in range(n_layers):
             k, f = dims[l], dims[l + 1]
-            nb = basis[l].size(0)
             if att[l].size(0) != r:
                 raise RuntimeError("att rows must equal the number of relations of the graph")
             bs, at, rt = basis[l].contiguous(), att[l].contiguous(), root[l].contiguous()
@@ -461,7 +485,9 @@ class RgcnStack(torch.autograd.Function):
             pre = RelPrologue.take(basis[l], att[l], n_in)
             w, image = pre if pre is not None else (rel_weights(bs, at), None)
             xin = M(x0) if l == 0 else outs[l]
-            hl = M(buf, offs[l + 1], f) if catout else M(_new(n, f, x0))
+            if not catout:
+                outs.append(M(_new(n, f, x0)))
+            hl = outs[l + 1]
             # root term X root (layers.py:193), next to the relation transforms; the segmented mean
             # accumulates onto it
             with br(xin.t, rt, hl.t):
@@ -470,7 +496,7 @@ class RgcnStack(torch.autograd.Function):
             # Partitioned run: the NARROW layer input (k floats per node) is what crosses NVLink, and every
             # rank transforms all the gathered rows itself — R*f/k times fewer bytes exchanged than gathering Y
             if dctx is not None:
-                xs = Slot(n, k, x0, dctx, blk)
+                xs = Slot.alloc(n, k, x0, dctx, blk)
                 map2d(_lib.EW_COPY, xin, xs.m)
                 xall = xs.gather()
             else:
@@ -481,82 +507,34 @@ class RgcnStack(torch.autograd.Function):
             br.join()
             spmm(graph.fwd, M(yfull.view(yfull.size(0) * r, f)), hl, f, row_scale=graph.inv_cnt, bias=b, addend=hl,
                  relu=relu_flags[l])
-            outs.append(hl)
-            ws_list.append((w, bs, at, rt))
+            saved += (w, bs, at, rt)
         br.join()
-        ctx.graph, ctx.relu_flags, ctx.catout, ctx.dims = graph, relu_flags, catout, dims
-        ctx.has_bias = [b is not None for b in bias]
-        ctx.param_refs = [None if p is None else weakref.ref(p) for p in params]
-        acts = [buf] if catout else [o.t for o in outs]
-        ctx.n_acts = len(acts)
-        flat = [t for tup in ws_list for t in tup]
-        ctx.save_for_backward(*acts, *flat)
-        return buf if catout else outs[-1].t
+        return _stack_save(ctx, graph, relu_flags, catout, dims, params, 4, buf, outs, saved)
 
     @staticmethod
     def backward(ctx, grad_out):
-        graph, relu_flags, catout, dims = ctx.graph, ctx.relu_flags, ctx.catout, ctx.dims
-        n_layers = len(relu_flags)
+        graph = ctx.graph
         n, r = graph.n_nodes, graph.n_rel
-        saved = ctx.saved_tensors
-        acts, flat = saved[: ctx.n_acts], saved[ctx.n_acts:]
-        ws_list = [tuple(flat[4 * i: 4 * i + 4]) for i in range(n_layers)]
-        if catout:
-            offs0 = [sum(dims[:i]) for i in range(len(dims))]
-            outs = [M(acts[0], offs0[i], dims[i]) for i in range(len(dims))]
-        else:
-            outs = [M(a) for a in acts]
-        g = _as_rows(grad_out, "grad")
-        dev = g.device
         dctx = getattr(graph, "ctx", None)
-        blk = graph.b if dctx is not None else None
-        if catout:
-            offs = [sum(dims[:i]) for i in range(len(dims))]
-            gs = [M(g, offs[i], dims[i]) for i in range(len(dims))]
-            dh = gs[n_layers]
-        else:
-            gs = None
-            dh = M(g)
-        grads = [None] * (4 * n_layers)
-        dz_slot = None
-        dx0 = None
-        br = streams.Branch(enabled=dctx is None or dctx.defer_grad_reduce, background=True)   # parameter gradients off the chain
-        for l in range(n_layers, 0, -1):
-            f, k = dims[l], dims[l - 1]
-            w, bs, at, rt = ws_list[l - 1]
-            nb = bs.size(0)
-            h_l, h_prev = outs[l], outs[l - 1]
-            if dz_slot is not None:
-                dzs = dz_slot
-            elif relu_flags[l - 1]:
-                dzs = Slot(n, f, g, dctx, blk)
-                relu_bwd(dh, h_l, dzs.m)
-            elif dctx is not None:
-                dzs = Slot(n, f, g, dctx, blk)
-                map2d(_lib.EW_COPY, dh, dzs.m)
-            else:
-                dzs = Slot.__new__(Slot)
-                dzs.m, dzs.full, dzs.dctx = dh, dh, None
+
+        def layer(saved, need, dzs, h_prev, dprev, addend, mask, br):
+            w, bs, at, rt = saved
             dz = dzs.m
-            base = 4 + 4 * (l - 1)
-            if ctx.has_bias[l - 1] and ctx.needs_input_grad[base + 3]:
-                db = torch.empty(f, dtype=torch.float32, device=dev)
-                with br(dz.t):
-                    colsum(dz, db)
-                grads[4 * (l - 1) + 3] = _reduce(dctx, db)
+            k, f, nb, dev = h_prev.f, dz.f, bs.size(0), dz.t.device
             # dY[(j,r)] = sum_{e: src=j, rel=r} dZ[dst_e] / c_dst   (transpose CSR, atomic-free)
             dy = torch.empty((n * r, f), dtype=torch.float32, device=dev)
             spmm(graph.bwd, dzs.gather(), M(dy), f)
-            if ctx.needs_input_grad[base + 2]:
+            dbasis = datt = droot = None
+            if need[2]:
                 droot = torch.empty((k, f), dtype=torch.float32, device=dev)
                 with br(dz.t, h_prev.t):
                     sgemm(True, False, k, f, n, h_prev.ptr, h_prev.ld, dz.ptr, dz.ld, droot.data_ptr(), f, dev)
-                grads[4 * (l - 1) + 2] = _reduce(dctx, droot)
-            if ctx.needs_input_grad[base] or ctx.needs_input_grad[base + 1]:
+                droot = _reduce(dctx, droot)
+            if need[0] or need[1]:
                 # dW[r] = H_{l-1}^T dY[:, r, :]
                 dw = torch.empty((r, k, f), dtype=torch.float32, device=dev)
-                datt = torch.empty((r, nb), dtype=torch.float32, device=dev) if ctx.needs_input_grad[base + 1] else None
-                dbasis = torch.empty((nb, k, f), dtype=torch.float32, device=dev) if ctx.needs_input_grad[base] else None
+                datt = torch.empty((r, nb), dtype=torch.float32, device=dev) if need[1] else None
+                dbasis = torch.empty((nb, k, f), dtype=torch.float32, device=dev) if need[0] else None
                 with br(dy, h_prev.t, dw, bs, at):
                     # dW[r] = X^T dY[:, r, :] for all relations at once: one TN product on the tensor cores
                     if not weight_grad(h_prev, M(dy.view(n, r * f)), dw, dev, c_inner=f, c_stride=k * f,
@@ -570,27 +548,19 @@ class RgcnStack(torch.autograd.Function):
                         sgemm(True, False, nb, k * f, r, at.data_ptr(), nb, dw.data_ptr(), k * f, dbasis.data_ptr(),
                               k * f, dev)
                 if datt is not None:
-                    grads[4 * (l - 1) + 1] = _reduce(dctx, datt)
+                    datt = _reduce(dctx, datt)
                 if dbasis is not None:
-                    grads[4 * (l - 1)] = _reduce(dctx, dbasis)
-            need_prev = (l > 1) or ctx.needs_input_grad[0]
-            dz_slot = None
-            if need_prev:
-                addend = gs[l - 1] if catout else None
-                mask = h_prev if (l > 1 and relu_flags[l - 2]) else None
-                dps = Slot(n, k, g, dctx if mask is not None else None, blk)
-                dprev = dps.m
+                    dbasis = _reduce(dctx, dbasis)
+            if dprev is not None:
                 # dH_{l-1} = dZ root^T (+ concat grad), then += sum_r dY[:, r, :] W[r]^T, then ReLU mask
-                sgemm(False, True, n, k, f, dz.ptr, dz.ld, rt.data_ptr(), f, dprev.ptr, dprev.ld, dev, addend=addend)
-                sgemm(False, True, n, k, f, dy.data_ptr(), r * f, w.data_ptr(), f, dprev.ptr, dprev.ld, dev,
+                d = dprev.m
+                sgemm(False, True, n, k, f, dz.ptr, dz.ld, rt.data_ptr(), f, d.ptr, d.ld, dev, addend=addend)
+                sgemm(False, True, n, k, f, dy.data_ptr(), r * f, w.data_ptr(), f, d.ptr, d.ld, dev,
                       batch=r, sa=f, sb=k * f, sc=0, batch_reduce=True, accumulate=True, mask=mask)
-                dh = dprev
-                if mask is not None:
-                    dz_slot = dps
-                if l == 1:
-                    dx0 = dprev.t
-        br.join(deferrable=_only_stored(ctx, dctx))
-        return (dx0, None, None, None) + tuple(grads)
+            return dbasis, datt, droot
+
+        # the partitioned relational graph has no halo plan: its layer inputs and dZ are gathered as whole blocks
+        return _stack_backward(ctx, grad_out, 4, n, n, graph.b if dctx is not None else None, None, layer)
 
 
 # ----------------------------------------------------------------------------
