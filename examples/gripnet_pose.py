@@ -4,11 +4,13 @@
     python examples/gripnet_pose.py EPOCHS datasets/pose/pose-0.pt [--out out/pose-0]
     python examples/gripnet_pose.py EPOCHS --synthetic            # pose-0-shaped synthetic supergraph
     python examples/gripnet_pose.py EPOCHS --synthetic --rank     # + filtered test MRR / Hits@10 every epoch
+    python examples/gripnet_pose.py EPOCHS --synthetic --novel 100   # + the 100 best new drug pairs per side effect
 
 Same model (``GripNet-pose.py:86-99``), optimiser (Adam, lr 0.01, ``:104``), per-epoch negative sampling
 (``:131``), loss (``:140-142``) and per-relation AUPRC / AUROC / AP@all records (``:148-164``, ``:174-199``) —
 but an epoch is ONE CUDA-graph replay (``training.PoseTrainer``) and the evaluation never leaves the device.
-Writes ``<out>-model.pt`` (``state_dict``, the reference's key names) and ``<out>-record.pt``.
+Writes ``<out>-model.pt`` (``state_dict``, the reference's key names) and ``<out>-record.pt``; with ``--novel K``
+also ``<out>-novel.pt``.
 """
 import argparse
 import os
@@ -31,6 +33,10 @@ def main():
                     help="also print the filtered test MRR and Hits@10 (all drugs as candidate tails, train + test "
                          "positives filtered) and the filtered test relation MRR and Hits@10 (all side effects as "
                          "candidates of each drug pair), macro-averaged over relations")
+    ap.add_argument("--novel", type=int, metavar="K", default=0,
+                    help="after training, write <out>-novel.pt: the K (<= 256) most likely drug pairs {s, t} of every "
+                         "side effect that are not train or test positives in either direction (scores after the "
+                         "sigmoid, src < dst, each [R, K])")
     args = ap.parse_args()
 
     from gripnet_b200 import data as gd, metrics, ranking, utils
@@ -91,6 +97,16 @@ def main():
         rec["test_rank_record"] = rank_rec.cpu()             # [epochs, 2 (mrr, hits@10), R]
         rec["test_relation_rank_record"] = rel_rank_rec.cpu()   # [epochs, 2 (mrr, hits@10), R]
     torch.save(rec, args.out + "-record.pt")
+    if args.novel:
+        pos = [(train["dd_edge_index"], train["dd_edge_type"]), (test["dd_edge_index"], test["dd_edge_type"])]
+        filt = ranking.EdgeFilter(pos, test["n_d"], n_rel)
+        with torch.no_grad():
+            scores, src, dst = model.dmt.topk_pairs(trainer.z.detach(), torch.arange(n_rel, device=dev), args.novel,
+                                                    filter=filt)
+        torch.save({"scores": scores.cpu(), "src": src.cpu(), "dst": dst.cpu()}, args.out + "-novel.pt")
+        print("side effect 0, best new pairs: " + ", ".join(
+            "({}, {}) {:0.4f}".format(a, b, v) for a, b, v in zip(src[0, :5].tolist(), dst[0, :5].tolist(),
+                                                                  scores[0, :5].tolist())))
 
 
 if __name__ == "__main__":

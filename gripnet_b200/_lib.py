@@ -130,6 +130,9 @@ SIGNATURES = {
     "gn_rank_pair_rows": (_INT, [_P, _I64, _I32, _P, _P, _P, _P, _I64, _P, _I64, _P]),
     "gn_rank_pair_count": (_INT, [_P, _I64, _I32, _I32, _P, _P, _P, _P, _P, _P, _P, _P]),
     "gn_rank_pair_topk": (_INT, [_P, _I64, _I32, _I64, _P, _P, _P, _I32, _INT, _P, _P, _P]),
+    "gn_rank_rel_pairs_workspace_bytes": (_SZ, [_I64, _I32, _I32]),
+    "gn_rank_rel_pairs_select": (_INT, [_P, _I64, _I32, _P, _I32, _I32, _P, _I64, _P, _P, _I32, _P, _SZ, _P]),
+    "gn_rank_rel_pairs_merge": (_INT, [_P, _SZ, _I32, _I64, _I32, _INT, _P, _P, _P, _P]),
     "gn_peer_max_world": (_INT, []),
     "gn_peer_allgather": (_INT, [_P, _I32, _I32, _I64, _I64, _I64, _I32, _P, _P, _P, _P]),
     "gn_peer_halo_grid": (_INT, []),

@@ -272,11 +272,15 @@ __global__ void __launch_bounds__(kMetricThreads) rank_metrics_kernel(const floa
 // entry overwritten with kMaskedBits first) has key 0.  The k-th largest key is found by an MSB-first radix select
 // (8 passes of 8 bits over the row, read from L1 / L2), the keys at or above it are gathered and bitonic-sorted.
 // ---------------------------------------------------------------------------------------------------------------
+__device__ __forceinline__ uint64_t score_key(uint32_t b, uint32_t id) {
+  const uint32_t u = (b & 0x80000000u) ? ~b : (b | 0x80000000u);
+  return (uint64_t(u) << 32) | uint64_t(~id);
+}
+
 __device__ __forceinline__ uint64_t topk_key(const float* srow, int c) {
   const uint32_t b = __float_as_uint(srow[c]);
   if (b == kMaskedBits) return 0ull;
-  const uint32_t u = (b & 0x80000000u) ? ~b : (b | 0x80000000u);
-  return (uint64_t(u) << 32) | uint64_t(~uint32_t(c));
+  return score_key(b, uint32_t(c));
 }
 
 __device__ __forceinline__ float topk_score(uint64_t key) {
@@ -284,43 +288,19 @@ __device__ __forceinline__ float topk_score(uint64_t key) {
   return __uint_as_float((u & 0x80000000u) ? (u & 0x7fffffffu) : ~u);
 }
 
-// the filter row of query row qi (-1: none): s*R + r of a tail query, the looked-up pair row of a relation query
-struct TailFilterRow {
-  const int64_t* node;
-  const int64_t* rel;
-  int32_t n_rel;
-  bool filtered;
-  __device__ __forceinline__ int64_t operator()(int64_t qi) const { return filtered ? node[qi] * n_rel + rel[qi] : -1; }
-};
-
-struct PairFilterRow {
-  const int32_t* f_row;       // nullptr: no filter
-  __device__ __forceinline__ int64_t operator()(int64_t qi) const { return f_row ? f_row[qi] : -1; }
-};
-
-template <class FilterRow>
-__global__ void __launch_bounds__(kTopkThreads) rank_topk_kernel(float* __restrict__ S, int64_t lds, int32_t n,
-                                                                 const FilterRow filter_row,
-                                                                 const int32_t* __restrict__ f_rowptr,
-                                                                 const int32_t* __restrict__ f_dst, int k, int sigmoid,
-                                                                 float* __restrict__ out_score,
-                                                                 int64_t* __restrict__ out_id) {
+// The k (<= kTopkMax) largest non-zero keys among keys(0 .. m-1), sorted descending into the returned shared array
+// of kTopkMax slots (0 past the last one).  Block-wide, kTopkThreads threads; keys(c) is read several times.
+template <class Keys>
+__device__ __forceinline__ const uint64_t* topk_select(const Keys& keys, int m, int k) {
   __shared__ int hist[256];
   __shared__ uint64_t sel[kTopkMax];
   __shared__ int warp_cnt[kTopkThreads / 32];
   __shared__ uint64_t prefix_s;
   __shared__ int remaining_s, n_sel;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int64_t qi = blockIdx.x;
-  float* srow = S + qi * lds;
-  const int64_t row = filter_row(qi);
-  if (row >= 0) {
-    for (int j = f_rowptr[row] + tid; j < f_rowptr[row + 1]; j += kTopkThreads) srow[f_dst[j]] = __uint_as_float(kMaskedBits);
-  }
-  __syncthreads();
   // admissible candidates
   int a = 0;
-  for (int c = tid; c < n; c += kTopkThreads) a += topk_key(srow, c) != 0ull;
+  for (int c = tid; c < m; c += kTopkThreads) a += keys(c) != 0ull;
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) a += __shfl_xor_sync(kFull, a, o);
   if (lane == 0) warp_cnt[warp] = a;
@@ -339,8 +319,8 @@ __global__ void __launch_bounds__(kTopkThreads) rank_topk_kernel(float* __restri
       hist[tid] = 0;
       __syncthreads();
       const uint64_t prefix = prefix_s;
-      for (int c = tid; c < n; c += kTopkThreads) {
-        const uint64_t key = topk_key(srow, c);
+      for (int c = tid; c < m; c += kTopkThreads) {
+        const uint64_t key = keys(c);
         if (key != 0ull && (key & mask) == prefix) atomicAdd(&hist[int(key >> shift) & 255], 1);
       }
       __syncthreads();
@@ -383,8 +363,8 @@ __global__ void __launch_bounds__(kTopkThreads) rank_topk_kernel(float* __restri
   if (tid == 0) n_sel = 0;
   sel[tid] = 0ull;
   __syncthreads();
-  for (int c = tid; c < n; c += kTopkThreads) {
-    const uint64_t key = topk_key(srow, c);
+  for (int c = tid; c < m; c += kTopkThreads) {
+    const uint64_t key = keys(c);
     if (key != 0ull && key >= thresh) {
       const int at = atomicAdd(&n_sel, 1);
       if (at < kTopkMax) sel[at] = key;
@@ -406,17 +386,185 @@ __global__ void __launch_bounds__(kTopkThreads) rank_topk_kernel(float* __restri
       __syncthreads();
     }
   }
+  return sel;
+}
+
+// the returned score of a selected key (NaN for an empty slot), after the sigmoid when `sigmoid`
+__device__ __forceinline__ float topk_out_score(uint64_t key, int sigmoid) {
+  float v = __uint_as_float(0x7fc00000u);
+  if (key != 0ull) {
+    v = topk_score(key);
+    if (sigmoid) v = 1.0f / (1.0f + expf(-v));
+  }
+  return v;
+}
+
+// the filter row of query row qi (-1: none): s*R + r of a tail query, the looked-up pair row of a relation query
+struct TailFilterRow {
+  const int64_t* node;
+  const int64_t* rel;
+  int32_t n_rel;
+  bool filtered;
+  __device__ __forceinline__ int64_t operator()(int64_t qi) const { return filtered ? node[qi] * n_rel + rel[qi] : -1; }
+};
+
+struct PairFilterRow {
+  const int32_t* f_row;       // nullptr: no filter
+  __device__ __forceinline__ int64_t operator()(int64_t qi) const { return f_row ? f_row[qi] : -1; }
+};
+
+struct RowKeys {
+  const float* srow;
+  __device__ __forceinline__ uint64_t operator()(int c) const { return topk_key(srow, c); }
+};
+
+template <class FilterRow>
+__global__ void __launch_bounds__(kTopkThreads) rank_topk_kernel(float* __restrict__ S, int64_t lds, int32_t n,
+                                                                 const FilterRow filter_row,
+                                                                 const int32_t* __restrict__ f_rowptr,
+                                                                 const int32_t* __restrict__ f_dst, int k, int sigmoid,
+                                                                 float* __restrict__ out_score,
+                                                                 int64_t* __restrict__ out_id) {
+  const int tid = threadIdx.x;
+  const int64_t qi = blockIdx.x;
+  float* srow = S + qi * lds;
+  const int64_t row = filter_row(qi);
+  if (row >= 0) {
+    for (int j = f_rowptr[row] + tid; j < f_rowptr[row + 1]; j += kTopkThreads) srow[f_dst[j]] = __uint_as_float(kMaskedBits);
+  }
+  __syncthreads();
+  const uint64_t* sel = topk_select(RowKeys{srow}, n, k);
   if (tid < k) {
     const uint64_t key = sel[tid];
-    float v = __uint_as_float(0x7fc00000u);
-    int64_t id = -1;
-    if (key != 0ull) {
-      v = topk_score(key);
-      if (sigmoid) v = 1.0f / (1.0f + expf(-v));
-      id = int64_t(~uint32_t(key));
+    out_score[qi * k + tid] = topk_out_score(key, sigmoid);
+    out_id[qi * k + tid] = key != 0ull ? int64_t(~uint32_t(key)) : -1;
+  }
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// top-k new pairs of a relation (?, r, ?): candidates are the unordered pairs {s, t}, s < t, scored with
+// S = sum_k z[s,k] w[r,k] z[t,k] and keyed as in the top-k above with id s*n + t.  Stage 1, one block per (query,
+// tile of kPairTile s rows): 64 x 64 score tiles of the triangle t > s by register-blocked FFMA (a 4 x 4 block per
+// thread, operands staged through shared memory in chunks of kPairKc features), never written out.  Scores whose
+// key beats the block's running threshold are tested against row s*R + r of the symmetrised filter (binary search)
+// and pushed to a shared buffer; when the buffer cannot take another tile it is cut to its top k by topk_select
+// and the threshold rises to the k-th key.  Each block writes its sorted top k keys; stage 2 (one block per query)
+// selects the top k of its tiles' keys and decodes them.
+// ---------------------------------------------------------------------------------------------------------------
+constexpr int kPairTile = 64;
+constexpr int kPairKc = 8;
+constexpr int kPairTileKeys = kPairTile * kPairTile;
+constexpr int kPairBuf = kPairTileKeys + 1024;      // room for one tile above a cut buffer (k <= kTopkMax < 1024)
+
+__device__ __forceinline__ bool pair_filtered(const int32_t* __restrict__ f_rowptr, const int32_t* __restrict__ f_dst,
+                                              int64_t row, int32_t t) {
+  int lo = f_rowptr[row];
+  const int end = f_rowptr[row + 1];
+  int hi = end;
+  while (lo < hi) {
+    const int mid = lo + ((hi - lo) >> 1);
+    if (f_dst[mid] < t) lo = mid + 1;
+    else hi = mid;
+  }
+  return lo < end && f_dst[lo] == t;
+}
+
+struct BufKeys {
+  const uint64_t* buf;
+  __device__ __forceinline__ uint64_t operator()(int c) const { return buf[c]; }
+};
+
+__global__ void __launch_bounds__(kTopkThreads) rank_rel_pairs_select_kernel(
+    const float* __restrict__ z, int64_t ldz, int D, const float* __restrict__ w, int32_t n_rel, int32_t n,
+    const int64_t* __restrict__ rel, int64_t count, int n_tiles, const int32_t* __restrict__ f_rowptr,
+    const int32_t* __restrict__ f_dst, int k, uint64_t* __restrict__ keys_out) {
+  __shared__ __align__(16) float As[kPairKc][kPairTile + 4];
+  __shared__ __align__(16) float Bs[kPairKc][kPairTile + 4];
+  __shared__ uint64_t buf[kPairBuf];
+  __shared__ int n_buf;
+  __shared__ uint64_t thr_s;
+  const int tid = threadIdx.x, ty = tid >> 4, tx = tid & 15;
+  // heavy tiles (small s) first: block b is tile b / count of query b % count
+  const int tile = int(blockIdx.x / count);
+  const int64_t qi = int64_t(blockIdx.x) - int64_t(tile) * count;
+  const int64_t r = rel[qi];
+  const float* wr = w + r * D;
+  const int s0 = tile * kPairTile;
+  if (tid == 0) {
+    n_buf = 0;
+    thr_s = 0ull;
+  }
+  for (int t0 = s0; t0 < n; t0 += kPairTile) {
+    float acc[4][4];
+#pragma unroll
+    for (int i = 0; i < 4; ++i)
+#pragma unroll
+      for (int j = 0; j < 4; ++j) acc[i][j] = 0.0f;
+    for (int kc = 0; kc < D; kc += kPairKc) {
+      __syncthreads();
+#pragma unroll
+      for (int e = tid; e < kPairTile * kPairKc; e += kTopkThreads) {
+        const int row = e / kPairKc, kk = e - row * kPairKc, f = kc + kk;
+        const int s = s0 + row, t = t0 + row;
+        As[kk][row] = (s < n && f < D) ? z[int64_t(s) * ldz + f] * wr[f] : 0.0f;
+        Bs[kk][row] = (t < n && f < D) ? z[int64_t(t) * ldz + f] : 0.0f;
+      }
+      __syncthreads();
+#pragma unroll
+      for (int kk = 0; kk < kPairKc; ++kk) {
+        const float4 a = *reinterpret_cast<const float4*>(&As[kk][ty * 4]);
+        const float4 b = *reinterpret_cast<const float4*>(&Bs[kk][tx * 4]);
+        const float av[4] = {a.x, a.y, a.z, a.w}, bv[4] = {b.x, b.y, b.z, b.w};
+#pragma unroll
+        for (int i = 0; i < 4; ++i)
+#pragma unroll
+          for (int j = 0; j < 4; ++j) acc[i][j] = fmaf(av[i], bv[j], acc[i][j]);
+      }
     }
-    out_score[qi * k + tid] = v;
-    out_id[qi * k + tid] = id;
+    const uint64_t thr = thr_s;
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+      const int s = s0 + ty * 4 + i;
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        const int t = t0 + tx * 4 + j;
+        if (s >= n || t >= n || t <= s) continue;
+        const uint64_t key = score_key(__float_as_uint(acc[i][j]), uint32_t(s * n + t));
+        if (key <= thr) continue;
+        if (f_rowptr != nullptr && pair_filtered(f_rowptr, f_dst, int64_t(s) * n_rel + r, t)) continue;
+        buf[atomicAdd(&n_buf, 1)] = key;
+      }
+    }
+    __syncthreads();
+    const int m = n_buf;
+    if (m > kPairBuf - kPairTileKeys) {                  // block-uniform: cut to the top k, raise the threshold
+      const uint64_t* sel = topk_select(BufKeys{buf}, m, k);
+      if (tid < k) buf[tid] = sel[tid];
+      if (tid == 0) {
+        n_buf = k;
+        thr_s = sel[k - 1];
+      }
+    }
+  }
+  __syncthreads();
+  const uint64_t* sel = topk_select(BufKeys{buf}, n_buf, k);
+  if (tid < k) keys_out[(qi * n_tiles + tile) * k + tid] = sel[tid];
+}
+
+__global__ void __launch_bounds__(kTopkThreads) rank_rel_pairs_merge_kernel(const uint64_t* __restrict__ keys,
+                                                                            int m, int32_t n, int k, int sigmoid,
+                                                                            float* __restrict__ out_score,
+                                                                            int64_t* __restrict__ out_src,
+                                                                            int64_t* __restrict__ out_dst) {
+  const int tid = threadIdx.x;
+  const int64_t qi = blockIdx.x;
+  const uint64_t* sel = topk_select(BufKeys{keys + qi * m}, m, k);
+  if (tid < k) {
+    const uint64_t key = sel[tid];
+    const int64_t id = key != 0ull ? int64_t(~uint32_t(key)) : -1;
+    out_score[qi * k + tid] = topk_out_score(key, sigmoid);
+    out_src[qi * k + tid] = id >= 0 ? id / n : -1;
+    out_dst[qi * k + tid] = id >= 0 ? id % n : -1;
   }
 }
 
@@ -611,6 +759,42 @@ int gn_rank_pair_topk(float* S, int64_t lds, int32_t n_rel, int64_t count, const
   const PairFilterRow frow{f_row};
   GN_LAUNCH(rank_topk_kernel<PairFilterRow>, (unsigned)count, kTopkThreads, 0, as_stream(stream), S, lds, n_rel, frow,
             f_rowptr, f_rel, k, sigmoid, out_score, out_id);
+  return GN_OK;
+}
+
+static int rel_pairs_tiles(int32_t n_nodes) { return int(ceil_div(n_nodes, kPairTile)); }
+
+size_t gn_rank_rel_pairs_workspace_bytes(int64_t count, int32_t n_nodes, int32_t k) {
+  if (count <= 0 || n_nodes <= 0 || k <= 0) return 256;
+  return align_up(size_t(count) * size_t(rel_pairs_tiles(n_nodes)) * size_t(k) * 8);
+}
+
+int gn_rank_rel_pairs_select(const float* z, int64_t ldz, int32_t D, const float* w, int32_t n_rel, int32_t n_nodes,
+                             const int64_t* rel, int64_t count, const int32_t* f_rowptr, const int32_t* f_dst,
+                             int32_t k, void* ws, size_t ws_bytes, void* stream) {
+  if (count < 0 || D <= 0 || n_rel <= 0 || n_nodes <= 0 || ldz < D || k < 1 || k > kTopkMax) return GN_ERR_ARG;
+  if (int64_t(n_nodes) * n_nodes >= (int64_t(1) << 31) || int64_t(n_nodes) * n_rel >= (int64_t(1) << 31))
+    return GN_ERR_RANGE;
+  if (count == 0) return GN_OK;
+  const int n_tiles = rel_pairs_tiles(n_nodes);
+  if (count * n_tiles >= (int64_t(1) << 31)) return GN_ERR_RANGE;
+  if (!z || !w || !rel || (f_rowptr && !f_dst)) return GN_ERR_ARG;
+  if (!ws || ws_bytes < gn_rank_rel_pairs_workspace_bytes(count, n_nodes, k)) return GN_ERR_WORKSPACE;
+  GN_LAUNCH(rank_rel_pairs_select_kernel, (unsigned)(count * n_tiles), kTopkThreads, 0, as_stream(stream), z, ldz, D,
+            w, n_rel, n_nodes, rel, count, n_tiles, f_rowptr, f_dst, k, static_cast<uint64_t*>(ws));
+  return GN_OK;
+}
+
+int gn_rank_rel_pairs_merge(const void* ws, size_t ws_bytes, int32_t n_nodes, int64_t count, int32_t k, int sigmoid,
+                            float* out_score, int64_t* out_src, int64_t* out_dst, void* stream) {
+  if (count < 0 || n_nodes <= 0 || k < 1 || k > kTopkMax) return GN_ERR_ARG;
+  if (count == 0) return GN_OK;
+  if (count >= (int64_t(1) << 31)) return GN_ERR_RANGE;
+  if (!out_score || !out_src || !out_dst) return GN_ERR_ARG;
+  if (!ws || ws_bytes < gn_rank_rel_pairs_workspace_bytes(count, n_nodes, k)) return GN_ERR_WORKSPACE;
+  GN_LAUNCH(rank_rel_pairs_merge_kernel, (unsigned)count, kTopkThreads, 0, as_stream(stream),
+            static_cast<const uint64_t*>(ws), rel_pairs_tiles(n_nodes) * k, n_nodes, k, sigmoid, out_score, out_src,
+            out_dst);
   return GN_OK;
 }
 

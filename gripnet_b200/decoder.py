@@ -48,6 +48,12 @@ class multiRelaInnerProductDecoder(Module):
         ``ranking.topk_relations``.  No gradient flows through it."""
         return ranking.topk_relations(z, self.weight, src, dst, k, filter=filter, sigmoid=sigmoid)
 
+    def topk_pairs(self, z, rel, k, filter=None, sigmoid=True):
+        """The ``k`` most likely new unordered pairs ``{s, t}`` (``s < t``) of every relation ``rel[i]`` under this
+        decoder's weight, skipping the pairs ``filter`` holds in either direction: ``(scores [Q, k], src int64 [Q, k],
+        dst int64 [Q, k])`` — ``ranking.topk_pairs``.  No gradient flows through it."""
+        return ranking.topk_pairs(z, self.weight, rel, k, filter=filter, sigmoid=sigmoid)
+
     def reset_parameters(self):
         with torch.no_grad():
             self.weight.normal_(std=1.0 / math.sqrt(self.in_dim))          # decoder.py:25-26

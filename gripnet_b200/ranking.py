@@ -36,6 +36,20 @@ Relation queries ``(s, ?, t)`` of a directed pair (``RelationRanker``, ``topk_re
 * ``P`` is bitwise symmetric (fp32 products commute): ``(s, t)`` and ``(t, s)`` give identical score rows whenever
   both rows take the same product path (the same chunk, hence the same dense-product kernel).
 
+Pair queries ``(?, r, ?)`` of a relation (``topk_pairs``: "which new drug pairs does the model predict for side effect
+``r``?") score every unordered node pair; the kernels score tiles of the triangle and keep only the best keys, so the
+``[n, n]`` score matrix of a relation is never written:
+
+* candidates are the unordered pairs ``{s, t}`` with ``s < t``: DistMult is symmetric in ``s`` and ``t``, so ``(s, t)``
+  and ``(t, s)`` are one prediction, and a self-pair is not an interaction; there is no ordered or self-pair mode;
+* ``S(s, t) = sum_k z[s,k] w[r,k] z[t,k]``, pre-sigmoid, as above;
+* the filter is the same ``EdgeFilter``: ``{s, t}`` is excluded for ``r`` when ``(s, r, t)`` OR ``(t, r, s)`` is in it;
+* order: descending pre-sigmoid score, ties by the smaller ``s``, then the smaller ``t`` (the smaller pair id
+  ``s * n + t``); ids ``-1`` / score NaN pad a query with fewer than ``k`` admissible pairs (e.g. ``n < 2``);
+  ``sigmoid`` applies to the returned scores;
+* ``1 <= k <= 256`` and ``n * n < 2^31`` (the pair id is the low word of the 64-bit selection key); the work grows as
+  ``Q * n^2 * D``.
+
 Single GPU: a partitioned ``z`` is gathered by the caller first (``parallel.all_gather_rows``).
 """
 import ctypes
@@ -132,7 +146,8 @@ class EdgeFilter:
     and sorted by ``c``.  ``edge_lists``: a sequence of ``(edge_index int64 [2, E], edge_type int64 [E])`` on one
     CUDA device.  Built once; reusable by any number of rankers and top-k calls of the same graph.  The first
     relation query that uses the filter (``RelationRanker``, ``topk_relations``) also builds its pair-grouped view
-    from the same edge lists (the filter keeps references to them) and caches it here."""
+    from the same edge lists (the filter keeps references to them) and caches it here; the first pair query
+    (``topk_pairs``) likewise builds and caches a symmetrised view."""
 
     def __init__(self, edge_lists, num_nodes, num_relations):
         self.num_nodes, self.num_relations = _sizes(num_nodes, num_relations)
@@ -148,6 +163,7 @@ class EdgeFilter:
         self._g = _Grouped(ei, et, self.num_nodes, self.num_relations, groups=False)
         self._lists = lists
         self._p = None
+        self._s = None
 
     def _check(self, n, r, device):
         if (n, r) != (self.num_nodes, self.num_relations) or device != self.device:
@@ -163,6 +179,16 @@ class EdgeFilter:
             et = torch.cat([l[1] for l in lists]) if len(lists) > 1 else lists[0][1]
             self._p = _Paired(ei, et, self.num_nodes, self.num_relations)
         return self._p
+
+    def _symmetric(self, n, r, device):
+        """The grouped view (``_Grouped``) of the filter's triples and their flipped copies, built on first use: row
+        ``s * R + r`` holds every ``t`` with ``(s, r, t)`` or ``(t, r, s)`` in the filter, sorted."""
+        self._check(n, r, device)
+        if self._s is None:
+            ei = torch.cat([l[0] for l in self._lists] + [l[0].flip(0) for l in self._lists], dim=1)
+            et = torch.cat([l[1] for l in self._lists] * 2)
+            self._s = _Grouped(ei, et, self.num_nodes, self.num_relations, groups=False)
+        return self._s
 
 
 def _embeddings(z, weight, n=None, r=None):
@@ -435,3 +461,38 @@ def topk_relations(z, weight, src, dst, k, filter=None, sigmoid=True):
                                          _ptr(f.rel) if f is not None else None, k, int(bool(sigmoid)),
                                          _ptr(scores[q0:]), _ptr(ids[q0:]), _stream()), "gn_rank_pair_topk")
     return scores, ids
+
+
+def topk_pairs(z, weight, rel, k, filter=None, sigmoid=True):
+    """The ``k`` (1..256) most likely unordered pairs ``{s, t}``, ``s < t``, of every relation query ``rel[i]`` with
+    neither ``(s, rel[i], t)`` nor ``(t, rel[i], s)`` in ``filter``: ``(scores float32 [Q, k], src int64 [Q, k],
+    dst int64 [Q, k])`` with ``src < dst``, descending pre-sigmoid score, ties by smaller ``src`` then smaller
+    ``dst``; scores after the sigmoid when ``sigmoid``; ids -1 / score NaN where fewer than ``k`` pairs are left.
+    ``rel`` may repeat a relation.  Needs ``n * n < 2^31``.  After the filter's symmetrised view exists (first use),
+    a call reads nothing back to the host and can be captured in a CUDA graph."""
+    lib = _lib.load()
+    z, w = _embeddings(z, weight)
+    n, r = _sizes(z.size(0), w.size(0))
+    if n * n >= 2 ** 31:
+        raise RuntimeError(f"gripnet_b200: topk_pairs needs num_nodes^2 < 2^31 (pair ids), got {n} nodes")
+    dev = z.device
+    k = _k_arg(k)
+    rel = rel if torch.is_tensor(rel) else torch.as_tensor(rel, dtype=torch.int64, device=dev)
+    require_cuda(rel, "rel", torch.int64)
+    rel = rel.contiguous().view(-1)
+    validate_index(rel, r, "rel")
+    f = filter._symmetric(n, r, dev) if filter is not None else None
+    nq = rel.numel()
+    scores = torch.empty((nq, k), dtype=torch.float32, device=dev)
+    src = torch.empty((nq, k), dtype=torch.int64, device=dev)
+    dst = torch.empty((nq, k), dtype=torch.int64, device=dev)
+    if nq == 0:
+        return scores, src, dst
+    ws = _ws(lib.gn_rank_rel_pairs_workspace_bytes(nq, n, k), dev)
+    _lib.check(lib.gn_rank_rel_pairs_select(z.data_ptr(), ops._ldz(z), z.size(1), w.data_ptr(), r, n, _ptr(rel), nq,
+                                            _ptr(f.rowptr) if f is not None else None,
+                                            _ptr(f.dst) if f is not None else None, k, _ptr(ws), ws.numel(),
+                                            _stream()), "gn_rank_rel_pairs_select")
+    _lib.check(lib.gn_rank_rel_pairs_merge(_ptr(ws), ws.numel(), n, nq, k, int(bool(sigmoid)), _ptr(scores), _ptr(src),
+                                           _ptr(dst), _stream()), "gn_rank_rel_pairs_merge")
+    return scores, src, dst

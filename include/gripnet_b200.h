@@ -468,6 +468,27 @@ int gn_rank_pair_topk(float* S, int64_t lds, int32_t n_rel, int64_t count, const
                       const int32_t* f_rowptr, const int32_t* f_rel, int32_t k, int sigmoid, float* out_score,
                       int64_t* out_id, void* stream);
 
+/* Top-k new pairs of a relation, queries (?, r, ?): the candidates are the UNORDERED pairs {s, t} with s < t (the
+ * DistMult score is symmetric in s and t; a self-pair is not an interaction), scored with the PRE-sigmoid
+ * S = sum_k z[s,k] w[r,k] z[t,k].  {s, t} is filtered for r when (s, r, t) OR (t, r, s) is in the filter: f_rowptr /
+ * f_dst is gn_rank_csr of the filter lists concatenated with their flipped copies (row s*n_rel + r holds every t of
+ * either direction, sorted), or f_rowptr == NULL.  Order: descending pre-sigmoid score, ties by the smaller pair id
+ * s*n + t (smaller s, then smaller t).  Requires n_nodes^2 < 2^31 (the pair id is the low word of a 64-bit key).
+ * No [n, n] score matrix is written: stage 1 (one block per query and tile of 64 s rows) scores 64 x 64 tiles of
+ * the triangle with FFMA and keeps the tile's top k keys; stage 2 (one block per query) merges them.
+ *
+ * gn_rank_rel_pairs_workspace_bytes: bytes of the keys passed from stage 1 to stage 2 (count * ceil(n/64) * k * 8).
+ * gn_rank_rel_pairs_select: stage 1 for the queries rel[0 .. count) (z rows at stride ldz >= D, w [n_rel, D]
+ *   contiguous, 1 <= k <= 256); writes ws.
+ * gn_rank_rel_pairs_merge: stage 2, reads ws.  out_score / out_src / out_dst [count, k]: score (sigmoid applied when
+ *   `sigmoid`), s and t (s < t); src = dst = -1 and score NaN pad a query with fewer than k admissible pairs. */
+size_t gn_rank_rel_pairs_workspace_bytes(int64_t count, int32_t n_nodes, int32_t k);
+int gn_rank_rel_pairs_select(const float* z, int64_t ldz, int32_t D, const float* w, int32_t n_rel, int32_t n_nodes,
+                             const int64_t* rel, int64_t count, const int32_t* f_rowptr /*or NULL*/,
+                             const int32_t* f_dst, int32_t k, void* ws, size_t ws_bytes, void* stream);
+int gn_rank_rel_pairs_merge(const void* ws, size_t ws_bytes, int32_t n_nodes, int64_t count, int32_t k, int sigmoid,
+                            float* out_score, int64_t* out_src, int64_t* out_dst, void* stream);
+
 /* ---- K12: slot all-gather over NVLink peer memory (multi-GPU exchange step) ------------------ */
 /* New design (the reference is single-device, SURVEY.md §8e).  Every rank of the node maps one
  * symmetric arena of identical layout; `arena_base` (HOST array, `world + 1` entries) holds every rank's

@@ -1,10 +1,10 @@
 #!/usr/bin/env python
-"""Filtered ranking (LinkRanker.metrics) and top-k (k = 10) over every (s, r) query group of a 90/10 test split, and
+"""Filtered ranking (LinkRanker.metrics) and top-k (k = 10) over every (s, r) query group of a 90/10 test split,
 filtered relation ranking (RelationRanker.metrics) and top-k relations (k = 10) over every directed (s, t) pair of
-the same split, at the pose-0 and pose-2 shapes, against torch-on-GPU restatements of the same computations timed
-in the same run.
+the same split, and top-k new pairs (topk_pairs, k = 10 and 100) of every relation with train + test filtered, at the
+pose-0 and pose-2 shapes, against torch-on-GPU restatements of the same computations timed in the same run.
 
-    python profiles/rank_bench.py --out DIR [--calls 20] [--workloads pose0,pose2] [--queries tail,relation]
+    python profiles/rank_bench.py --out DIR [--calls 20] [--workloads pose0,pose2] [--queries tail,relation,pair]
 
 Warm-up, then the median of `--calls` calls, each bracketed by CUDA events (warm L2: the score chunks are meant to
 stay there).  Writes DIR/rank_bench.json with the device name and power limit beside the numbers.
@@ -152,6 +152,30 @@ class TorchRelationRestatement:
         return torch.topk(S, K, dim=1)
 
 
+class TorchPairRestatement:
+    """Pair queries in eager torch: relation chunks of batched S_r = (z * w_r) z^T in fp32, a dense upper-triangle and
+    symmetric filter mask, a flatten and torch.topk (ties in torch.topk's own order)."""
+
+    def __init__(self, lists, n, r, dev, chunk_bytes=256 << 20):
+        self.n, self.r = n, r
+        self.chunk = max(1, chunk_bytes // (4 * n * n))
+        self.adm = torch.ones((r, n, n), dtype=torch.bool, device=dev).triu_(1)
+        for ei, et in lists:
+            self.adm[et, ei[0], ei[1]] = False
+            self.adm[et, ei[1], ei[0]] = False
+
+    def topk(self, z, w, k):
+        n = self.n
+        out_s = torch.empty((self.r, k), dtype=torch.float32, device=z.device)
+        out_i = torch.empty((self.r, k), dtype=torch.int64, device=z.device)
+        for a in range(0, self.r, self.chunk):
+            b = min(self.r, a + self.chunk)
+            S = torch.matmul(z[None] * w[a:b, None, :], z.t())
+            S.masked_fill_(~self.adm[a:b], float("-inf"))
+            out_s[a:b], out_i[a:b] = torch.topk(S.view(b - a, n * n), k, dim=1)
+        return out_s, out_i // n, out_i % n
+
+
 def _inputs(g, dev):
     train, test = _split(g)
     train = (train[0].to(dev), train[1].to(dev))
@@ -207,6 +231,39 @@ def run_relations(name, g, calls, dev):
         "metrics_product_tflops": round(flops / (t_metrics * 1e-3) / 1e12, 3),
         "agreement": agree, "agree": ok,
     }
+
+
+def run_pairs(name, g, calls, dev):
+    from gripnet_b200 import ranking
+    train, test, z, w = _inputs(g, dev)
+    n, r = g["n_d"], g["n_rel"]
+    import gripnet_b200 as gb
+    filt = gb.EdgeFilter([train, test], n, r)
+    rel = torch.arange(r, device=dev)
+    ref = TorchPairRestatement([train, test], n, r, dev)
+    flops = 2.0 * D * r * n * (n - 1) / 2
+    res = []
+    for k in (10, 100):
+        t_fused = _median_ms(lambda: ranking.topk_pairs(z, w, rel, k, filter=filt, sigmoid=False), calls)
+        t_ref = _median_ms(lambda: ref.topk(z, w, k), calls)
+        s, a, b = ranking.topk_pairs(z, w, rel, k, filter=filt, sigmoid=False)
+        s_ref, a_ref, b_ref = ref.topk(z, w, k)
+        scale = torch.stack([(z * w[i]) @ z.t() for i in range(r)]).abs().amax((1, 2))[:, None]
+        agree = {
+            "pair_ids_equal_fraction": float(((a == a_ref) & (b == b_ref)).double().mean()),
+            "score_max_rel_diff": float(((s - s_ref).abs() / scale).max()),
+            "filtered_or_ordered_pairs_returned": int((~ref.adm[rel[:, None], a, b]).sum()),
+        }
+        ok = agree["score_max_rel_diff"] < 1e-5 and agree["filtered_or_ordered_pairs_returned"] == 0 and \
+            agree["pair_ids_equal_fraction"] > 0.95
+        res.append({
+            "workload": name, "query": "pair", "n": n, "R": r, "D": D, "k": k, "queries": r,
+            "topk_pairs_ms": round(t_fused, 4), "torch_topk_pairs_ms": round(t_ref, 4),
+            "pair_flop": flops, "topk_pairs_tflops": round(flops / (t_fused * 1e-3) / 1e12, 3),
+            "torch_tflops": round(flops / (t_ref * 1e-3) / 1e12, 3),
+            "agreement": agree, "agree": ok,
+        })
+    return res
 
 
 def run(name, g, calls, dev):
@@ -273,13 +330,14 @@ def main():
         smi = f"unavailable ({e})"
     out = {"device": torch.cuda.get_device_name(dev), "nvidia_smi_name_power_limit_max_sm_clock": smi, "results": []}
     graphs = {"pose0": synthdata.pose_graph, "pose2": synthdata.pose2_graph}
-    runs = {"tail": run, "relation": run_relations}
+    runs = {"tail": run, "relation": run_relations, "pair": run_pairs}
     for name in args.workloads.split(","):
         g = graphs[name]()
         for query in args.queries.split(","):
             res = runs[query](name, g, args.calls, dev)
-            print(json.dumps(res), flush=True)
-            out["results"].append(res)
+            for one in res if isinstance(res, list) else [res]:
+                print(json.dumps(one), flush=True)
+                out["results"].append(one)
     os.makedirs(args.out, exist_ok=True)
     with open(os.path.join(args.out, "rank_bench.json"), "w") as f:
         json.dump(out, f, indent=1)
