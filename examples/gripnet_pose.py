@@ -3,7 +3,7 @@
 
     python examples/gripnet_pose.py EPOCHS datasets/pose/pose-0.pt [--out out/pose-0]
     python examples/gripnet_pose.py EPOCHS --synthetic            # pose-0-shaped synthetic supergraph
-    python examples/gripnet_pose.py EPOCHS --synthetic --rank     # + filtered test MRR / Hits@10 every epoch
+    python examples/gripnet_pose.py EPOCHS --synthetic --rank     # + filtered test MRR / Hits@k every epoch
     python examples/gripnet_pose.py EPOCHS --synthetic --novel 100   # + the 100 best new drug pairs per side effect
 
 Same model (``GripNet-pose.py:86-99``), optimiser (Adam, lr 0.01, ``:104``), per-epoch negative sampling
@@ -31,8 +31,9 @@ def main():
     ap.add_argument("--seed", type=int, default=1111)
     ap.add_argument("--rank", action="store_true",
                     help="also print the filtered test MRR and Hits@10 (all drugs as candidate tails, train + test "
-                         "positives filtered) and the filtered test relation MRR and Hits@10 (all side effects as "
-                         "candidates of each drug pair), macro-averaged over relations")
+                         "positives filtered), the filtered test relation MRR and Hits@10 (all side effects as "
+                         "candidates of each drug pair) and the filtered test pair MRR and Hits@100 (all drug pairs "
+                         "as candidates of each side effect), macro-averaged over relations")
     ap.add_argument("--novel", type=int, metavar="K", default=0,
                     help="after training, write <out>-novel.pt: the K (<= 256) most likely drug pairs {s, t} of every "
                          "side effect that are not train or test positives in either direction (scores after the "
@@ -71,6 +72,9 @@ def main():
                                             filter=filt)
         rank_rec = torch.empty(args.epochs, 2, n_rel, dtype=torch.float64, device=dev)
         rel_rank_rec = torch.empty(args.epochs, 2, n_rel, dtype=torch.float64, device=dev)
+        # about 2 * 10^5 candidate pairs per side effect at pose shapes: Hits@100
+        pair_ranker = ranking.PairRanker(test["dd_edge_index"], test["dd_edge_type"], test["n_d"], n_rel, filter=filt)
+        pair_rank_rec = torch.empty(args.epochs, 2, n_rel, dtype=torch.float64, device=dev)
     for epoch in range(args.epochs):
         t0 = time.time()
         losses[epoch] = trainer.train_epoch().detach()
@@ -83,12 +87,14 @@ def main():
             if ranker is not None:
                 ranker.metrics(z, model.dmt.weight, hits=(10,), out=rank_rec[epoch])
                 rel_ranker.metrics(z, model.dmt.weight, hits=(10,), out=rel_rank_rec[epoch])
+                pair_ranker.metrics(z, model.dmt.weight, hits=(100,), out=pair_rank_rec[epoch])
         tr, te = train_rec[epoch].nanmean(dim=1).tolist(), test_rec[epoch].nanmean(dim=1).tolist()   # one sync per epoch
         line = "{:3d}   loss:{:0.4f}   train auprc:{:0.4f} auroc:{:0.4f} ap:{:0.4f}   test auprc:{:0.4f} auroc:{:0.4f} " \
                "ap:{:0.4f}".format(epoch, float(losses[epoch].detach()), *tr, *te)
         if ranker is not None:
             line += "   test mrr:{:0.4f} hits@10:{:0.4f}".format(*rank_rec[epoch].nanmean(dim=1).tolist())
             line += "   test relation mrr:{:0.4f} hits@10:{:0.4f}".format(*rel_rank_rec[epoch].nanmean(dim=1).tolist())
+            line += "   test pair mrr:{:0.4f} hits@100:{:0.4f}".format(*pair_rank_rec[epoch].nanmean(dim=1).tolist())
         print(line + "   time:{:0.3f}".format(time.time() - t0))
     os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
     torch.save({k: v.cpu() for k, v in model.state_dict().items()}, args.out + "-model.pt")
@@ -96,6 +102,7 @@ def main():
     if ranker is not None:
         rec["test_rank_record"] = rank_rec.cpu()             # [epochs, 2 (mrr, hits@10), R]
         rec["test_relation_rank_record"] = rel_rank_rec.cpu()   # [epochs, 2 (mrr, hits@10), R]
+        rec["test_pair_rank_record"] = pair_rank_rec.cpu()   # [epochs, 2 (mrr, hits@100), R]
     torch.save(rec, args.out + "-record.pt")
     if args.novel:
         pos = [(train["dd_edge_index"], train["dd_edge_type"]), (test["dd_edge_index"], test["dd_edge_type"])]

@@ -29,7 +29,7 @@ from . import graph, ops, parallel, layers, decoder, encoder, losses, utils, met
 from .layers import myGCN, myRGCN, homoGraph, interGraph  # noqa: E402,F401
 from .decoder import multiRelaInnerProductDecoder, multiClassInnerProductDecoder  # noqa: E402,F401
 from .losses import link_prediction_loss, node_classification_loss  # noqa: E402,F401
-from .ranking import EdgeFilter, LinkRanker, RelationRanker  # noqa: E402,F401
+from .ranking import EdgeFilter, LinkRanker, PairRanker, RelationRanker  # noqa: E402,F401
 
 
 def install_as_gripnet():

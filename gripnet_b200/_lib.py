@@ -133,6 +133,11 @@ SIGNATURES = {
     "gn_rank_rel_pairs_workspace_bytes": (_SZ, [_I64, _I32, _I32]),
     "gn_rank_rel_pairs_select": (_INT, [_P, _I64, _I32, _P, _I32, _I32, _P, _I64, _P, _P, _I32, _P, _SZ, _P]),
     "gn_rank_rel_pairs_merge": (_INT, [_P, _SZ, _I32, _I64, _I32, _INT, _P, _P, _P, _P]),
+    "gn_rank_rel_pairs_rank_workspace_bytes": (_SZ, [_I64, _I32]),
+    "gn_rank_rel_pairs_targets": (_INT, [_P, _P, _P, _P, _I64, _I32, _P, _P, _P, _P]),
+    "gn_rank_rel_pairs_count": (_INT, [_P, _I64, _I32, _P, _I32, _I32, _P, _P, _P, _P, _P, _I64, _P, _I32, _P, _P,
+                                       _P, _SZ, _P]),
+    "gn_rank_rel_pairs_finish": (_INT, [_P, _SZ, _I32, _P, _P, _I64, _P, _P, _P]),
     "gn_peer_max_world": (_INT, []),
     "gn_peer_allgather": (_INT, [_P, _I32, _I32, _I64, _I64, _I64, _I32, _P, _P, _P, _P]),
     "gn_peer_halo_grid": (_INT, []),

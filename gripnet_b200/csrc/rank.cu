@@ -272,9 +272,11 @@ __global__ void __launch_bounds__(kMetricThreads) rank_metrics_kernel(const floa
 // entry overwritten with kMaskedBits first) has key 0.  The k-th largest key is found by an MSB-first radix select
 // (8 passes of 8 bits over the row, read from L1 / L2), the keys at or above it are gathered and bitonic-sorted.
 // ---------------------------------------------------------------------------------------------------------------
+// order-preserving bits of a float: a larger unsigned value is a larger score
+__device__ __forceinline__ uint32_t order_bits(uint32_t b) { return (b & 0x80000000u) ? ~b : (b | 0x80000000u); }
+
 __device__ __forceinline__ uint64_t score_key(uint32_t b, uint32_t id) {
-  const uint32_t u = (b & 0x80000000u) ? ~b : (b | 0x80000000u);
-  return (uint64_t(u) << 32) | uint64_t(~id);
+  return (uint64_t(order_bits(b)) << 32) | uint64_t(~id);
 }
 
 __device__ __forceinline__ uint64_t topk_key(const float* srow, int c) {
@@ -474,26 +476,16 @@ struct BufKeys {
   __device__ __forceinline__ uint64_t operator()(int c) const { return buf[c]; }
 };
 
-__global__ void __launch_bounds__(kTopkThreads) rank_rel_pairs_select_kernel(
-    const float* __restrict__ z, int64_t ldz, int D, const float* __restrict__ w, int32_t n_rel, int32_t n,
-    const int64_t* __restrict__ rel, int64_t count, int n_tiles, const int32_t* __restrict__ f_rowptr,
-    const int32_t* __restrict__ f_dst, int k, uint64_t* __restrict__ keys_out) {
+// The score tiles of one 64-row tile of s, s0 = 64 * tile: for t0 = s0, s0 + 64, ... < n, thread (ty, tx) holds
+// acc[i][j] = S(s0 + 4 ty + i, t0 + 4 tx + j) and the block calls epi(t0, acc).  Every score is the one per-pair
+// sequence q_f = z[s,f] * w[r,f] (rounded), acc = fmaf(q_f, z[t,f], acc) for f = 0 .. D-1, then zero padding to a
+// multiple of kPairKc (which can only turn -0 into +0); rank_rel_pairs_query_kernel restates it per pair.
+template <class Epilogue>
+__device__ __forceinline__ void pair_tiles(const float* __restrict__ z, int64_t ldz, int D,
+                                           const float* __restrict__ wr, int32_t n, int s0, Epilogue&& epi) {
   __shared__ __align__(16) float As[kPairKc][kPairTile + 4];
   __shared__ __align__(16) float Bs[kPairKc][kPairTile + 4];
-  __shared__ uint64_t buf[kPairBuf];
-  __shared__ int n_buf;
-  __shared__ uint64_t thr_s;
   const int tid = threadIdx.x, ty = tid >> 4, tx = tid & 15;
-  // heavy tiles (small s) first: block b is tile b / count of query b % count
-  const int tile = int(blockIdx.x / count);
-  const int64_t qi = int64_t(blockIdx.x) - int64_t(tile) * count;
-  const int64_t r = rel[qi];
-  const float* wr = w + r * D;
-  const int s0 = tile * kPairTile;
-  if (tid == 0) {
-    n_buf = 0;
-    thr_s = 0ull;
-  }
   for (int t0 = s0; t0 < n; t0 += kPairTile) {
     float acc[4][4];
 #pragma unroll
@@ -521,6 +513,29 @@ __global__ void __launch_bounds__(kTopkThreads) rank_rel_pairs_select_kernel(
           for (int j = 0; j < 4; ++j) acc[i][j] = fmaf(av[i], bv[j], acc[i][j]);
       }
     }
+    epi(t0, acc);
+  }
+}
+
+__global__ void __launch_bounds__(kTopkThreads) rank_rel_pairs_select_kernel(
+    const float* __restrict__ z, int64_t ldz, int D, const float* __restrict__ w, int32_t n_rel, int32_t n,
+    const int64_t* __restrict__ rel, int64_t count, int n_tiles, const int32_t* __restrict__ f_rowptr,
+    const int32_t* __restrict__ f_dst, int k, uint64_t* __restrict__ keys_out) {
+  __shared__ uint64_t buf[kPairBuf];
+  __shared__ int n_buf;
+  __shared__ uint64_t thr_s;
+  const int tid = threadIdx.x, ty = tid >> 4, tx = tid & 15;
+  // heavy tiles (small s) first: block b is tile b / count of query b % count
+  const int tile = int(blockIdx.x / count);
+  const int64_t qi = int64_t(blockIdx.x) - int64_t(tile) * count;
+  const int64_t r = rel[qi];
+  const float* wr = w + r * D;
+  const int s0 = tile * kPairTile;
+  if (tid == 0) {
+    n_buf = 0;
+    thr_s = 0ull;
+  }
+  pair_tiles(z, ldz, D, wr, n, s0, [&](int t0, const float (&acc)[4][4]) {
     const uint64_t thr = thr_s;
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
@@ -545,7 +560,7 @@ __global__ void __launch_bounds__(kTopkThreads) rank_rel_pairs_select_kernel(
         thr_s = sel[k - 1];
       }
     }
-  }
+  });
   __syncthreads();
   const uint64_t* sel = topk_select(BufKeys{buf}, n_buf, k);
   if (tid < k) keys_out[(qi * n_tiles + tile) * k + tid] = sel[tid];
@@ -565,6 +580,185 @@ __global__ void __launch_bounds__(kTopkThreads) rank_rel_pairs_merge_kernel(cons
     out_score[qi * k + tid] = topk_out_score(key, sigmoid);
     out_src[qi * k + tid] = id >= 0 ? id / n : -1;
     out_dst[qi * k + tid] = id >= 0 ? id % n : -1;
+  }
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// filtered pair ranks (?, r, ?): every query triple (s, r, t), s != t, is ranked against the unordered pairs
+// {a, b}, a < b, of its relation.  The query triples are grouped by relation (gn_index_prep order i, edge
+// rel_perm[i]); per call their scores are computed with the tiles' per-pair sequence and sorted ascending inside
+// their relation.  The count kernel walks the same score tiles as rank_rel_pairs_select_kernel and, for a
+// candidate at or above the relation's smallest query score, finds lb = #{query scores < S} and whether S ties
+// query score lb; an unfiltered candidate adds 1 to gt[lb] (lb > 0) and to eq[lb] (tie).  A query at tie block
+// [L, U) of the sorted scores then has opt = sum_{j >= U} gt[j] and pess = opt + eq[L] - [its own pair counted].
+// Relation r's counters are the m_r + 1 slots from rel_rowptr[r] + r of gt and of eq.
+// ---------------------------------------------------------------------------------------------------------------
+constexpr int kRankStage = 3072;     // a relation of at most kRankStage - 1 query triples is staged in shared memory
+constexpr int kFinishThreads = 256;
+
+__device__ __forceinline__ void canonical_pair(const int64_t* __restrict__ src, const int64_t* __restrict__ dst,
+                                               int32_t e, int64_t& a, int64_t& b) {
+  const int64_t s = src[e], t = dst[e];
+  a = s < t ? s : t;
+  b = s < t ? t : s;
+}
+
+// whether the pair of query i is in the symmetrised filter (construction time)
+__global__ void rank_rel_pairs_targets_kernel(const int64_t* __restrict__ src, const int64_t* __restrict__ dst,
+                                              const int64_t* __restrict__ etype, const int32_t* __restrict__ perm,
+                                              int32_t count, int32_t n_rel, const int32_t* __restrict__ f_rowptr,
+                                              const int32_t* __restrict__ f_dst, int32_t* __restrict__ filtered) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= count) return;
+  const int32_t e = perm[i];
+  int64_t a, b;
+  canonical_pair(src, dst, e, a, b);
+  filtered[i] = pair_filtered(f_rowptr, f_dst, a * n_rel + etype[e], int32_t(b)) ? 1 : 0;
+}
+
+// score of query i in the tiles' per-pair sequence, its order-preserving key and its relation
+__global__ void rank_rel_pairs_query_kernel(const float* __restrict__ z, int64_t ldz, int D,
+                                            const float* __restrict__ w, const int64_t* __restrict__ src,
+                                            const int64_t* __restrict__ dst, const int64_t* __restrict__ etype,
+                                            const int32_t* __restrict__ perm, int32_t count,
+                                            float* __restrict__ score, int32_t* __restrict__ key,
+                                            int32_t* __restrict__ qrel) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= count) return;
+  const int32_t e = perm[i];
+  int64_t a, b;
+  canonical_pair(src, dst, e, a, b);
+  const int64_t r = etype[e];
+  const float *za = z + a * ldz, *zb = z + b * ldz, *wr = w + r * D;
+  float acc = 0.0f;
+  for (int f = 0; f < D; ++f) acc = fmaf(__fmul_rn(za[f], wr[f]), zb[f], acc);
+  score[i] = acc;
+  key[i] = int32_t(order_bits(__float_as_uint(acc)));
+  qrel[i] = int32_t(r);
+}
+
+template <class T>
+__global__ void rank_gather_kernel(const T* __restrict__ v, const int32_t* __restrict__ idx, int32_t count,
+                                   T* __restrict__ out) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < count) out[i] = v[idx[i]];
+}
+
+__global__ void __launch_bounds__(kTopkThreads) rank_rel_pairs_count_kernel(
+    const float* __restrict__ z, int64_t ldz, int D, const float* __restrict__ w, int32_t n_rel, int32_t n,
+    const int32_t* __restrict__ group_rel, int32_t n_groups, const int32_t* __restrict__ rel_rowptr,
+    const float* __restrict__ sorted, const int32_t* __restrict__ f_rowptr, const int32_t* __restrict__ f_dst,
+    int32_t* __restrict__ gt, int32_t* __restrict__ eq) {
+  __shared__ float ss_s[kRankStage];
+  __shared__ int gt_s[kRankStage], eq_s[kRankStage];
+  const int tid = threadIdx.x, ty = tid >> 4, tx = tid & 15;
+  // tile order of rank_rel_pairs_select_kernel: block b is tile b / n_groups of query relation b % n_groups
+  const int tile = int(blockIdx.x / n_groups);
+  const int32_t r = group_rel[blockIdx.x - tile * n_groups];
+  const int b = rel_rowptr[r], m = rel_rowptr[r + 1] - b;
+  const int64_t c0 = int64_t(b) + r;
+  const bool staged = m < kRankStage;
+  const float* ss = staged ? ss_s : sorted + b;
+  int* gtp = staged ? gt_s : gt + c0;
+  int* eqp = staged ? eq_s : eq + c0;
+  if (staged) {
+    for (int j = tid; j <= m; j += kTopkThreads) {
+      if (j < m) ss_s[j] = sorted[b + j];
+      gt_s[j] = 0;
+      eq_s[j] = 0;
+    }
+  }
+  __syncthreads();
+  const float smin = ss[0];
+  const int s0 = tile * kPairTile;
+  pair_tiles(z, ldz, D, w + int64_t(r) * D, n, s0, [&](int t0, const float (&acc)[4][4]) {
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+      const int s = s0 + ty * 4 + i;
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        const int t = t0 + tx * 4 + j;
+        const float v = acc[i][j];
+        if (s >= n || t >= n || t <= s || !(v >= smin)) continue;   // most candidates: below every query score
+        int lo = 0, hi = m;
+        while (lo < hi) {
+          const int mid = (lo + hi) >> 1;
+          if (ss[mid] < v) lo = mid + 1;
+          else hi = mid;
+        }
+        const bool tie = lo < m && ss[lo] == v;
+        if (f_rowptr != nullptr && pair_filtered(f_rowptr, f_dst, int64_t(s) * n_rel + r, t)) continue;
+        if (lo > 0) atomicAdd(&gtp[lo], 1);
+        if (tie) atomicAdd(&eqp[lo], 1);
+      }
+    }
+  });
+  if (staged) {
+    __syncthreads();
+    for (int j = tid; j <= m; j += kTopkThreads) {
+      if (gt_s[j] != 0) atomicAdd(&gt[c0 + j], gt_s[j]);
+      if (eq_s[j] != 0) atomicAdd(&eq[c0 + j], eq_s[j]);
+    }
+  }
+}
+
+// one block per relation r < n_rel: suffix sums of gt in place, then the rank of each query; block n_rel writes NaN
+// for the self-pair triples (key n_rel of the relation index)
+__global__ void __launch_bounds__(kFinishThreads) rank_rel_pairs_finish_kernel(
+    const int32_t* __restrict__ rel_rowptr, const int32_t* __restrict__ rel_perm, int32_t n_rel,
+    const float* __restrict__ score, const float* __restrict__ sorted, int32_t* __restrict__ gt,
+    const int32_t* __restrict__ eq, const int32_t* __restrict__ t_filtered, float* __restrict__ rank) {
+  __shared__ int warp_sum[kFinishThreads / 32];
+  const int r = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int b = rel_rowptr[r], e = rel_rowptr[r + 1], m = e - b;
+  if (r == n_rel) {
+    for (int i = b + tid; i < e; i += kFinishThreads) rank[rel_perm[i]] = __uint_as_float(0x7fc00000u);
+    return;
+  }
+  if (m == 0) return;
+  int* g = gt + b + r;
+  const int* q = eq + b + r;
+  // suffix sums over the m + 1 slots, chunks of kFinishThreads from the top (thread 0 takes the highest slot)
+  int carry = 0;
+  for (int top = m; top >= 0; top -= kFinishThreads) {
+    const int j = top - tid;
+    int incl = j >= 0 ? g[j] : 0;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const int t = __shfl_up_sync(kFull, incl, o);
+      if (lane >= o) incl += t;
+    }
+    if (lane == 31) warp_sum[warp] = incl;
+    __syncthreads();
+    int off = carry, total = carry;
+#pragma unroll
+    for (int w2 = 0; w2 < kFinishThreads / 32; ++w2) {
+      off += w2 < warp ? warp_sum[w2] : 0;
+      total += warp_sum[w2];
+    }
+    if (j >= 0) g[j] = incl + off;
+    carry = total;
+    __syncthreads();
+  }
+  const float* ss = sorted + b;
+  for (int i = b + tid; i < e; i += kFinishThreads) {
+    const float x = score[i];
+    int lo = 0, hi = m;
+    while (lo < hi) {
+      const int mid = (lo + hi) >> 1;
+      if (ss[mid] < x) lo = mid + 1;
+      else hi = mid;
+    }
+    const int L = lo;
+    hi = m;
+    while (lo < hi) {
+      const int mid = (lo + hi) >> 1;
+      if (ss[mid] <= x) lo = mid + 1;
+      else hi = mid;
+    }
+    const int opt = g[lo];                                   // lo = U <= m
+    const int pess = opt + q[L] - ((t_filtered != nullptr && t_filtered[i]) ? 0 : 1);
+    rank[rel_perm[i]] = 1.0f + 0.5f * float(opt + pess);
   }
 }
 
@@ -795,6 +989,96 @@ int gn_rank_rel_pairs_merge(const void* ws, size_t ws_bytes, int32_t n_nodes, in
   GN_LAUNCH(rank_rel_pairs_merge_kernel, (unsigned)count, kTopkThreads, 0, as_stream(stream),
             static_cast<const uint64_t*>(ws), rel_pairs_tiles(n_nodes) * k, n_nodes, k, sigmoid, out_score, out_src,
             out_dst);
+  return GN_OK;
+}
+
+// the per-call workspace of the pair ranks: what gn_rank_rel_pairs_finish reads first, the sort scratch after it
+struct RelPairsRankWs {
+  float* score;       // [Q] query scores, grouped order
+  float* sorted;      // [Q] ascending inside each relation
+  int32_t* cnt;       // [2 (Q + R)] gt, then eq
+  int32_t *key, *qrel, *skey, *idx1, *idx2;
+  void* rest;
+  size_t rest_bytes;
+  bool ok;
+  RelPairsRankWs(void* ws, size_t ws_bytes, int64_t nq, int32_t n_rel) {
+    Arena a(ws, ws_bytes);
+    const size_t q = size_t(nq > 0 ? nq : 1);
+    score = a.take<float>(q);
+    sorted = a.take<float>(q);
+    cnt = a.take<int32_t>(2 * (size_t(nq) + size_t(n_rel)));
+    key = a.take<int32_t>(q);
+    qrel = a.take<int32_t>(q);
+    skey = a.take<int32_t>(q);
+    idx1 = a.take<int32_t>(q);
+    idx2 = a.take<int32_t>(q);
+    ok = a.ok();
+    rest = ok ? a.base + a.off : nullptr;
+    rest_bytes = ok ? a.cap - a.off : 0;
+  }
+};
+
+static bool rel_pairs_rank_args(int32_t n_rel, int64_t n_queries) {
+  return n_rel > 0 && n_queries >= 0 && n_queries < (int64_t(1) << 31) - n_rel;
+}
+
+size_t gn_rank_rel_pairs_rank_workspace_bytes(int64_t n_queries, int32_t n_rel) {
+  const size_t q = align_up(size_t(n_queries > 0 ? n_queries : 1) * 4);
+  const size_t r = size_t(n_rel > 0 ? n_rel : 1);
+  return 7 * q + align_up(2 * (size_t(n_queries > 0 ? n_queries : 0) + r) * 4) + sort_ws_bytes(n_queries) + 4096;
+}
+
+int gn_rank_rel_pairs_targets(const int64_t* src, const int64_t* dst, const int64_t* etype, const int32_t* rel_perm,
+                              int64_t n_queries, int32_t n_rel, const int32_t* f_rowptr, const int32_t* f_dst,
+                              int32_t* filtered, void* stream) {
+  if (!rel_pairs_rank_args(n_rel, n_queries)) return GN_ERR_ARG;
+  if (n_queries == 0) return GN_OK;
+  if (!src || !dst || !etype || !rel_perm || !f_rowptr || !f_dst || !filtered) return GN_ERR_ARG;
+  GN_LAUNCH(rank_rel_pairs_targets_kernel, (unsigned)ceil_div(n_queries, 256), 256, 0, as_stream(stream), src, dst,
+            etype, rel_perm, int32_t(n_queries), n_rel, f_rowptr, f_dst, filtered);
+  return GN_OK;
+}
+
+int gn_rank_rel_pairs_count(const float* z, int64_t ldz, int32_t D, const float* w, int32_t n_rel, int32_t n_nodes,
+                            const int64_t* src, const int64_t* dst, const int64_t* etype, const int32_t* rel_rowptr,
+                            const int32_t* rel_perm, int64_t n_queries, const int32_t* group_rel, int32_t n_groups,
+                            const int32_t* f_rowptr, const int32_t* f_dst, void* ws, size_t ws_bytes, void* stream) {
+  if (D <= 0 || n_nodes <= 0 || ldz < D || n_groups < 0 || !rel_pairs_rank_args(n_rel, n_queries)) return GN_ERR_ARG;
+  if (int64_t(n_nodes) * n_nodes >= (int64_t(1) << 31) || int64_t(n_nodes) * n_rel >= (int64_t(1) << 31))
+    return GN_ERR_RANGE;
+  if (n_queries == 0 || n_groups == 0) return GN_OK;
+  const int n_tiles = rel_pairs_tiles(n_nodes);
+  if (int64_t(n_groups) * n_tiles >= (int64_t(1) << 31)) return GN_ERR_RANGE;
+  if (!z || !w || !src || !dst || !etype || !rel_rowptr || !rel_perm || !group_rel || (f_rowptr && !f_dst))
+    return GN_ERR_ARG;
+  const RelPairsRankWs p(ws, ws_bytes, n_queries, n_rel);
+  if (!p.ok) return GN_ERR_WORKSPACE;
+  cudaStream_t st = as_stream(stream);
+  const int32_t nq = int32_t(n_queries);
+  const unsigned gq = (unsigned)ceil_div(nq, 256);
+  GN_LAUNCH(rank_rel_pairs_query_kernel, gq, 256, 0, st, z, ldz, D, w, src, dst, etype, rel_perm, nq, p.score, p.key,
+            p.qrel);
+  // stable: by score key, then by relation -> ascending scores inside each relation's range of the grouped order
+  GN_CHECK(sort_pairs(p.key, nullptr, p.skey, p.idx1, nq, 32, p.rest, p.rest_bytes, st));
+  GN_LAUNCH(rank_gather_kernel<int32_t>, gq, 256, 0, st, (const int32_t*)p.qrel, (const int32_t*)p.idx1, nq, p.key);
+  GN_CHECK(sort_pairs(p.key, p.idx1, p.skey, p.idx2, nq, bits_for(n_rel > 1 ? n_rel : 2), p.rest, p.rest_bytes, st));
+  GN_LAUNCH(rank_gather_kernel<float>, gq, 256, 0, st, (const float*)p.score, (const int32_t*)p.idx2, nq, p.sorted);
+  if (cudaMemsetAsync(p.cnt, 0, 2 * (size_t(nq) + size_t(n_rel)) * 4, st) != cudaSuccess) return GN_ERR_CUDA;
+  GN_LAUNCH(rank_rel_pairs_count_kernel, (unsigned)(int64_t(n_groups) * n_tiles), kTopkThreads, 0, st, z, ldz, D, w,
+            n_rel, n_nodes, group_rel, n_groups, rel_rowptr, (const float*)p.sorted, f_rowptr, f_dst, p.cnt,
+            p.cnt + nq + n_rel);
+  return GN_OK;
+}
+
+int gn_rank_rel_pairs_finish(void* ws, size_t ws_bytes, int32_t n_rel, const int32_t* rel_rowptr,
+                             const int32_t* rel_perm, int64_t n_queries, const int32_t* target_filtered, float* rank,
+                             void* stream) {
+  if (!rel_pairs_rank_args(n_rel, n_queries) || !rel_rowptr || !rel_perm || !rank) return GN_ERR_ARG;
+  const RelPairsRankWs p(ws, ws_bytes, n_queries, n_rel);
+  if (!p.ok) return GN_ERR_WORKSPACE;
+  GN_LAUNCH(rank_rel_pairs_finish_kernel, (unsigned)n_rel + 1, kFinishThreads, 0, as_stream(stream), rel_rowptr,
+            rel_perm, n_rel, (const float*)p.score, (const float*)p.sorted, p.cnt, (const int32_t*)(p.cnt + n_queries + n_rel),
+            target_filtered, rank);
   return GN_OK;
 }
 

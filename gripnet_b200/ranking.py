@@ -48,7 +48,18 @@ Pair queries ``(?, r, ?)`` of a relation (``topk_pairs``: "which new drug pairs 
   ``s * n + t``); ids ``-1`` / score NaN pad a query with fewer than ``k`` admissible pairs (e.g. ``n < 2``);
   ``sigmoid`` applies to the returned scores;
 * ``1 <= k <= 256`` and ``n * n < 2^31`` (the pair id is the low word of the 64-bit selection key); the work grows as
-  ``Q * n^2 * D``.
+  ``Q * n^2 * D``;
+* pair ranking (``PairRanker``): each triple ``(s, r, t)`` of a list is the query ``(?, r, ?)`` with answer
+  ``{s, t}``, canonicalised to ``(min(s, t), r, max(s, t))`` (so ``(s, r, t)`` and ``(t, r, s)`` get one rank); the
+  candidates are those of ``topk_pairs``; with ``N = {a < b : {a, b} != {s, t}, {a, b} not filtered for r}``,
+  ``opt = #{N : S > S(s, t)}``, ``pess = #{N : S >= S(s, t)}``, ``rank = 1 + (opt + pess) / 2``; the target is
+  left out of ``N`` whether or not the filter holds it;
+* every pair score, the target's and each candidate's, is the one fp32 sequence ``q_f = z[a,f] * w[r,f]`` (rounded),
+  ``acc = fmaf(q_f, z[b,f], acc)`` for ``f = 0 .. D-1`` with ``a < b``: a target never ties or beats itself through
+  two code paths, and the ranker's scores equal those ``topk_pairs`` selects on (+0 / -0 aside, which compare equal);
+* a self-pair triple ``s == t`` is no candidate of any query: its rank is NaN and ``metrics`` leaves it out;
+* ranks are exact in float32 while ``n (n - 1) / 2 < 2^23`` (``n <= 4096``) and round to the nearest float32 beyond;
+  counts are int32 (``n * n < 2^31``).
 
 Single GPU: a partitioned ``z`` is gathered by the caller first (``parallel.all_gather_rows``).
 """
@@ -235,9 +246,10 @@ def _relation_index(et, num_relations, device):
 
 
 class _Ranker:
-    """What ``LinkRanker`` and ``RelationRanker`` share: the output checks of ``ranks`` and the per-relation
-    reduction of ``metrics``.  Subclasses set ``num_relations``, ``device``, ``n_edges``, ``_rel_rowptr``,
-    ``_rel_perm`` and define ``ranks``."""
+    """What ``LinkRanker``, ``RelationRanker`` and ``PairRanker`` share: the output checks of ``ranks`` and the
+    per-relation reduction of ``metrics``.  Subclasses set ``num_relations``, ``device``, ``n_edges``,
+    ``_rel_rowptr``, ``_rel_perm`` (the edges of relation ``r`` are ``_rel_perm[_rel_rowptr[r]:_rel_rowptr[r + 1]]``
+    for ``r < R``) and define ``ranks``."""
 
     def _rank_out(self, out):
         if out is None:
@@ -376,6 +388,74 @@ class RelationRanker(_Ranker):
                                               _ptr(self._q.eid),
                                               _ptr(self._f_row[g0:]) if self._f_row is not None else None, _ptr(fr),
                                               _ptr(fd), out.data_ptr(), _stream()), "gn_rank_pair_count")
+        return out
+
+
+class PairRanker(_Ranker):
+    """Filtered ranks of the triples of one list among all unordered pairs of their relation, and their per-relation
+    MRR / Hits@k.
+
+    ``edge_index`` int64 ``[2, E]`` / ``edge_type`` int64 ``[E]``: the triples ``(s, r, t)`` to rank (e.g. the test
+    split), each the query ``(?, r, ?)`` with answer ``{s, t}``; ``filter``: an ``EdgeFilter`` of the known triples,
+    read in both directions (None: raw ranks).  ``(s, r, t)`` and ``(t, r, s)`` get the same rank; a self-pair
+    triple ``s == t`` is no candidate, so its rank is NaN and ``metrics`` leaves it out.  Needs ``n * n < 2^31``;
+    ranks are exact in float32 while ``n (n - 1) / 2 < 2^23`` (``n <= 4096``) and round to the nearest float32
+    beyond.  Construction does the host reads (the filter's symmetrised view, the relation index, whether each
+    target pair is filtered); ``ranks`` / ``metrics`` then read nothing back and branch on no device value, so they
+    can be captured in a CUDA graph.  One GPU: gather a partitioned ``z`` first."""
+
+    def __init__(self, edge_index, edge_type, num_nodes, num_relations, filter=None):
+        lib = _lib.load()
+        self.num_nodes, self.num_relations = _sizes(num_nodes, num_relations)
+        n, r = self.num_nodes, self.num_relations
+        if n * n >= 2 ** 31:
+            raise RuntimeError(f"gripnet_b200: PairRanker needs num_nodes^2 < 2^31, got {n} nodes")
+        ei, et = _edge_list(edge_index, edge_type, n, r, "query")
+        self.device = ei.device
+        self.n_edges = int(ei.size(1))
+        self.filter = filter
+        self._f = filter._symmetric(n, r, self.device) if filter is not None else None
+        self._ei, self._et = ei, et
+        # relation index over R + 1 keys: a self-pair triple takes key R, so metrics (rows 0 .. R - 1) skip it
+        key = torch.where(ei[0] == ei[1], torch.full_like(et, r), et)
+        self._rel_rowptr, self._rel_perm = _relation_index(key, r + 1, self.device)
+        counts = self._rel_rowptr[:r + 1].cpu()                         # the one host read of the index
+        self._n_queries = int(counts[r])
+        self._groups = torch.nonzero(counts[1:] > counts[:-1]).view(-1).to(torch.int32).to(self.device)
+        self._t_filtered = None
+        if self._f is not None and self._n_queries > 0:
+            self._t_filtered = torch.empty(self._n_queries, dtype=torch.int32, device=self.device)
+            _lib.check(lib.gn_rank_rel_pairs_targets(_ptr(ei[0]), _ptr(ei[1]), _ptr(et), _ptr(self._rel_perm),
+                                                     self._n_queries, r, _ptr(self._f.rowptr), _ptr(self._f.dst),
+                                                     _ptr(self._t_filtered), _stream()), "gn_rank_rel_pairs_targets")
+        self._ws_bytes = int(lib.gn_rank_rel_pairs_rank_workspace_bytes(self._n_queries, r))
+
+    @property
+    def n_groups(self):
+        """Number of distinct relations with rankable (non-self-pair) triples."""
+        return int(self._groups.numel())
+
+    def ranks(self, z, weight, out=None):
+        """float32 ``[E]``: the filtered pair rank of every triple, in the list's order (NaN for a self-pair)."""
+        lib = _lib.load()
+        z, w = _embeddings(z, weight, self.num_nodes, self.num_relations)
+        if z.device != self.device:
+            raise RuntimeError("gripnet_b200: z is not on the ranker's device")
+        out = self._rank_out(out)
+        if self.n_edges == 0:
+            return out
+        r = self.num_relations
+        ws = _ws(self._ws_bytes, self.device)
+        fr, fd = (self._f.rowptr, self._f.dst) if self._f is not None else (None, None)
+        ei, et = self._ei, self._et
+        _lib.check(lib.gn_rank_rel_pairs_count(z.data_ptr(), ops._ldz(z), z.size(1), w.data_ptr(), r, self.num_nodes,
+                                               _ptr(ei[0]), _ptr(ei[1]), _ptr(et), _ptr(self._rel_rowptr),
+                                               _ptr(self._rel_perm), self._n_queries, _ptr(self._groups),
+                                               self.n_groups, _ptr(fr), _ptr(fd), _ptr(ws), ws.numel(), _stream()),
+                   "gn_rank_rel_pairs_count")
+        _lib.check(lib.gn_rank_rel_pairs_finish(_ptr(ws), ws.numel(), r, _ptr(self._rel_rowptr), _ptr(self._rel_perm),
+                                                self._n_queries, _ptr(self._t_filtered), out.data_ptr(), _stream()),
+                   "gn_rank_rel_pairs_finish")
         return out
 
 

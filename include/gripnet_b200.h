@@ -489,6 +489,39 @@ int gn_rank_rel_pairs_select(const float* z, int64_t ldz, int32_t D, const float
 int gn_rank_rel_pairs_merge(const void* ws, size_t ws_bytes, int32_t n_nodes, int64_t count, int32_t k, int sigmoid,
                             float* out_score, int64_t* out_src, int64_t* out_dst, void* stream);
 
+/* Filtered ranks of pair queries (?, r, ?): a query triple (s, r, t) with s != t is ranked among the unordered pairs
+ * {a, b}, a < b, of relation r.  Canonical pair: a = min(s, t), b = max(s, t).  Every score, the target's and each
+ * candidate's, is the per-pair sequence of gn_rank_rel_pairs_select: q_f = z[a,f] * w[r,f] rounded, then
+ * acc = fmaf(q_f, z[b,f], acc) for f = 0 .. D-1 (so a target never ties or beats itself through two code paths).
+ * Filter: the symmetrised f_rowptr / f_dst of gn_rank_rel_pairs_select, or f_rowptr == NULL.  With
+ * N = {a < b : {a, b} != {s, t}, {a, b} not filtered for r}: opt = #{N : S > S(s,t)}, pess = #{N : S >= S(s,t)},
+ * rank = 1 + (opt + pess) / 2 (float32; exact while n(n-1)/2 < 2^23).  Requires n_nodes^2 < 2^31.
+ * The triples are given by src / dst / etype (int64 [E]) and their relation index rel_rowptr [n_rel + 2] /
+ * rel_perm [E]: gn_index_prep over n_rel + 1 keys, the key of a self-pair triple being n_rel, so the n_queries =
+ * rel_rowptr[n_rel] rankable triples come first, grouped by relation (position i: edge rel_perm[i]).
+ *
+ * gn_rank_rel_pairs_rank_workspace_bytes: bytes of the per-call workspace shared by count and finish.
+ * gn_rank_rel_pairs_targets: filtered[i] = 1 when the pair of query i is in the filter (once, at construction).
+ * gn_rank_rel_pairs_count: scores the queries, sorts them inside their relation (two stable sort passes: score
+ *   key, then relation), and counts, in one block per (query relation group_rel[g], 64-row tile of a), every
+ *   unfiltered candidate against its relation's sorted query scores; no [n, n] score matrix is written.
+ *   group_rel [n_groups]: the relations with at least one query.  Integer counters: deterministic.
+ * gn_rank_rel_pairs_finish: reads the workspace of the preceding count (same arguments) and writes rank[edge id]
+ *   for every triple of the list: the OGB rank above (target_filtered from gn_rank_rel_pairs_targets, NULL without
+ *   a filter), NaN for a self-pair.  Count and finish read nothing back to the host: capturable. */
+size_t gn_rank_rel_pairs_rank_workspace_bytes(int64_t n_queries, int32_t n_rel);
+int gn_rank_rel_pairs_targets(const int64_t* src, const int64_t* dst, const int64_t* etype, const int32_t* rel_perm,
+                              int64_t n_queries, int32_t n_rel, const int32_t* f_rowptr, const int32_t* f_dst,
+                              int32_t* filtered, void* stream);
+int gn_rank_rel_pairs_count(const float* z, int64_t ldz, int32_t D, const float* w, int32_t n_rel, int32_t n_nodes,
+                            const int64_t* src, const int64_t* dst, const int64_t* etype, const int32_t* rel_rowptr,
+                            const int32_t* rel_perm, int64_t n_queries, const int32_t* group_rel, int32_t n_groups,
+                            const int32_t* f_rowptr /*or NULL*/, const int32_t* f_dst, void* ws, size_t ws_bytes,
+                            void* stream);
+int gn_rank_rel_pairs_finish(void* ws, size_t ws_bytes, int32_t n_rel, const int32_t* rel_rowptr,
+                             const int32_t* rel_perm, int64_t n_queries, const int32_t* target_filtered /*or NULL*/,
+                             float* rank, void* stream);
+
 /* ---- K12: slot all-gather over NVLink peer memory (multi-GPU exchange step) ------------------ */
 /* New design (the reference is single-device, SURVEY.md §8e).  Every rank of the node maps one
  * symmetric arena of identical layout; `arena_base` (HOST array, `world + 1` entries) holds every rank's

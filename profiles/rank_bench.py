@@ -1,8 +1,9 @@
 #!/usr/bin/env python
 """Filtered ranking (LinkRanker.metrics) and top-k (k = 10) over every (s, r) query group of a 90/10 test split,
 filtered relation ranking (RelationRanker.metrics) and top-k relations (k = 10) over every directed (s, t) pair of
-the same split, and top-k new pairs (topk_pairs, k = 10 and 100) of every relation with train + test filtered, at the
-pose-0 and pose-2 shapes, against torch-on-GPU restatements of the same computations timed in the same run.
+the same split, top-k new pairs (topk_pairs, k = 10 and 100) of every relation with train + test filtered, and filtered
+pair ranking (PairRanker.metrics, Hits@1/10/100) of every test triple among the pairs of its relation, at the pose-0
+and pose-2 shapes, against torch-on-GPU restatements of the same computations timed in the same run.
 
     python profiles/rank_bench.py --out DIR [--calls 20] [--workloads pose0,pose2] [--queries tail,relation,pair]
 
@@ -23,6 +24,7 @@ import torch  # noqa: E402
 D = 80
 K = 10
 HITS = (1, 3, 10)
+PAIR_HITS = (1, 10, 100)          # a relation has about 2 * 10^5 candidate pairs at the pose shapes
 
 
 def _median_ms(fn, calls, warmup=3):
@@ -176,6 +178,62 @@ class TorchPairRestatement:
         return out_s, out_i // n, out_i % n
 
 
+class TorchPairRankRestatement:
+    """Pair ranks in eager torch: relation chunks of S_r = (z * w_r) z^T in fp32 with the upper-triangle and symmetric
+    filter mask of TorchPairRestatement, torch.sort of each relation's admissible scores and searchsorted of its test
+    triples' scores (padded per relation); per-relation means as above, self pairs left out."""
+
+    def __init__(self, test, adm, n, r, chunk_bytes=256 << 20):
+        self.n, self.r, self.adm = n, r, adm
+        self.chunk = max(1, chunk_bytes // (4 * n * n))
+        ei, et = test
+        self.e = et.numel()
+        a, b = torch.minimum(ei[0], ei[1]), torch.maximum(ei[0], ei[1])
+        eid = torch.nonzero(a != b).view(-1)
+        order = torch.argsort(et[eid], stable=True)
+        self.eid, self.a, self.b, self.rel = eid[order], a[eid][order], b[eid][order], et[eid][order]
+        cnt = torch.bincount(self.rel, minlength=r)
+        start = torch.cumsum(cnt, 0) - cnt
+        self.pos = torch.arange(self.rel.numel(), device=ei.device) - start[self.rel]
+        self.t_adm = adm[self.rel, self.a, self.b].long()
+        self.cnt = cnt.double()
+        self.et = self.rel
+        cnt_h, start_h = cnt.tolist(), start.tolist()
+        self.chunks = []
+        for c0 in range(0, r, self.chunk):
+            c1 = min(r, c0 + self.chunk)
+            q0 = start_h[c0]
+            q1 = start_h[c1 - 1] + cnt_h[c1 - 1]
+            self.chunks.append((c0, c1, q0, q1, max(1, max(cnt_h[c0:c1]))))
+
+    def ranks(self, z, w):
+        n = self.n
+        out = torch.full((self.e,), float("nan"), dtype=torch.float32, device=z.device)
+        for c0, c1, q0, q1, m in self.chunks:
+            if q1 == q0:
+                continue
+            S = torch.matmul(z[None] * w[c0:c1, None, :], z.t())
+            rl = self.rel[q0:q1] - c0
+            x = S[rl, self.a[q0:q1], self.b[q0:q1]]
+            S.masked_fill_(~self.adm[c0:c1], float("-inf"))
+            srt = torch.sort(S.view(c1 - c0, n * n), dim=1).values
+            vals = torch.full((c1 - c0, m), float("inf"), dtype=torch.float32, device=z.device)
+            vals[rl, self.pos[q0:q1]] = x
+            lt = torch.searchsorted(srt, vals)[rl, self.pos[q0:q1]]
+            le = torch.searchsorted(srt, vals, right=True)[rl, self.pos[q0:q1]]
+            opt, pess = n * n - le, n * n - lt - self.t_adm[q0:q1]       # -inf (not admissible) sorts first
+            out[self.eid[q0:q1]] = 1.0 + (opt + pess).float() * 0.5
+        return out
+
+    def metrics(self, z, w):
+        rk = self.ranks(z, w)[self.eid].double()
+        rows = [torch.zeros(self.r, dtype=torch.float64, device=z.device).index_add_(0, self.et, 1.0 / rk)]
+        for k in PAIR_HITS:
+            rows.append(torch.zeros(self.r, dtype=torch.float64, device=z.device).index_add_(0, self.et,
+                                                                                          (rk <= k).double()))
+        return torch.stack(rows) / self.cnt
+
+
 def _inputs(g, dev):
     train, test = _split(g)
     train = (train[0].to(dev), train[1].to(dev))
@@ -263,6 +321,29 @@ def run_pairs(name, g, calls, dev):
             "torch_tflops": round(flops / (t_ref * 1e-3) / 1e12, 3),
             "agreement": agree, "agree": ok,
         })
+    ranker = gb.PairRanker(test[0], test[1], n, r, filter=filt)
+    rank_ref = TorchPairRankRestatement(test, ref.adm, n, r)
+    rec = torch.empty((1 + len(PAIR_HITS), r), dtype=torch.float64, device=dev)
+    t_metrics = _median_ms(lambda: ranker.metrics(z, w, hits=PAIR_HITS, out=rec), calls)
+    t_ref = _median_ms(lambda: rank_ref.metrics(z, w), calls)
+    rk, rk_ref = ranker.ranks(z, w), rank_ref.ranks(z, w)
+    m, m_ref = ranker.metrics(z, w, hits=PAIR_HITS), rank_ref.metrics(z, w)
+    both = ~torch.isnan(rk_ref)
+    agree = {
+        "ranks_equal_fraction": float((rk[both] == rk_ref[both]).double().mean()),
+        "ranks_max_abs_diff": float((rk[both] - rk_ref[both]).abs().max()),
+        "self_pairs_nan": bool(torch.equal(torch.isnan(rk), ~both)),
+        "metrics_max_abs_diff": float((m - m_ref).abs().nan_to_num(0.0).max()),
+    }
+    ok = agree["ranks_equal_fraction"] > 0.99 and agree["self_pairs_nan"] and agree["metrics_max_abs_diff"] < 1e-3
+    flops = 2.0 * D * ranker.n_groups * n * (n - 1) / 2
+    res.append({
+        "workload": name, "query": "pair_rank", "n": n, "R": r, "D": D, "test_edges": test[0].size(1),
+        "rankable_triples": int(both.sum()), "query_relations": ranker.n_groups, "hits": list(PAIR_HITS),
+        "metrics_ms": round(t_metrics, 4), "torch_metrics_ms": round(t_ref, 4),
+        "pair_flop": flops, "metrics_tflops": round(flops / (t_metrics * 1e-3) / 1e12, 3),
+        "agreement": agree, "agree": ok,
+    })
     return res
 
 
