@@ -117,19 +117,16 @@ SIGNATURES = {
     "gn_argmax_rows": (_INT, [_P, _I64, _I64, _I32, _P, _P]),
     "gn_nc_metrics_workspace_bytes": (_SZ, [_I32]),
     "gn_nc_metrics": (_INT, [_P, _P, _I64, _I32, _P, _P, _SZ, _P]),
-    "gn_rank_csr_workspace_bytes": (_SZ, [_I64, _I32, _I32]),
-    "gn_rank_csr": (_INT, [_P, _P, _P, _I64, _I32, _I32, _P, _P, _P, _P, _P, _P, _SZ, _P]),
-    "gn_rank_query_rows": (_INT, [_P, _I64, _I32, _P, _I32, _P, _P, _P, _I64, _P, _I64, _P]),
-    "gn_rank_count": (_INT, [_P, _I64, _I32, _P, _I32, _P, _P, _P, _P, _P, _P, _P]),
+    "gn_rank_group_workspace_bytes": (_SZ, [_I64]),
+    "gn_rank_group": (_INT, [_P, _P, _P, _I64, _I32, _I32, _I32, _P, _P, _P, _P, _P, _P, _P, _SZ, _P]),
+    "gn_rank_lookup": (_INT, [_P, _P, _I32, _P, _P, _P, _P, _I64, _P, _P]),
+    "gn_rank_rows": (_INT, [_P, _I64, _P, _I64, _I32, _P, _P, _P, _P, _I64, _P, _I64, _P]),
+    "gn_rank_count": (_INT, [_P, _I64, _I32, _I32, _P, _P, _P, _P, _P, _P, _P, _P]),
     "gn_rank_max_hits": (_INT, []),
     "gn_rank_metrics": (_INT, [_P, _P, _P, _I32, _P, _I32, _P, _P]),
-    "gn_rank_topk": (_INT, [_P, _I64, _I32, _I32, _P, _P, _I64, _P, _P, _I32, _INT, _P, _P, _P]),
-    "gn_rank_pair_csr_workspace_bytes": (_SZ, [_I64]),
-    "gn_rank_pair_csr": (_INT, [_P, _P, _P, _I64, _I32, _I32, _P, _P, _P, _P, _P, _P, _P, _SZ, _P]),
-    "gn_rank_pair_lookup": (_INT, [_P, _P, _I32, _P, _P, _P, _P, _I64, _P, _P]),
-    "gn_rank_pair_rows": (_INT, [_P, _I64, _I32, _P, _P, _P, _P, _I64, _P, _I64, _P]),
-    "gn_rank_pair_count": (_INT, [_P, _I64, _I32, _I32, _P, _P, _P, _P, _P, _P, _P, _P]),
-    "gn_rank_pair_topk": (_INT, [_P, _I64, _I32, _I64, _P, _P, _P, _I32, _INT, _P, _P, _P]),
+    "gn_rank_topk": (_INT, [_P, _I64, _I32, _I64, _P, _P, _P, _I32, _INT, _P, _P, _P]),
+    "gn_rank_csr_workspace_bytes": (_SZ, [_I64]),
+    "gn_rank_csr": (_INT, [_P, _P, _P, _I64, _I32, _I32, _P, _P, _P, _P, _SZ, _P]),
     "gn_rank_rel_pairs_workspace_bytes": (_SZ, [_I64, _I32, _I32]),
     "gn_rank_rel_pairs_select": (_INT, [_P, _I64, _I32, _P, _I32, _I32, _P, _I64, _P, _P, _I32, _P, _SZ, _P]),
     "gn_rank_rel_pairs_merge": (_INT, [_P, _SZ, _I32, _I64, _I32, _INT, _P, _P, _P, _P]),

@@ -1,11 +1,12 @@
 // K16: filtered candidate ranking (OGB rank rule, per-relation MRR / Hits@k) and top-k link prediction of the
-// DistMult decoder.  Every candidate tail c of a query (s, r) is scored as one row of S = Q . z^T with
-// Q[g] = z[s_g] .* w[r_g]; the product itself is the existing dense GEMM (gn_sgemm / gn_tc_gemm).  This file holds
-// what sits around it: the (src, rel)-grouped edge structure, the query rows, the filtered rank count, the
-// per-relation reduction and the per-query top-k selection.
-// Relation queries (s, ?, t) of a directed pair score every relation r' as one row of S = P . W^T with
-// P[g] = z[s_g] .* z[t_g]; they share the count and top-k kernels, templated on how a row finds its filter row, and
-// add a pair-grouped structure (rows = distinct directed pairs, sorted by (src, dst)) and a pair lookup.
+// DistMult decoder.  Tail queries (s, r, ?) and relation queries (s, ?, t) are one computation over different data:
+// the triples are grouped by a key pair (a, b) = (s, r) or (s, t); one query row q[g] = x[a_g] .* y[b_g] per group
+// (y = w for tail queries, y = z for relation queries); one row of S = Q . C^T per group against the candidate table C
+// (z: every tail, w: every relation), computed by the existing dense GEMM (gn_sgemm / gn_tc_gemm); then the filtered
+// ranks of the group's entries, or the top k, over that row.  This file holds what sits around the product: the
+// compacted grouped structure and its lookup, the query rows, the filtered rank count, the per-relation reduction
+// and the per-query top-k selection.  Pair queries (?, r, ?) score node pairs in fused tiles (below) and read the
+// dense symmetrised filter view of gn_rank_csr.
 #include "sortkit.cuh"
 
 namespace gn {
@@ -15,15 +16,16 @@ constexpr int kTopkThreads = 256;
 constexpr int kTopkMax = 256;                  // largest k: one selected key per thread of the sort
 constexpr uint32_t kMaskedBits = 0xffffffffu;  // NaN payload no arithmetic produces: "filtered" in a top-k row
 
-// ---------------------------------------------------------------------------------------------------------------
-// grouped edge structure: rows s*R + r, entries (dst, edge id) sorted by dst inside a row (two stable counting
-// sorts: by dst, then by row), and the compacted list of non-empty rows
-// ---------------------------------------------------------------------------------------------------------------
-__global__ void rank_dst_keys_kernel(const int64_t* __restrict__ dst, int64_t n, int32_t* __restrict__ key) {
-  const int64_t e = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
-  if (e < n) key[e] = int32_t(dst[e]);
+__global__ void rank_gather_keys_kernel(const int64_t* __restrict__ v, const int32_t* __restrict__ perm, int64_t n,
+                                        int32_t* __restrict__ key) {
+  const int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (i < n) key[i] = int32_t(v[perm ? perm[i] : int32_t(i)]);
 }
 
+// ---------------------------------------------------------------------------------------------------------------
+// dense grouped structure (the symmetrised filter view of pair queries): rows s*R + r, entries (dst, edge id) sorted
+// by dst inside a row (two stable counting sorts: by dst, then by row)
+// ---------------------------------------------------------------------------------------------------------------
 __global__ void rank_row_keys_kernel(const int64_t* __restrict__ src, const int64_t* __restrict__ etype,
                                      const int32_t* __restrict__ perm, int64_t n, int32_t n_rel,
                                      int32_t* __restrict__ key) {
@@ -33,168 +35,93 @@ __global__ void rank_row_keys_kernel(const int64_t* __restrict__ src, const int6
   key[i] = int32_t(src[e]) * n_rel + int32_t(etype[e]);
 }
 
-__global__ void rank_fill_kernel(const int64_t* __restrict__ dst, const int32_t* __restrict__ eid, int64_t n,
-                                 int32_t* __restrict__ ent_dst) {
-  const int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
-  if (i < n) ent_dst[i] = int32_t(dst[eid[i]]);
-}
-
-__global__ void rank_row_flags_kernel(const int32_t* __restrict__ rowptr, int32_t n_rows, int32_t* __restrict__ flag) {
-  const int r = blockIdx.x * blockDim.x + threadIdx.x;
-  if (r < n_rows) flag[r] = rowptr[r + 1] > rowptr[r] ? 1 : 0;
-}
-
-__global__ void rank_groups_kernel(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ pos, int32_t n_rows,
-                                   int32_t* __restrict__ group_row) {
-  const int r = blockIdx.x * blockDim.x + threadIdx.x;
-  if (r < n_rows && rowptr[r + 1] > rowptr[r]) group_row[pos[r]] = r;
-}
-
 // ---------------------------------------------------------------------------------------------------------------
-// pair-grouped structure: entries ordered by (src, dst, rel) with three stable counting sorts (by rel, by dst, by
-// src), rows = the distinct directed pairs in that order, entries (rel, edge id) sorted by rel inside a row.  Rows
-// are compacted pairs, not s*n + t: n^2 does not fit int32 for general n.
+// compacted grouped structure of three columns (a, b, c): entries ordered by (a, b, c) with three stable counting
+// sorts (by c, by b, by a), rows = the distinct key pairs (a, b) in that order, entries (c, edge id) sorted by c
+// inside a row.  Rows are compacted, not a*nb + b: n^2 does not fit int32 for general n.
 // ---------------------------------------------------------------------------------------------------------------
-__global__ void rank_gather_keys_kernel(const int64_t* __restrict__ v, const int32_t* __restrict__ perm, int64_t n,
-                                        int32_t* __restrict__ key) {
-  const int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
-  if (i < n) key[i] = int32_t(v[perm ? perm[i] : int32_t(i)]);
-}
-
-__global__ void rank_pair_heads_kernel(const int64_t* __restrict__ src, const int64_t* __restrict__ dst,
-                                       const int32_t* __restrict__ eid, int64_t n, int32_t* __restrict__ flag) {
+__global__ void rank_group_heads_kernel(const int64_t* __restrict__ a, const int64_t* __restrict__ b,
+                                        const int32_t* __restrict__ eid, int64_t n, int32_t* __restrict__ flag) {
   const int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= n) return;
   const int32_t e = eid[i];
-  flag[i] = i == 0 || src[e] != src[eid[i - 1]] || dst[e] != dst[eid[i - 1]] ? 1 : 0;
+  flag[i] = i == 0 || a[e] != a[eid[i - 1]] || b[e] != b[eid[i - 1]] ? 1 : 0;
 }
 
-__global__ void rank_pair_fill_kernel(const int64_t* __restrict__ src, const int64_t* __restrict__ dst,
-                                      const int64_t* __restrict__ etype, const int32_t* __restrict__ eid,
-                                      const int32_t* __restrict__ flag, const int32_t* __restrict__ pos, int64_t n,
-                                      int32_t* __restrict__ rowptr, int32_t* __restrict__ pair_src,
-                                      int32_t* __restrict__ pair_dst, int32_t* __restrict__ ent_rel) {
+__global__ void rank_group_fill_kernel(const int64_t* __restrict__ a, const int64_t* __restrict__ b,
+                                       const int64_t* __restrict__ c, const int32_t* __restrict__ eid,
+                                       const int32_t* __restrict__ flag, const int32_t* __restrict__ pos, int64_t n,
+                                       int32_t* __restrict__ rowptr, int32_t* __restrict__ group_a,
+                                       int32_t* __restrict__ group_b, int32_t* __restrict__ ent_c) {
   const int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= n) return;
   const int32_t e = eid[i];
-  ent_rel[i] = int32_t(etype[e]);
+  ent_c[i] = int32_t(c[e]);
   if (flag[i]) {
     const int32_t p = pos[i];
     rowptr[p] = int32_t(i);
-    pair_src[p] = int32_t(src[e]);
-    pair_dst[p] = int32_t(dst[e]);
+    group_a[p] = int32_t(a[e]);
+    group_b[p] = int32_t(b[e]);
   }
   if (i == n - 1) rowptr[pos[i] + flag[i]] = int32_t(n);
 }
 
-// row of the filter's pair (s, t) by binary search over its (src, dst)-sorted pairs, or -1
-__global__ void rank_pair_lookup_kernel(const int32_t* __restrict__ f_src, const int32_t* __restrict__ f_dst,
-                                        int32_t n_fpairs, const int32_t* __restrict__ pair_src,
-                                        const int32_t* __restrict__ pair_dst, const int64_t* __restrict__ src,
-                                        const int64_t* __restrict__ dst, int64_t count, int32_t* __restrict__ row) {
+// row of the key pair (a, b) in a structure by binary search over its (a, b)-sorted groups, or -1
+__global__ void rank_lookup_kernel(const int32_t* __restrict__ f_a, const int32_t* __restrict__ f_b, int32_t n_f,
+                                   const int32_t* __restrict__ a32, const int32_t* __restrict__ b32,
+                                   const int64_t* __restrict__ a64, const int64_t* __restrict__ b64, int64_t count,
+                                   int32_t* __restrict__ row) {
   const int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= count) return;
-  const int32_t s = pair_src ? pair_src[i] : int32_t(src[i]);
-  const int32_t t = pair_src ? pair_dst[i] : int32_t(dst[i]);
-  int lo = 0, hi = n_fpairs;
+  const int32_t s = a32 ? a32[i] : int32_t(a64[i]);
+  const int32_t t = a32 ? b32[i] : int32_t(b64[i]);
+  int lo = 0, hi = n_f;
   while (lo < hi) {
     const int mid = lo + ((hi - lo) >> 1);
-    const int32_t ms = f_src[mid];
-    if (ms < s || (ms == s && f_dst[mid] < t)) lo = mid + 1;
+    const int32_t ms = f_a[mid];
+    if (ms < s || (ms == s && f_b[mid] < t)) lo = mid + 1;
     else hi = mid;
   }
-  row[i] = (lo < n_fpairs && f_src[lo] == s && f_dst[lo] == t) ? lo : -1;
+  row[i] = (lo < n_f && f_a[lo] == s && f_b[lo] == t) ? lo : -1;
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-// query rows q[i, :] = a_i .* b_i.  Tail queries: a = z[s], b = w[r], (s, r) from a group row id s*R + r or from two
-// index lists.  Relation queries: a = z[s], b = z[t], (s, t) from a pair-grouped structure or from two index lists.
+// query rows q[i, :] = x[a_i] .* y[b_i], (a_i, b_i) from a grouped structure's key columns (int32) or from two index
+// lists (int64)
 // ---------------------------------------------------------------------------------------------------------------
-struct TailOperands {
-  const float* z;
-  int64_t ldz;
-  const float* w;
-  int D;
-  int32_t n_rel;
-  const int32_t* group_row;
-  const int64_t* node;
-  const int64_t* rel;
-  __device__ __forceinline__ void at(int64_t i, const float*& a, const float*& b) const {
-    int64_t s, r;
-    if (group_row != nullptr) {
-      const int32_t g = group_row[i];
-      s = g / n_rel;
-      r = g - s * n_rel;
-    } else {
-      s = node[i];
-      r = rel[i];
-    }
-    a = z + s * ldz;
-    b = w + r * D;
-  }
-};
-
-struct PairOperands {
-  const float* z;
-  int64_t ldz;
-  const int32_t* pair_src;    // group pairs, or nullptr: the index lists
-  const int32_t* pair_dst;
-  const int64_t* src;
-  const int64_t* dst;
-  __device__ __forceinline__ void at(int64_t i, const float*& a, const float*& b) const {
-    const int64_t s = pair_src ? int64_t(pair_src[i]) : src[i];
-    const int64_t t = pair_src ? int64_t(pair_dst[i]) : dst[i];
-    a = z + s * ldz;
-    b = z + t * ldz;
-  }
-};
-
-template <class Operands>
-__global__ void rank_query_rows_kernel(const Operands ops, int D, int64_t count, float* __restrict__ q, int64_t ldq) {
+__global__ void rank_rows_kernel(const float* __restrict__ x, int64_t ldx, const float* __restrict__ y, int64_t ldy,
+                                 int D, const int32_t* __restrict__ a32, const int32_t* __restrict__ b32,
+                                 const int64_t* __restrict__ a64, const int64_t* __restrict__ b64, int64_t count,
+                                 float* __restrict__ q, int64_t ldq) {
   const int64_t t = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
   if (t >= count * D) return;
   const int64_t i = t / D;
   const int f = int(t - i * D);
-  const float *a, *b;
-  ops.at(i, a, b);
-  q[i * ldq + f] = a[f] * b[f];
+  const int64_t a = a32 ? int64_t(a32[i]) : a64[i];
+  const int64_t b = a32 ? int64_t(b32[i]) : b64[i];
+  q[i * ldq + f] = x[a * ldx + f] * y[b * ldy + f];
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-// filtered rank: one warp per group (a row of S), the group's targets in turn.  opt / pess count the candidates
-// c != t above / at-or-above S(t) over the whole row, then the distinct filtered candidates other than t that met
-// the same comparisons are taken back out.  S(t) is read from the same row as every S(c).  Rows says where group g's
-// targets and filter entries are: tail groups use the row s*R + r of both structures, relation groups (pairs) their
-// own compacted row and the filter row found by gn_rank_pair_lookup (-1: the pair has no filtered triple).
+// filtered rank: one warp per group g (row g of S), the group's entries (target candidates) in turn.  opt / pess
+// count the candidates c != t above / at-or-above S(t) over the whole row, then the distinct filtered candidates
+// other than t that met the same comparisons are taken back out.  S(t) is read from the same row as every S(c).
+// f_row[g] is the group's row in the filter (gn_rank_lookup; -1: the filter holds no triple of its key pair).
 // ---------------------------------------------------------------------------------------------------------------
 constexpr int kCountWarps = 8;
 
-struct TailRows {
-  const int32_t* group_row;
-  bool filtered;
-  __device__ __forceinline__ int32_t query(int g) const { return group_row[g]; }
-  __device__ __forceinline__ int32_t filter(int g) const { return filtered ? group_row[g] : -1; }
-};
-
-struct PairRows {
-  const int32_t* f_row;       // nullptr: no filter
-  __device__ __forceinline__ int32_t query(int g) const { return g; }
-  __device__ __forceinline__ int32_t filter(int g) const { return f_row ? f_row[g] : -1; }
-};
-
-template <class Rows>
 __global__ void __launch_bounds__(kCountWarps * 32) rank_count_kernel(
-    const float* __restrict__ S, int64_t lds, int32_t n, const Rows rows, int32_t n_groups,
-    const int32_t* __restrict__ q_rowptr, const int32_t* __restrict__ q_dst, const int32_t* __restrict__ q_eid,
-    const int32_t* __restrict__ f_rowptr, const int32_t* __restrict__ f_dst, float* __restrict__ rank) {
+    const float* __restrict__ S, int64_t lds, int32_t n, int32_t n_groups, const int32_t* __restrict__ q_rowptr,
+    const int32_t* __restrict__ q_c, const int32_t* __restrict__ q_eid, const int32_t* __restrict__ f_row,
+    const int32_t* __restrict__ f_rowptr, const int32_t* __restrict__ f_c, float* __restrict__ rank) {
   const int lane = threadIdx.x & 31;
   const int g = blockIdx.x * kCountWarps + (threadIdx.x >> 5);
   if (g >= n_groups) return;
-  const int32_t row = rows.query(g), frow = rows.filter(g);
+  const int32_t frow = f_row ? f_row[g] : -1;
   const float* srow = S + int64_t(g) * lds;
   const int f0 = frow >= 0 ? f_rowptr[frow] : 0, f1 = frow >= 0 ? f_rowptr[frow + 1] : 0;
-  for (int j = q_rowptr[row]; j < q_rowptr[row + 1]; ++j) {
-    const int t = q_dst[j];
+  for (int j = q_rowptr[g]; j < q_rowptr[g + 1]; ++j) {
+    const int t = q_c[j];
     const float st = srow[t];
     int opt = 0, pess = 0;
     for (int c = lane; c < n; c += 32) {
@@ -203,8 +130,8 @@ __global__ void __launch_bounds__(kCountWarps * 32) rank_count_kernel(
       pess += (c != t) & (v >= st);
     }
     for (int k = f0 + lane; k < f1; k += 32) {
-      const int c = f_dst[k];
-      if (c == t || (k > f0 && f_dst[k - 1] == c)) continue;   // the target itself; duplicates count once
+      const int c = f_c[k];
+      if (c == t || (k > f0 && f_c[k - 1] == c)) continue;   // the target itself; duplicates count once
       const float v = srow[c];
       opt -= v > st;
       pess -= v >= st;
@@ -401,38 +328,24 @@ __device__ __forceinline__ float topk_out_score(uint64_t key, int sigmoid) {
   return v;
 }
 
-// the filter row of query row qi (-1: none): s*R + r of a tail query, the looked-up pair row of a relation query
-struct TailFilterRow {
-  const int64_t* node;
-  const int64_t* rel;
-  int32_t n_rel;
-  bool filtered;
-  __device__ __forceinline__ int64_t operator()(int64_t qi) const { return filtered ? node[qi] * n_rel + rel[qi] : -1; }
-};
-
-struct PairFilterRow {
-  const int32_t* f_row;       // nullptr: no filter
-  __device__ __forceinline__ int64_t operator()(int64_t qi) const { return f_row ? f_row[qi] : -1; }
-};
-
 struct RowKeys {
   const float* srow;
   __device__ __forceinline__ uint64_t operator()(int c) const { return topk_key(srow, c); }
 };
 
-template <class FilterRow>
+// f_row[qi]: the filter row of query row qi (gn_rank_lookup; -1: none), or f_row == nullptr: no filter
 __global__ void __launch_bounds__(kTopkThreads) rank_topk_kernel(float* __restrict__ S, int64_t lds, int32_t n,
-                                                                 const FilterRow filter_row,
+                                                                 const int32_t* __restrict__ f_row,
                                                                  const int32_t* __restrict__ f_rowptr,
-                                                                 const int32_t* __restrict__ f_dst, int k, int sigmoid,
+                                                                 const int32_t* __restrict__ f_c, int k, int sigmoid,
                                                                  float* __restrict__ out_score,
                                                                  int64_t* __restrict__ out_id) {
   const int tid = threadIdx.x;
   const int64_t qi = blockIdx.x;
   float* srow = S + qi * lds;
-  const int64_t row = filter_row(qi);
+  const int32_t row = f_row ? f_row[qi] : -1;
   if (row >= 0) {
-    for (int j = f_rowptr[row] + tid; j < f_rowptr[row + 1]; j += kTopkThreads) srow[f_dst[j]] = __uint_as_float(kMaskedBits);
+    for (int j = f_rowptr[row] + tid; j < f_rowptr[row + 1]; j += kTopkThreads) srow[f_c[j]] = __uint_as_float(kMaskedBits);
   }
   __syncthreads();
   const uint64_t* sel = topk_select(RowKeys{srow}, n, k);
@@ -768,18 +681,16 @@ using namespace gn;
 
 extern "C" {
 
-size_t gn_rank_csr_workspace_bytes(int64_t n_edges, int32_t n_nodes, int32_t n_rel) {
+size_t gn_rank_csr_workspace_bytes(int64_t n_edges) {
   const size_t E = size_t(n_edges > 0 ? n_edges : 1);
-  const int64_t rows = int64_t(n_nodes > 0 ? n_nodes : 1) * (n_rel > 0 ? n_rel : 1);
-  return 4 * align_up(E * 4) + sort_ws_bytes(n_edges) + 2 * align_up(size_t(rows) * 4) + scan_ws_bytes(rows) + 4096;
+  return 4 * align_up(E * 4) + sort_ws_bytes(n_edges) + 4096;
 }
 
 int gn_rank_csr(const int64_t* src, const int64_t* dst, const int64_t* etype, int64_t n_edges, int32_t n_nodes,
-                int32_t n_rel, int32_t* rowptr, int32_t* ent_dst, int32_t* ent_eid, int32_t* group_row,
-                int32_t* n_groups, void* ws, size_t ws_bytes, void* stream) {
+                int32_t n_rel, int32_t* rowptr, int32_t* ent_dst, int32_t* ent_eid, void* ws, size_t ws_bytes,
+                void* stream) {
   if (n_edges < 0 || n_nodes <= 0 || n_rel <= 0 || !rowptr) return GN_ERR_ARG;
   if (n_edges > 0 && (!src || !dst || !etype || !ent_dst || !ent_eid)) return GN_ERR_ARG;
-  if ((group_row == nullptr) != (n_groups == nullptr)) return GN_ERR_ARG;
   if (n_edges >= (int64_t(1) << 31) || int64_t(n_nodes) * n_rel >= (int64_t(1) << 31)) return GN_ERR_RANGE;
   cudaStream_t st = as_stream(stream);
   const int32_t n_rows = n_nodes * n_rel;
@@ -789,52 +700,96 @@ int gn_rank_csr(const int64_t* src, const int64_t* dst, const int64_t* etype, in
   int32_t* sorted1 = a.take<int32_t>(Ea);
   int32_t* perm1 = a.take<int32_t>(Ea);
   int32_t* key2 = a.take<int32_t>(Ea);
-  int32_t* flag = a.take<int32_t>(size_t(n_rows));
-  int32_t* pos = a.take<int32_t>(size_t(n_rows));
   if (!a.ok()) return GN_ERR_WORKSPACE;
   void* rest = a.base + a.off;
   const size_t rest_bytes = a.cap - a.off;
   int32_t* sorted2 = sorted1;                        // free once key2 is formed
   if (n_edges > 0) {
     const unsigned ge = (unsigned)ceil_div(n_edges, 256);
-    GN_LAUNCH(rank_dst_keys_kernel, ge, 256, 0, st, dst, n_edges, key1);
+    GN_LAUNCH(rank_gather_keys_kernel, ge, 256, 0, st, dst, (const int32_t*)nullptr, n_edges, key1);
     GN_CHECK(sort_pairs(key1, nullptr, sorted1, perm1, n_edges, bits_for(n_nodes > 1 ? n_nodes : 2), rest,
                         rest_bytes, st));
     GN_LAUNCH(rank_row_keys_kernel, ge, 256, 0, st, src, etype, (const int32_t*)perm1, n_edges, n_rel, key2);
     GN_CHECK(sort_pairs(key2, perm1, sorted2, ent_eid, n_edges, bits_for(n_rows > 1 ? n_rows : 2), rest, rest_bytes,
                         st));
-    GN_LAUNCH(rank_fill_kernel, ge, 256, 0, st, dst, (const int32_t*)ent_eid, n_edges, ent_dst);
+    GN_LAUNCH(rank_gather_keys_kernel, ge, 256, 0, st, dst, (const int32_t*)ent_eid, n_edges, ent_dst);
   }
   GN_CHECK(rowptr_from_sorted(sorted2, n_edges, n_rows, rowptr, st));
-  if (group_row != nullptr) {
-    const unsigned gr = (unsigned)ceil_div(n_rows, 256);
-    GN_LAUNCH(rank_row_flags_kernel, gr, 256, 0, st, (const int32_t*)rowptr, n_rows, flag);
-    GN_CHECK(exclusive_scan_i32(flag, pos, n_rows, n_groups, rest, rest_bytes, st));
-    GN_LAUNCH(rank_groups_kernel, gr, 256, 0, st, (const int32_t*)rowptr, (const int32_t*)pos, n_rows, group_row);
+  return GN_OK;
+}
+
+size_t gn_rank_group_workspace_bytes(int64_t n_edges) {
+  const size_t E = size_t(n_edges > 0 ? n_edges : 1);
+  return 4 * align_up(E * 4) + sort_ws_bytes(n_edges) + scan_ws_bytes(n_edges) + 4096;
+}
+
+int gn_rank_group(const int64_t* a, const int64_t* b, const int64_t* c, int64_t n_edges, int32_t na, int32_t nb,
+                  int32_t nc, int32_t* rowptr, int32_t* group_a, int32_t* group_b, int32_t* ent_c, int32_t* ent_eid,
+                  int32_t* n_groups, void* ws, size_t ws_bytes, void* stream) {
+  if (n_edges < 0 || na <= 0 || nb <= 0 || nc <= 0 || !rowptr || !n_groups) return GN_ERR_ARG;
+  if (n_edges > 0 && (!a || !b || !c || !group_a || !group_b || !ent_c || !ent_eid)) return GN_ERR_ARG;
+  if (n_edges >= (int64_t(1) << 31)) return GN_ERR_RANGE;
+  cudaStream_t st = as_stream(stream);
+  if (n_edges == 0) {
+    if (cudaMemsetAsync(rowptr, 0, 4, st) != cudaSuccess || cudaMemsetAsync(n_groups, 0, 4, st) != cudaSuccess)
+      return GN_ERR_CUDA;
+    return GN_OK;
   }
+  Arena ar(ws, ws_bytes);
+  int32_t* key = ar.take<int32_t>(size_t(n_edges));
+  int32_t* sorted = ar.take<int32_t>(size_t(n_edges));
+  int32_t* perm1 = ar.take<int32_t>(size_t(n_edges));
+  int32_t* perm2 = ar.take<int32_t>(size_t(n_edges));
+  if (!ar.ok()) return GN_ERR_WORKSPACE;
+  void* rest = ar.base + ar.off;
+  const size_t rest_bytes = ar.cap - ar.off;
+  const unsigned ge = (unsigned)ceil_div(n_edges, 256);
+  // stable passes by c, then b, then a: entries in (a, b, c) order
+  GN_LAUNCH(rank_gather_keys_kernel, ge, 256, 0, st, c, (const int32_t*)nullptr, n_edges, key);
+  GN_CHECK(sort_pairs(key, nullptr, sorted, perm1, n_edges, bits_for(nc > 1 ? nc : 2), rest, rest_bytes, st));
+  GN_LAUNCH(rank_gather_keys_kernel, ge, 256, 0, st, b, (const int32_t*)perm1, n_edges, key);
+  GN_CHECK(sort_pairs(key, perm1, sorted, perm2, n_edges, bits_for(nb > 1 ? nb : 2), rest, rest_bytes, st));
+  GN_LAUNCH(rank_gather_keys_kernel, ge, 256, 0, st, a, (const int32_t*)perm2, n_edges, key);
+  GN_CHECK(sort_pairs(key, perm2, sorted, ent_eid, n_edges, bits_for(na > 1 ? na : 2), rest, rest_bytes, st));
+  // run heads -> compacted group rows
+  int32_t* flag = key;
+  int32_t* pos = sorted;
+  GN_LAUNCH(rank_group_heads_kernel, ge, 256, 0, st, a, b, (const int32_t*)ent_eid, n_edges, flag);
+  GN_CHECK(exclusive_scan_i32(flag, pos, n_edges, n_groups, rest, rest_bytes, st));
+  GN_LAUNCH(rank_group_fill_kernel, ge, 256, 0, st, a, b, c, (const int32_t*)ent_eid, (const int32_t*)flag,
+            (const int32_t*)pos, n_edges, rowptr, group_a, group_b, ent_c);
   return GN_OK;
 }
 
-int gn_rank_query_rows(const float* z, int64_t ldz, int32_t D, const float* w, int32_t n_rel, const int32_t* group_row,
-                       const int64_t* node, const int64_t* rel, int64_t count, float* q, int64_t ldq, void* stream) {
-  if (count < 0 || D <= 0 || n_rel <= 0 || ldq < D) return GN_ERR_ARG;
+int gn_rank_lookup(const int32_t* f_a, const int32_t* f_b, int32_t n_f, const int32_t* a32, const int32_t* b32,
+                   const int64_t* a64, const int64_t* b64, int64_t count, int32_t* row, void* stream) {
+  if (count < 0 || n_f < 0) return GN_ERR_ARG;
   if (count == 0) return GN_OK;
-  if (!z || !w || !q || (!group_row && (!node || !rel))) return GN_ERR_ARG;
-  const TailOperands ops{z, ldz, w, D, n_rel, group_row, node, rel};
-  GN_LAUNCH(rank_query_rows_kernel<TailOperands>, (unsigned)ceil_div(count * D, 256), 256, 0, as_stream(stream), ops,
-            D, count, q, ldq);
+  if (!row || (n_f > 0 && (!f_a || !f_b)) || (a32 ? !b32 : (!a64 || !b64))) return GN_ERR_ARG;
+  GN_LAUNCH(rank_lookup_kernel, (unsigned)ceil_div(count, 256), 256, 0, as_stream(stream), f_a, f_b, n_f, a32, b32,
+            a64, b64, count, row);
   return GN_OK;
 }
 
-int gn_rank_count(const float* S, int64_t lds, int32_t n_nodes, const int32_t* group_row, int32_t n_groups,
-                  const int32_t* q_rowptr, const int32_t* q_dst, const int32_t* q_eid, const int32_t* f_rowptr,
-                  const int32_t* f_dst, float* rank, void* stream) {
-  if (n_groups < 0 || n_nodes <= 0 || lds < n_nodes) return GN_ERR_ARG;
+int gn_rank_rows(const float* x, int64_t ldx, const float* y, int64_t ldy, int32_t D, const int32_t* a32,
+                 const int32_t* b32, const int64_t* a64, const int64_t* b64, int64_t count, float* q, int64_t ldq,
+                 void* stream) {
+  if (count < 0 || D <= 0 || ldq < D) return GN_ERR_ARG;
+  if (count == 0) return GN_OK;
+  if (!x || !y || !q || (a32 ? !b32 : (!a64 || !b64))) return GN_ERR_ARG;
+  GN_LAUNCH(rank_rows_kernel, (unsigned)ceil_div(count * D, 256), 256, 0, as_stream(stream), x, ldx, y, ldy, D, a32,
+            b32, a64, b64, count, q, ldq);
+  return GN_OK;
+}
+
+int gn_rank_count(const float* S, int64_t lds, int32_t n_cand, int32_t n_groups, const int32_t* q_rowptr,
+                  const int32_t* q_c, const int32_t* q_eid, const int32_t* f_row, const int32_t* f_rowptr,
+                  const int32_t* f_c, float* rank, void* stream) {
+  if (n_groups < 0 || n_cand <= 0 || lds < n_cand) return GN_ERR_ARG;
   if (n_groups == 0) return GN_OK;
-  if (!S || !group_row || !q_rowptr || !q_dst || !q_eid || !rank || (f_rowptr && !f_dst)) return GN_ERR_ARG;
-  const TailRows rows{group_row, f_rowptr != nullptr};
-  GN_LAUNCH(rank_count_kernel<TailRows>, (unsigned)ceil_div(n_groups, kCountWarps), kCountWarps * 32, 0,
-            as_stream(stream), S, lds, n_nodes, rows, n_groups, q_rowptr, q_dst, q_eid, f_rowptr, f_dst, rank);
+  if (!S || !q_rowptr || !q_c || !q_eid || !rank || (f_row && (!f_rowptr || !f_c))) return GN_ERR_ARG;
+  GN_LAUNCH(rank_count_kernel, (unsigned)ceil_div(n_groups, kCountWarps), kCountWarps * 32, 0, as_stream(stream), S,
+            lds, n_cand, n_groups, q_rowptr, q_c, q_eid, f_row, f_rowptr, f_c, rank);
   return GN_OK;
 }
 
@@ -852,107 +807,14 @@ int gn_rank_metrics(const float* rank, const int32_t* rel_rowptr, const int32_t*
   return GN_OK;
 }
 
-int gn_rank_topk(float* S, int64_t lds, int32_t n_nodes, int32_t n_rel, const int64_t* node, const int64_t* rel,
-                 int64_t count, const int32_t* f_rowptr, const int32_t* f_dst, int32_t k, int sigmoid,
-                 float* out_score, int64_t* out_id, void* stream) {
-  if (count < 0 || n_nodes <= 0 || n_rel <= 0 || lds < n_nodes || k < 1 || k > kTopkMax) return GN_ERR_ARG;
+int gn_rank_topk(float* S, int64_t lds, int32_t n_cand, int64_t count, const int32_t* f_row, const int32_t* f_rowptr,
+                 const int32_t* f_c, int32_t k, int sigmoid, float* out_score, int64_t* out_id, void* stream) {
+  if (count < 0 || n_cand <= 0 || lds < n_cand || k < 1 || k > kTopkMax) return GN_ERR_ARG;
   if (count == 0) return GN_OK;
   if (count >= (int64_t(1) << 31)) return GN_ERR_RANGE;
-  if (!S || !node || !rel || !out_score || !out_id || (f_rowptr && !f_dst)) return GN_ERR_ARG;
-  const TailFilterRow frow{node, rel, n_rel, f_rowptr != nullptr};
-  GN_LAUNCH(rank_topk_kernel<TailFilterRow>, (unsigned)count, kTopkThreads, 0, as_stream(stream), S, lds, n_nodes,
-            frow, f_rowptr, f_dst, k, sigmoid, out_score, out_id);
-  return GN_OK;
-}
-
-size_t gn_rank_pair_csr_workspace_bytes(int64_t n_edges) {
-  const size_t E = size_t(n_edges > 0 ? n_edges : 1);
-  return 4 * align_up(E * 4) + sort_ws_bytes(n_edges) + scan_ws_bytes(n_edges) + 4096;
-}
-
-int gn_rank_pair_csr(const int64_t* src, const int64_t* dst, const int64_t* etype, int64_t n_edges, int32_t n_nodes,
-                     int32_t n_rel, int32_t* rowptr, int32_t* pair_src, int32_t* pair_dst, int32_t* ent_rel,
-                     int32_t* ent_eid, int32_t* n_pairs, void* ws, size_t ws_bytes, void* stream) {
-  if (n_edges < 0 || n_nodes <= 0 || n_rel <= 0 || !rowptr || !n_pairs) return GN_ERR_ARG;
-  if (n_edges > 0 && (!src || !dst || !etype || !pair_src || !pair_dst || !ent_rel || !ent_eid)) return GN_ERR_ARG;
-  if (n_edges >= (int64_t(1) << 31)) return GN_ERR_RANGE;
-  cudaStream_t st = as_stream(stream);
-  if (n_edges == 0) {
-    if (cudaMemsetAsync(rowptr, 0, 4, st) != cudaSuccess || cudaMemsetAsync(n_pairs, 0, 4, st) != cudaSuccess)
-      return GN_ERR_CUDA;
-    return GN_OK;
-  }
-  Arena a(ws, ws_bytes);
-  int32_t* key = a.take<int32_t>(size_t(n_edges));
-  int32_t* sorted = a.take<int32_t>(size_t(n_edges));
-  int32_t* perm1 = a.take<int32_t>(size_t(n_edges));
-  int32_t* perm2 = a.take<int32_t>(size_t(n_edges));
-  if (!a.ok()) return GN_ERR_WORKSPACE;
-  void* rest = a.base + a.off;
-  const size_t rest_bytes = a.cap - a.off;
-  const unsigned ge = (unsigned)ceil_div(n_edges, 256);
-  const int node_bits = bits_for(n_nodes > 1 ? n_nodes : 2);
-  // stable passes by rel, then dst, then src: entries in (src, dst, rel) order
-  GN_LAUNCH(rank_gather_keys_kernel, ge, 256, 0, st, etype, (const int32_t*)nullptr, n_edges, key);
-  GN_CHECK(sort_pairs(key, nullptr, sorted, perm1, n_edges, bits_for(n_rel > 1 ? n_rel : 2), rest, rest_bytes, st));
-  GN_LAUNCH(rank_gather_keys_kernel, ge, 256, 0, st, dst, (const int32_t*)perm1, n_edges, key);
-  GN_CHECK(sort_pairs(key, perm1, sorted, perm2, n_edges, node_bits, rest, rest_bytes, st));
-  GN_LAUNCH(rank_gather_keys_kernel, ge, 256, 0, st, src, (const int32_t*)perm2, n_edges, key);
-  GN_CHECK(sort_pairs(key, perm2, sorted, ent_eid, n_edges, node_bits, rest, rest_bytes, st));
-  // run heads -> compacted pair rows
-  int32_t* flag = key;
-  int32_t* pos = sorted;
-  GN_LAUNCH(rank_pair_heads_kernel, ge, 256, 0, st, src, dst, (const int32_t*)ent_eid, n_edges, flag);
-  GN_CHECK(exclusive_scan_i32(flag, pos, n_edges, n_pairs, rest, rest_bytes, st));
-  GN_LAUNCH(rank_pair_fill_kernel, ge, 256, 0, st, src, dst, etype, (const int32_t*)ent_eid, (const int32_t*)flag,
-            (const int32_t*)pos, n_edges, rowptr, pair_src, pair_dst, ent_rel);
-  return GN_OK;
-}
-
-int gn_rank_pair_lookup(const int32_t* f_src, const int32_t* f_dst, int32_t n_fpairs, const int32_t* pair_src,
-                        const int32_t* pair_dst, const int64_t* src, const int64_t* dst, int64_t count, int32_t* row,
-                        void* stream) {
-  if (count < 0 || n_fpairs < 0) return GN_ERR_ARG;
-  if (count == 0) return GN_OK;
-  if (!row || (n_fpairs > 0 && (!f_src || !f_dst)) || (pair_src ? !pair_dst : (!src || !dst))) return GN_ERR_ARG;
-  GN_LAUNCH(rank_pair_lookup_kernel, (unsigned)ceil_div(count, 256), 256, 0, as_stream(stream), f_src, f_dst,
-            n_fpairs, pair_src, pair_dst, src, dst, count, row);
-  return GN_OK;
-}
-
-int gn_rank_pair_rows(const float* z, int64_t ldz, int32_t D, const int32_t* pair_src, const int32_t* pair_dst,
-                      const int64_t* src, const int64_t* dst, int64_t count, float* p, int64_t ldp, void* stream) {
-  if (count < 0 || D <= 0 || ldp < D) return GN_ERR_ARG;
-  if (count == 0) return GN_OK;
-  if (!z || !p || (pair_src ? !pair_dst : (!src || !dst))) return GN_ERR_ARG;
-  const PairOperands ops{z, ldz, pair_src, pair_dst, src, dst};
-  GN_LAUNCH(rank_query_rows_kernel<PairOperands>, (unsigned)ceil_div(count * D, 256), 256, 0, as_stream(stream), ops,
-            D, count, p, ldp);
-  return GN_OK;
-}
-
-int gn_rank_pair_count(const float* S, int64_t lds, int32_t n_rel, int32_t n_pairs, const int32_t* q_rowptr,
-                       const int32_t* q_rel, const int32_t* q_eid, const int32_t* f_row, const int32_t* f_rowptr,
-                       const int32_t* f_rel, float* rank, void* stream) {
-  if (n_pairs < 0 || n_rel <= 0 || lds < n_rel) return GN_ERR_ARG;
-  if (n_pairs == 0) return GN_OK;
-  if (!S || !q_rowptr || !q_rel || !q_eid || !rank || (f_row && (!f_rowptr || !f_rel))) return GN_ERR_ARG;
-  const PairRows rows{f_row};
-  GN_LAUNCH(rank_count_kernel<PairRows>, (unsigned)ceil_div(n_pairs, kCountWarps), kCountWarps * 32, 0,
-            as_stream(stream), S, lds, n_rel, rows, n_pairs, q_rowptr, q_rel, q_eid, f_rowptr, f_rel, rank);
-  return GN_OK;
-}
-
-int gn_rank_pair_topk(float* S, int64_t lds, int32_t n_rel, int64_t count, const int32_t* f_row,
-                      const int32_t* f_rowptr, const int32_t* f_rel, int32_t k, int sigmoid, float* out_score,
-                      int64_t* out_id, void* stream) {
-  if (count < 0 || n_rel <= 0 || lds < n_rel || k < 1 || k > kTopkMax) return GN_ERR_ARG;
-  if (count == 0) return GN_OK;
-  if (count >= (int64_t(1) << 31)) return GN_ERR_RANGE;
-  if (!S || !out_score || !out_id || (f_row && (!f_rowptr || !f_rel))) return GN_ERR_ARG;
-  const PairFilterRow frow{f_row};
-  GN_LAUNCH(rank_topk_kernel<PairFilterRow>, (unsigned)count, kTopkThreads, 0, as_stream(stream), S, lds, n_rel, frow,
-            f_rowptr, f_rel, k, sigmoid, out_score, out_id);
+  if (!S || !out_score || !out_id || (f_row && (!f_rowptr || !f_c))) return GN_ERR_ARG;
+  GN_LAUNCH(rank_topk_kernel, (unsigned)count, kTopkThreads, 0, as_stream(stream), S, lds, n_cand, f_row, f_rowptr,
+            f_c, k, sigmoid, out_score, out_id);
   return GN_OK;
 }
 

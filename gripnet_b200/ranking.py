@@ -96,60 +96,74 @@ def _sizes(num_nodes, num_relations):
     return n, r
 
 
+def _edge_count(ei):
+    e = int(ei.size(-1))
+    if e >= 2 ** 31:
+        raise RuntimeError("gripnet_b200: edge lists must hold < 2^31 edges")
+    return e
+
+
+def _ptr_at(t, i):
+    """Address of ``t[i]`` (None for None) without building a view: the chunk loops run once per chunk."""
+    return None if t is None else t.data_ptr() + i * t.element_size()
+
+
 class _Grouped:
-    """``gn_rank_csr`` of one edge list: rows ``s * R + r``, entries (dst, edge id) sorted by dst."""
-
-    def __init__(self, ei, et, n, r, groups):
-        lib = _lib.load()
-        dev = ei.device
-        e = int(ei.size(1))
-        if e >= 2 ** 31:
-            raise RuntimeError("gripnet_b200: edge lists must hold < 2^31 edges")
-        i32 = dict(dtype=torch.int32, device=dev)
-        self.rowptr = torch.empty(n * r + 1, **i32)
-        self.dst = torch.empty(max(e, 1), **i32)
-        self.eid = torch.empty(max(e, 1), **i32)
-        self.group_row = torch.empty(n * r, **i32) if groups else None
-        count = torch.zeros(1, **i32) if groups else None
-        ws = _ws(lib.gn_rank_csr_workspace_bytes(e, n, r), dev)
-        _lib.check(lib.gn_rank_csr(_ptr(ei[0]) if e else None, _ptr(ei[1]) if e else None, _ptr(et) if e else None, e,
-                                   n, r, _ptr(self.rowptr), _ptr(self.dst), _ptr(self.eid), _ptr(self.group_row),
-                                   _ptr(count), _ptr(ws), ws.numel(), _stream()), "gn_rank_csr")
-        self.n_groups = _host_int(count[0]) if groups else 0          # the one host read, at build time
-
-
-class _Paired:
-    """``gn_rank_pair_csr`` of one edge list: rows are the distinct directed pairs ``(s, t)`` in ``(src, dst)`` order,
-    entries (relation, edge id) sorted by relation inside a row."""
+    """``gn_rank_csr`` of one edge list, the dense view pair queries read at any row: rows ``s * R + r``, entries
+    (dst, edge id) sorted by dst."""
 
     def __init__(self, ei, et, n, r):
         lib = _lib.load()
         dev = ei.device
-        e = int(ei.size(1))
-        if e >= 2 ** 31:
-            raise RuntimeError("gripnet_b200: edge lists must hold < 2^31 edges")
+        e = _edge_count(ei)
+        i32 = dict(dtype=torch.int32, device=dev)
+        self.rowptr = torch.empty(n * r + 1, **i32)
+        self.dst = torch.empty(max(e, 1), **i32)
+        self.eid = torch.empty(max(e, 1), **i32)
+        ws = _ws(lib.gn_rank_csr_workspace_bytes(e), dev)
+        _lib.check(lib.gn_rank_csr(_ptr(ei[0]) if e else None, _ptr(ei[1]) if e else None, _ptr(et) if e else None, e,
+                                   n, r, _ptr(self.rowptr), _ptr(self.dst), _ptr(self.eid), _ptr(ws), ws.numel(),
+                                   _stream()), "gn_rank_csr")
+
+
+class _KeyGroups:
+    """``gn_rank_group`` of the columns ``(a, b, c)`` of one edge list: rows ("groups") are the distinct key pairs
+    ``(a, b)`` in ascending order, entries (``c``, edge id) sorted by ``c`` inside a row."""
+
+    def __init__(self, a, b, c, sizes):
+        lib = _lib.load()
+        dev = a.device
+        e = _edge_count(a)
         i32 = dict(dtype=torch.int32, device=dev)
         self.rowptr = torch.empty(e + 1, **i32)
-        self.src = torch.empty(max(e, 1), **i32)
-        self.dst = torch.empty(max(e, 1), **i32)
-        self.rel = torch.empty(max(e, 1), **i32)
-        self.eid = torch.empty(max(e, 1), **i32)
+        self.a, self.b, self.c, self.eid = (torch.empty(max(e, 1), **i32) for _ in range(4))
         count = torch.zeros(1, **i32)
-        ws = _ws(lib.gn_rank_pair_csr_workspace_bytes(e), dev)
-        _lib.check(lib.gn_rank_pair_csr(_ptr(ei[0]) if e else None, _ptr(ei[1]) if e else None, _ptr(et) if e else None,
-                                        e, n, r, _ptr(self.rowptr), _ptr(self.src), _ptr(self.dst), _ptr(self.rel),
-                                        _ptr(self.eid), _ptr(count), _ptr(ws), ws.numel(), _stream()),
-                   "gn_rank_pair_csr")
-        self.n_pairs = _host_int(count[0])                             # the one host read, at build time
+        ws = _ws(lib.gn_rank_group_workspace_bytes(e), dev)
+        _lib.check(lib.gn_rank_group(_ptr(a) if e else None, _ptr(b) if e else None, _ptr(c) if e else None, e,
+                                     *sizes, _ptr(self.rowptr), _ptr(self.a), _ptr(self.b), _ptr(self.c),
+                                     _ptr(self.eid), _ptr(count), _ptr(ws), ws.numel(), _stream()), "gn_rank_group")
+        self.n_groups = _host_int(count[0])                             # the one host read, at build time
 
-    def lookup(self, count, pair_src=None, pair_dst=None, src=None, dst=None):
-        """int32 ``[count]``: the row of every query pair in this structure, -1 where it holds no such pair."""
-        dev = self.rowptr.device
-        row = torch.empty(max(count, 1), dtype=torch.int32, device=dev)
-        _lib.check(_lib.load().gn_rank_pair_lookup(_ptr(self.src), _ptr(self.dst), self.n_pairs, _ptr(pair_src),
-                                                   _ptr(pair_dst), _ptr(src), _ptr(dst), count, _ptr(row), _stream()),
-                   "gn_rank_pair_lookup")
+    def lookup(self, count, a32=None, b32=None, a64=None, b64=None):
+        """int32 ``[count]``: the row of every query key pair in this structure, -1 where it holds no such pair."""
+        row = torch.empty(max(count, 1), dtype=torch.int32, device=self.rowptr.device)
+        _lib.check(_lib.load().gn_rank_lookup(_ptr(self.a), _ptr(self.b), self.n_groups, _ptr(a32), _ptr(b32),
+                                              _ptr(a64), _ptr(b64), count, _ptr(row), _stream()), "gn_rank_lookup")
         return row
+
+
+# Tail queries (s, r, ?) group a triple list by (src, rel) with candidates dst and score the rows z[s] .* w[r]
+# against z; relation queries (s, ?, t) group it by (src, dst) with candidates rel and score z[s] .* z[t] against w.
+def _columns(view, ei, et, n, r):
+    """The key columns ``(a, b)``, the candidate column ``c`` and their sizes of a triple list."""
+    if view == "tail":
+        return (ei[0], et, ei[1]), (n, r, n)
+    return (ei[0], ei[1], et), (n, n, r)
+
+
+def _tables(view, z, w):
+    """``y`` of the query rows ``z[a] .* y[b]`` and the candidate table."""
+    return (w, z) if view == "tail" else (z, w)
 
 
 class EdgeFilter:
@@ -157,8 +171,8 @@ class EdgeFilter:
     and sorted by ``c``.  ``edge_lists``: a sequence of ``(edge_index int64 [2, E], edge_type int64 [E])`` on one
     CUDA device.  Built once; reusable by any number of rankers and top-k calls of the same graph.  The first
     relation query that uses the filter (``RelationRanker``, ``topk_relations``) also builds its pair-grouped view
-    from the same edge lists (the filter keeps references to them) and caches it here; the first pair query
-    (``topk_pairs``) likewise builds and caches a symmetrised view."""
+    from the same triples (the filter keeps them) and caches it here; the first pair query (``topk_pairs``,
+    ``PairRanker``) likewise builds and caches a symmetrised view."""
 
     def __init__(self, edge_lists, num_nodes, num_relations):
         self.num_nodes, self.num_relations = _sizes(num_nodes, num_relations)
@@ -168,38 +182,26 @@ class EdgeFilter:
         self.device = lists[0][0].device
         if any(ei.device != self.device for ei, _ in lists):
             raise RuntimeError("gripnet_b200: the filter's edge lists must be on one device")
-        ei = torch.cat([l[0] for l in lists], dim=1) if len(lists) > 1 else lists[0][0]
-        et = torch.cat([l[1] for l in lists]) if len(lists) > 1 else lists[0][1]
-        self.n_edges = int(ei.size(1))
-        self._g = _Grouped(ei, et, self.num_nodes, self.num_relations, groups=False)
-        self._lists = lists
-        self._p = None
-        self._s = None
+        self._ei = torch.cat([l[0] for l in lists], dim=1) if len(lists) > 1 else lists[0][0]
+        self._et = torch.cat([l[1] for l in lists]) if len(lists) > 1 else lists[0][1]
+        self.n_edges = int(self._ei.size(1))
+        self._views = {}
+        self._view("tail", self.num_nodes, self.num_relations, self.device)
 
-    def _check(self, n, r, device):
+    def _view(self, view, n, r, device):
+        """The filter's triples grouped for one query kind, built on first use: ``"tail"`` and ``"relation"`` as
+        ``_KeyGroups`` of ``_columns``; ``"symmetric"``, the ``_Grouped`` view of the triples and their flipped copies
+        (row ``s * R + r`` holds every ``t`` with ``(s, r, t)`` or ``(t, r, s)`` in the filter, sorted)."""
         if (n, r) != (self.num_nodes, self.num_relations) or device != self.device:
             raise RuntimeError("gripnet_b200: the filter was built for another graph (node / relation count or device)")
-        return self._g
-
-    def _pairs(self, n, r, device):
-        """The pair-grouped view (``_Paired``) of the filter's triples, built on first use."""
-        self._check(n, r, device)
-        if self._p is None:
-            lists = self._lists
-            ei = torch.cat([l[0] for l in lists], dim=1) if len(lists) > 1 else lists[0][0]
-            et = torch.cat([l[1] for l in lists]) if len(lists) > 1 else lists[0][1]
-            self._p = _Paired(ei, et, self.num_nodes, self.num_relations)
-        return self._p
-
-    def _symmetric(self, n, r, device):
-        """The grouped view (``_Grouped``) of the filter's triples and their flipped copies, built on first use: row
-        ``s * R + r`` holds every ``t`` with ``(s, r, t)`` or ``(t, r, s)`` in the filter, sorted."""
-        self._check(n, r, device)
-        if self._s is None:
-            ei = torch.cat([l[0] for l in self._lists] + [l[0].flip(0) for l in self._lists], dim=1)
-            et = torch.cat([l[1] for l in self._lists] * 2)
-            self._s = _Grouped(ei, et, self.num_nodes, self.num_relations, groups=False)
-        return self._s
+        if view not in self._views:
+            ei, et = self._ei, self._et
+            if view == "symmetric":
+                self._views[view] = _Grouped(torch.cat([ei, ei.flip(0)], dim=1), torch.cat([et, et]), n, r)
+            else:
+                cols, sizes = _columns(view, ei, et, n, r)
+                self._views[view] = _KeyGroups(*cols, sizes)
+        return self._views[view]
 
 
 def _embeddings(z, weight, n=None, r=None):
@@ -223,13 +225,22 @@ def _chunk_rows(n, total):
     return lds, max(1, min(int(total), CHUNK_BYTES // (4 * lds)))
 
 
-def _pair_scores(z, w, p, s, rows, lds, pair_src=None, pair_dst=None, src=None, dst=None):
-    """``S[0:rows] = (z[s_i] .* z[t_i]) . w^T`` for one chunk of pairs."""
+def _score_chunks(z, y, cand, total, a32=None, b32=None, a64=None, b64=None):
+    """Score rows ``S[i] = (z[a_i] .* y[b_i]) . cand^T`` of the queries ``i < total``, one chunk at a time: yields
+    ``(i0, cnt, S, lds)`` with the rows of queries ``i0 .. i0 + cnt - 1`` in ``S[0:cnt]`` (one buffer for all)."""
     lib = _lib.load()
-    d = z.size(1)
-    _lib.check(lib.gn_rank_pair_rows(z.data_ptr(), ops._ldz(z), d, _ptr(pair_src), _ptr(pair_dst), _ptr(src),
-                                     _ptr(dst), rows, p.data_ptr(), d, _stream()), "gn_rank_pair_rows")
-    ops.sgemm(False, True, rows, w.size(0), d, p.data_ptr(), d, w.data_ptr(), d, s.data_ptr(), lds, z.device)
+    d, m = z.size(1), cand.size(0)
+    lds, rows = _chunk_rows(m, total)
+    q = torch.empty((rows, d), dtype=torch.float32, device=z.device)
+    s = torch.empty((rows, lds), dtype=torch.float32, device=z.device)
+    for i0 in range(0, total, rows):
+        cnt = min(rows, total - i0)
+        _lib.check(lib.gn_rank_rows(z.data_ptr(), ops._ldz(z), y.data_ptr(), ops._ldz(y), d, _ptr_at(a32, i0),
+                                    _ptr_at(b32, i0), _ptr_at(a64, i0), _ptr_at(b64, i0), cnt, q.data_ptr(), d,
+                                    _stream()), "gn_rank_rows")
+        ops.sgemm(False, True, cnt, m, d, q.data_ptr(), d, cand.data_ptr(), ops._ldz(cand), s.data_ptr(), lds,
+                  z.device)
+        yield i0, cnt, s, lds
 
 
 def _relation_index(et, num_relations, device):
@@ -246,17 +257,31 @@ def _relation_index(et, num_relations, device):
 
 
 class _Ranker:
-    """What ``LinkRanker``, ``RelationRanker`` and ``PairRanker`` share: the output checks of ``ranks`` and the
-    per-relation reduction of ``metrics``.  Subclasses set ``num_relations``, ``device``, ``n_edges``,
-    ``_rel_rowptr``, ``_rel_perm`` (the edges of relation ``r`` are ``_rel_perm[_rel_rowptr[r]:_rel_rowptr[r + 1]]``
-    for ``r < R``) and define ``ranks``."""
+    """What ``LinkRanker``, ``RelationRanker`` and ``PairRanker`` share: the checked triple list, the prologue and
+    output checks of ``ranks`` and the per-relation reduction of ``metrics``.  Subclasses set ``_rel_rowptr``,
+    ``_rel_perm`` (the edges of relation ``r`` are ``_rel_perm[_rel_rowptr[r]:_rel_rowptr[r + 1]]`` for ``r < R``)
+    and define ``_rank(z, w, out)``, called for a non-empty list."""
 
-    def _rank_out(self, out):
+    def __init__(self, edge_index, edge_type, num_nodes, num_relations, filter):
+        self.num_nodes, self.num_relations = _sizes(num_nodes, num_relations)
+        self._ei, self._et = _edge_list(edge_index, edge_type, self.num_nodes, self.num_relations, "query")
+        self.device = self._ei.device
+        self.n_edges = int(self._ei.size(1))
+        self.filter = filter
+
+    def ranks(self, z, weight, out=None):
+        """float32 ``[E]``: the filtered rank of every triple against the candidates of the ranker's query kind, in
+        the list's order."""
+        z, w = _embeddings(z, weight, self.num_nodes, self.num_relations)
+        if z.device != self.device:
+            raise RuntimeError("gripnet_b200: z is not on the ranker's device")
         if out is None:
-            return torch.empty(self.n_edges, dtype=torch.float32, device=self.device)
-        if out.shape != (self.n_edges,) or out.dtype != torch.float32 or not out.is_contiguous() or \
+            out = torch.empty(self.n_edges, dtype=torch.float32, device=self.device)
+        elif out.shape != (self.n_edges,) or out.dtype != torch.float32 or not out.is_contiguous() or \
                 out.device != self.device:
             raise RuntimeError("gripnet_b200: out must be a contiguous float32 [E] tensor on the ranker's device")
+        if self.n_edges > 0:
+            self._rank(z, w, out)
         return out
 
     def metrics(self, z, weight, hits=(1, 3, 10), out=None):
@@ -280,65 +305,49 @@ class _Ranker:
         return out
 
 
-def _score_rows(z, w, q, s, rows, lds, group_row=None, node=None, rel=None):
-    """``S[0:rows] = (z[s_i] .* w[r_i]) . z^T`` for one chunk of queries."""
-    lib = _lib.load()
-    d = z.size(1)
-    _lib.check(lib.gn_rank_query_rows(z.data_ptr(), ops._ldz(z), d, w.data_ptr(), w.size(0), _ptr(group_row),
-                                      _ptr(node), _ptr(rel), rows, q.data_ptr(), d, _stream()), "gn_rank_query_rows")
-    ops.sgemm(False, True, rows, z.size(0), d, q.data_ptr(), d, z.data_ptr(), ops._ldz(z), s.data_ptr(), lds, z.device)
+class _GroupRanker(_Ranker):
+    """``LinkRanker`` and ``RelationRanker``: the list grouped by its key pairs (``_columns`` of the class's
+    ``_VIEW``), the filter row of every group found once here, and one loop over chunks of score rows that counts
+    the ranks of each group's triples."""
+
+    def __init__(self, edge_index, edge_type, num_nodes, num_relations, filter=None):
+        super().__init__(edge_index, edge_type, num_nodes, num_relations, filter)
+        n, r = self.num_nodes, self.num_relations
+        self._f = filter._view(self._VIEW, n, r, self.device) if filter is not None else None
+        cols, sizes = _columns(self._VIEW, self._ei, self._et, n, r)
+        self._q = _KeyGroups(*cols, sizes)
+        self._f_row = self._f.lookup(self._q.n_groups, a32=self._q.a, b32=self._q.b) if self._f is not None else None
+        self._rel_rowptr, self._rel_perm = _relation_index(self._et, r, self.device)
+
+    def _rank(self, z, w, out):
+        lib = _lib.load()
+        y, cand = _tables(self._VIEW, z, w)
+        q = self._q
+        fr, fc = (self._f.rowptr, self._f.c) if self._f is not None else (None, None)
+        for g0, cnt, s, lds in _score_chunks(z, y, cand, q.n_groups, a32=q.a, b32=q.b):
+            _lib.check(lib.gn_rank_count(s.data_ptr(), lds, cand.size(0), cnt, _ptr_at(q.rowptr, g0), _ptr(q.c),
+                                         _ptr(q.eid), _ptr_at(self._f_row, g0), _ptr(fr), _ptr(fc), out.data_ptr(),
+                                         _stream()), "gn_rank_count")
 
 
-class LinkRanker(_Ranker):
+class LinkRanker(_GroupRanker):
     """Filtered ranks of the edges of one list against all candidate tails, and their per-relation MRR / Hits@k.
 
     ``edge_index`` int64 ``[2, E]`` / ``edge_type`` int64 ``[E]``: the edges to rank (e.g. the test split);
-    ``filter``: an ``EdgeFilter`` of the known positives to skip (None: raw ranks).  The query structure is built once
-    here (one device->host read, the number of distinct ``(s, r)`` queries); ``ranks`` / ``metrics`` then read nothing
-    back and branch on no device value, so they can be captured in a CUDA graph and replayed every epoch.  One GPU:
-    gather a partitioned ``z`` first (``parallel.all_gather_rows``)."""
+    ``filter``: an ``EdgeFilter`` of the known positives to skip (None: raw ranks).  The query structure and each
+    query's filter row are built once here (one device->host read, the number of distinct ``(s, r)`` queries);
+    ``ranks`` / ``metrics`` then read nothing back and branch on no device value, so they can be captured in a CUDA
+    graph and replayed every epoch.  One GPU: gather a partitioned ``z`` first (``parallel.all_gather_rows``)."""
 
-    def __init__(self, edge_index, edge_type, num_nodes, num_relations, filter=None):
-        self.num_nodes, self.num_relations = _sizes(num_nodes, num_relations)
-        ei, et = _edge_list(edge_index, edge_type, self.num_nodes, self.num_relations, "query")
-        self.device = ei.device
-        self.n_edges = int(ei.size(1))
-        self.filter = filter
-        self._f = filter._check(self.num_nodes, self.num_relations, self.device) if filter is not None else None
-        self._q = _Grouped(ei, et, self.num_nodes, self.num_relations, groups=True)
-        self._rel_rowptr, self._rel_perm = _relation_index(et, self.num_relations, self.device)
+    _VIEW = "tail"
 
     @property
     def n_groups(self):
         """Number of distinct ``(s, r)`` queries of the list."""
         return self._q.n_groups
 
-    def ranks(self, z, weight, out=None):
-        """float32 ``[E]``: the filtered rank of every edge, in the list's order."""
-        lib = _lib.load()
-        z, w = _embeddings(z, weight, self.num_nodes, self.num_relations)
-        if z.device != self.device:
-            raise RuntimeError("gripnet_b200: z is not on the ranker's device")
-        out = self._rank_out(out)
-        g_total = self._q.n_groups
-        if g_total == 0:
-            return out
-        n, d = self.num_nodes, z.size(1)
-        lds, rows = _chunk_rows(n, g_total)
-        q = torch.empty((rows, d), dtype=torch.float32, device=self.device)
-        s = torch.empty((rows, lds), dtype=torch.float32, device=self.device)
-        fr, fd = (self._f.rowptr, self._f.dst) if self._f is not None else (None, None)
-        for g0 in range(0, g_total, rows):
-            cnt = min(rows, g_total - g0)
-            grp = self._q.group_row[g0:]
-            _score_rows(z, w, q, s, cnt, lds, group_row=grp)
-            _lib.check(lib.gn_rank_count(s.data_ptr(), lds, n, _ptr(grp), cnt, _ptr(self._q.rowptr), _ptr(self._q.dst),
-                                         _ptr(self._q.eid), _ptr(fr), _ptr(fd), out.data_ptr(), _stream()),
-                       "gn_rank_count")
-        return out
 
-
-class RelationRanker(_Ranker):
+class RelationRanker(_GroupRanker):
     """Filtered ranks of the triples of one list against all ``R`` relations of their pair, and their per-relation
     MRR / Hits@k.
 
@@ -348,47 +357,12 @@ class RelationRanker(_Ranker):
     device->host read, the number of distinct directed pairs); ``ranks`` / ``metrics`` then read nothing back and
     branch on no device value, so they can be captured in a CUDA graph.  One GPU: gather a partitioned ``z`` first."""
 
-    def __init__(self, edge_index, edge_type, num_nodes, num_relations, filter=None):
-        self.num_nodes, self.num_relations = _sizes(num_nodes, num_relations)
-        ei, et = _edge_list(edge_index, edge_type, self.num_nodes, self.num_relations, "query")
-        self.device = ei.device
-        self.n_edges = int(ei.size(1))
-        self.filter = filter
-        self._f = filter._pairs(self.num_nodes, self.num_relations, self.device) if filter is not None else None
-        self._q = _Paired(ei, et, self.num_nodes, self.num_relations)
-        self._f_row = None
-        if self._f is not None:
-            self._f_row = self._f.lookup(self._q.n_pairs, pair_src=self._q.src, pair_dst=self._q.dst)
-        self._rel_rowptr, self._rel_perm = _relation_index(et, self.num_relations, self.device)
+    _VIEW = "relation"
 
     @property
     def n_groups(self):
         """Number of distinct directed pairs ``(s, t)`` of the list."""
-        return self._q.n_pairs
-
-    def ranks(self, z, weight, out=None):
-        """float32 ``[E]``: the filtered relation rank of every triple, in the list's order."""
-        lib = _lib.load()
-        z, w = _embeddings(z, weight, self.num_nodes, self.num_relations)
-        if z.device != self.device:
-            raise RuntimeError("gripnet_b200: z is not on the ranker's device")
-        out = self._rank_out(out)
-        g_total = self._q.n_pairs
-        if g_total == 0:
-            return out
-        r, d = self.num_relations, z.size(1)
-        lds, rows = _chunk_rows(r, g_total)
-        p = torch.empty((rows, d), dtype=torch.float32, device=self.device)
-        s = torch.empty((rows, lds), dtype=torch.float32, device=self.device)
-        fr, fd = (self._f.rowptr, self._f.rel) if self._f is not None else (None, None)
-        for g0 in range(0, g_total, rows):
-            cnt = min(rows, g_total - g0)
-            _pair_scores(z, w, p, s, cnt, lds, pair_src=self._q.src[g0:], pair_dst=self._q.dst[g0:])
-            _lib.check(lib.gn_rank_pair_count(s.data_ptr(), lds, r, cnt, _ptr(self._q.rowptr[g0:]), _ptr(self._q.rel),
-                                              _ptr(self._q.eid),
-                                              _ptr(self._f_row[g0:]) if self._f_row is not None else None, _ptr(fr),
-                                              _ptr(fd), out.data_ptr(), _stream()), "gn_rank_pair_count")
-        return out
+        return self._q.n_groups
 
 
 class PairRanker(_Ranker):
@@ -405,17 +379,13 @@ class PairRanker(_Ranker):
     can be captured in a CUDA graph.  One GPU: gather a partitioned ``z`` first."""
 
     def __init__(self, edge_index, edge_type, num_nodes, num_relations, filter=None):
+        super().__init__(edge_index, edge_type, num_nodes, num_relations, filter)
         lib = _lib.load()
-        self.num_nodes, self.num_relations = _sizes(num_nodes, num_relations)
         n, r = self.num_nodes, self.num_relations
         if n * n >= 2 ** 31:
             raise RuntimeError(f"gripnet_b200: PairRanker needs num_nodes^2 < 2^31, got {n} nodes")
-        ei, et = _edge_list(edge_index, edge_type, n, r, "query")
-        self.device = ei.device
-        self.n_edges = int(ei.size(1))
-        self.filter = filter
-        self._f = filter._symmetric(n, r, self.device) if filter is not None else None
-        self._ei, self._et = ei, et
+        ei, et = self._ei, self._et
+        self._f = filter._view("symmetric", n, r, self.device) if filter is not None else None
         # relation index over R + 1 keys: a self-pair triple takes key R, so metrics (rows 0 .. R - 1) skip it
         key = torch.where(ei[0] == ei[1], torch.full_like(et, r), et)
         self._rel_rowptr, self._rel_perm = _relation_index(key, r + 1, self.device)
@@ -435,15 +405,8 @@ class PairRanker(_Ranker):
         """Number of distinct relations with rankable (non-self-pair) triples."""
         return int(self._groups.numel())
 
-    def ranks(self, z, weight, out=None):
-        """float32 ``[E]``: the filtered pair rank of every triple, in the list's order (NaN for a self-pair)."""
+    def _rank(self, z, w, out):
         lib = _lib.load()
-        z, w = _embeddings(z, weight, self.num_nodes, self.num_relations)
-        if z.device != self.device:
-            raise RuntimeError("gripnet_b200: z is not on the ranker's device")
-        out = self._rank_out(out)
-        if self.n_edges == 0:
-            return out
         r = self.num_relations
         ws = _ws(self._ws_bytes, self.device)
         fr, fd = (self._f.rowptr, self._f.dst) if self._f is not None else (None, None)
@@ -456,7 +419,6 @@ class PairRanker(_Ranker):
         _lib.check(lib.gn_rank_rel_pairs_finish(_ptr(ws), ws.numel(), r, _ptr(self._rel_rowptr), _ptr(self._rel_perm),
                                                 self._n_queries, _ptr(self._t_filtered), out.data_ptr(), _stream()),
                    "gn_rank_rel_pairs_finish")
-        return out
 
 
 def _k_arg(k):
@@ -469,47 +431,53 @@ def _k_arg(k):
     return operator.index(k)
 
 
+def _query_list(a, name, bound, dev):
+    """An int64 CUDA index list, flattened and range-checked."""
+    a = a if torch.is_tensor(a) else torch.as_tensor(a, dtype=torch.int64, device=dev)
+    require_cuda(a, name, torch.int64)
+    a = a.contiguous().view(-1)
+    validate_index(a, bound, name)
+    return a
+
+
 def _query_lists(a, b, names, bounds, dev):
     """Two equally long int64 CUDA index lists, flattened and range-checked."""
-    a = a if torch.is_tensor(a) else torch.as_tensor(a, dtype=torch.int64, device=dev)
-    b = b if torch.is_tensor(b) else torch.as_tensor(b, dtype=torch.int64, device=dev)
-    require_cuda(a, names[0], torch.int64)
-    require_cuda(b, names[1], torch.int64)
-    a, b = a.contiguous().view(-1), b.contiguous().view(-1)
+    a, b = _query_list(a, names[0], bounds[0], dev), _query_list(b, names[1], bounds[1], dev)
     if a.numel() != b.numel():
         raise RuntimeError(f"gripnet_b200: {names[0]} and {names[1]} must have the same length")
-    validate_index(a, bounds[0], names[0])
-    validate_index(b, bounds[1], names[1])
     return a, b
+
+
+def _topk(view, z, w, a, b, k, filter, sigmoid):
+    """``topk`` / ``topk_relations`` after their argument checks: the top ``k`` candidates of the query rows
+    ``z[a_i] .* y[b_i]``, the filter row of ``(a_i, b_i)`` skipped."""
+    lib = _lib.load()
+    dev = z.device
+    f = filter._view(view, z.size(0), w.size(0), dev) if filter is not None else None
+    y, cand = _tables(view, z, w)
+    nq = a.numel()
+    scores = torch.empty((nq, k), dtype=torch.float32, device=dev)
+    ids = torch.empty((nq, k), dtype=torch.int64, device=dev)
+    if nq == 0:
+        return scores, ids
+    f_row = f.lookup(nq, a64=a, b64=b) if f is not None else None
+    fr, fc = (f.rowptr, f.c) if f is not None else (None, None)
+    for q0, cnt, s, lds in _score_chunks(z, y, cand, nq, a64=a, b64=b):
+        _lib.check(lib.gn_rank_topk(s.data_ptr(), lds, cand.size(0), cnt, _ptr_at(f_row, q0), _ptr(fr), _ptr(fc), k,
+                                    int(bool(sigmoid)), _ptr_at(scores, q0 * k), _ptr_at(ids, q0 * k), _stream()),
+                   "gn_rank_topk")
+    return scores, ids
 
 
 def topk(z, weight, node, rel, k, filter=None, sigmoid=True):
     """The ``k`` (1..256) most likely tails ``c`` of every query ``(node[i], rel[i])`` with ``(node[i], rel[i], c)``
     not in ``filter``: ``(scores float32 [Q, k], ids int64 [Q, k])``, descending pre-sigmoid score, ties by smaller
     id; scores after the sigmoid when ``sigmoid``; id -1 / score NaN where fewer than ``k`` candidates are left."""
-    lib = _lib.load()
     z, w = _embeddings(z, weight)
     n, r = _sizes(z.size(0), w.size(0))
-    dev = z.device
     k = _k_arg(k)
-    node, rel = _query_lists(node, rel, ("node", "rel"), (n, r), dev)
-    f = filter._check(n, r, dev) if filter is not None else None
-    nq = node.numel()
-    scores = torch.empty((nq, k), dtype=torch.float32, device=dev)
-    ids = torch.empty((nq, k), dtype=torch.int64, device=dev)
-    if nq == 0:
-        return scores, ids
-    lds, rows = _chunk_rows(n, nq)
-    q = torch.empty((rows, z.size(1)), dtype=torch.float32, device=dev)
-    s = torch.empty((rows, lds), dtype=torch.float32, device=dev)
-    for q0 in range(0, nq, rows):
-        cnt = min(rows, nq - q0)
-        _score_rows(z, w, q, s, cnt, lds, node=node[q0:], rel=rel[q0:])
-        _lib.check(lib.gn_rank_topk(s.data_ptr(), lds, n, r, _ptr(node[q0:]), _ptr(rel[q0:]), cnt,
-                                    _ptr(f.rowptr) if f is not None else None, _ptr(f.dst) if f is not None else None,
-                                    k, int(bool(sigmoid)), _ptr(scores[q0:]), _ptr(ids[q0:]), _stream()),
-                   "gn_rank_topk")
-    return scores, ids
+    node, rel = _query_lists(node, rel, ("node", "rel"), (n, r), z.device)
+    return _topk("tail", z, w, node, rel, k, filter, sigmoid)
 
 
 def topk_relations(z, weight, src, dst, k, filter=None, sigmoid=True):
@@ -517,30 +485,11 @@ def topk_relations(z, weight, src, dst, k, filter=None, sigmoid=True):
     ``(src[i], r, dst[i])`` not in ``filter``: ``(scores float32 [Q, k], ids int64 [Q, k])``, descending pre-sigmoid
     score, ties by smaller relation id; scores after the sigmoid when ``sigmoid``; id -1 / score NaN where fewer than
     ``k`` relations are left (``k`` may exceed ``R``)."""
-    lib = _lib.load()
     z, w = _embeddings(z, weight)
     n, r = _sizes(z.size(0), w.size(0))
-    dev = z.device
     k = _k_arg(k)
-    src, dst = _query_lists(src, dst, ("src", "dst"), (n, n), dev)
-    f = filter._pairs(n, r, dev) if filter is not None else None
-    nq = src.numel()
-    scores = torch.empty((nq, k), dtype=torch.float32, device=dev)
-    ids = torch.empty((nq, k), dtype=torch.int64, device=dev)
-    if nq == 0:
-        return scores, ids
-    f_row = f.lookup(nq, src=src, dst=dst) if f is not None else None
-    lds, rows = _chunk_rows(r, nq)
-    p = torch.empty((rows, z.size(1)), dtype=torch.float32, device=dev)
-    s = torch.empty((rows, lds), dtype=torch.float32, device=dev)
-    for q0 in range(0, nq, rows):
-        cnt = min(rows, nq - q0)
-        _pair_scores(z, w, p, s, cnt, lds, src=src[q0:], dst=dst[q0:])
-        _lib.check(lib.gn_rank_pair_topk(s.data_ptr(), lds, r, cnt, _ptr(f_row[q0:]) if f is not None else None,
-                                         _ptr(f.rowptr) if f is not None else None,
-                                         _ptr(f.rel) if f is not None else None, k, int(bool(sigmoid)),
-                                         _ptr(scores[q0:]), _ptr(ids[q0:]), _stream()), "gn_rank_pair_topk")
-    return scores, ids
+    src, dst = _query_lists(src, dst, ("src", "dst"), (n, n), z.device)
+    return _topk("relation", z, w, src, dst, k, filter, sigmoid)
 
 
 def topk_pairs(z, weight, rel, k, filter=None, sigmoid=True):
@@ -557,11 +506,8 @@ def topk_pairs(z, weight, rel, k, filter=None, sigmoid=True):
         raise RuntimeError(f"gripnet_b200: topk_pairs needs num_nodes^2 < 2^31 (pair ids), got {n} nodes")
     dev = z.device
     k = _k_arg(k)
-    rel = rel if torch.is_tensor(rel) else torch.as_tensor(rel, dtype=torch.int64, device=dev)
-    require_cuda(rel, "rel", torch.int64)
-    rel = rel.contiguous().view(-1)
-    validate_index(rel, r, "rel")
-    f = filter._symmetric(n, r, dev) if filter is not None else None
+    rel = _query_list(rel, "rel", r, dev)
+    f = filter._view("symmetric", n, r, dev) if filter is not None else None
     nq = rel.numel()
     scores = torch.empty((nq, k), dtype=torch.float32, device=dev)
     src = torch.empty((nq, k), dtype=torch.int64, device=dev)

@@ -385,88 +385,71 @@ int gn_nc_metrics(const int64_t* target, const int64_t* pred, int64_t n, int32_t
 
 /* ---- K16: filtered candidate ranking and top-k of the DistMult decoder --------------------------- */
 /* New capability (the reference evaluates each positive against ONE sampled negative, GripNet-pose.py:148-164).
- * Every candidate tail c in [0, n) of a query (s, r), c == s included, is scored with the PRE-sigmoid DistMult
- * score S(c) = sum_k z[s,k] w[r,k] z[c,k], evaluated as one row of S = Q . z^T with Q[g] = z[s_g] .* w[r_g]
- * (gn_rank_query_rows, then the dense product gn_sgemm / gn_tc_gemm with transB = 1).  Only tail queries
- * (s, r, ?) are ranked: lists holding both directions of every pair rank the head through the mirrored edge.
+ * Tail queries (s, r, ?) and relation queries (s, ?, t) share one structure, one scoring path and one set of
+ * kernels; only the data differs.  The triples are grouped by a key pair (a, b): (s, r) for tail queries, (s, t) for
+ * relation queries.  Every candidate c of a group is scored with the PRE-sigmoid DistMult score, evaluated as one row
+ * of S = Q . C^T with Q[g] = x[a_g] .* y[b_g] (gn_rank_rows, then the dense product gn_sgemm / gn_tc_gemm with
+ * transB = 1):
+ *   tail:     S(c)  = sum_k z[s,k] w[r,k] z[c,k],  x = z, y = w, C = z; every tail c in [0, n), c == s included;
+ *   relation: S(r') = sum_k z[s,k] z[t,k] w[r',k], x = y = z, C = w (the decoder weight [n_rel, D]); every relation
+ *             r' in [0, n_rel).  Q is bitwise symmetric (fp32 products commute), so (s, t) and (t, s) give identical
+ *             rows when both take the same product path.
+ * Only tail queries (s, r, ?) rank the tail: lists holding both directions of every pair rank the head through the
+ * mirrored edge.  A FILTER is the set of directed known positives (s, r, t), e.g. train + test: the grouped
+ * structure of the concatenated filter lists with the same key columns; duplicates stay stored and count once.
  *
- * gn_rank_csr: one-sided grouped structure of an edge list — rowptr [n_nodes*n_rel + 1] (row s*n_rel + r), entries
- *   ent_dst / ent_eid [E] (candidate, edge id) sorted by candidate inside a row (two stable counting sorts).  A
- *   FILTER (the set of directed known positives (s, r, c), e.g. train + test) is the structure of the concatenated
- *   filter lists; duplicates stay stored and are skipped where they are read.  group_row / n_groups (both or
- *   neither): the ids of the non-empty rows in ascending order ("groups", capacity n_nodes*n_rel) and their count
- *   (device int32).
- * gn_rank_query_rows: q[i, 0:D] = z[s_i] .* w[r_i], with (s_i, r_i) taken from group_row[i] = s*n_rel + r, or, when
- *   group_row is NULL, from node[i] / rel[i].
- * gn_rank_count: filtered rank of every target of groups [0, n_groups) whose score rows are S[g] (leading dimension
- *   lds >= n_nodes; group_row points at the first group of the chunk).  OGB rule: with the negatives
- *   N = {c != t : (s, r, c) not in the filter}, opt = #{c in N : S(c) > S(t)}, pess = #{c in N : S(c) >= S(t)},
- *   rank[edge id] = 1 + (opt + pess) / 2 (float32).  S(t) is read from the same row as every S(c).  f_rowptr ==
- *   NULL: no filter.
+ * gn_rank_group: compacted grouped structure of three int64 columns (a, b, c) of sizes (na, nb, nc): tail callers
+ *   pass (src, rel, dst), relation callers (src, dst, rel).  Three stable counting sorts (by c, by b, by a) order the
+ *   entries by (a, b, c); rows ("groups") are the distinct key pairs (a, b) in that order, compacted (not a*nb + b,
+ *   which does not fit int32 for general n): rowptr [capacity n_edges + 1], group_a / group_b [capacity n_edges],
+ *   entries ent_c / ent_eid [n_edges] (candidate, edge id) sorted by candidate inside a row; n_groups (device int32)
+ *   the row count.
+ * gn_rank_lookup: row[i] = the row of key pair (a_i, b_i) in a grouped structure of n_f rows whose key columns are
+ *   f_a / f_b (binary search), or -1 when it holds no such pair.  (a_i, b_i) from a32 / b32 (int32, e.g. a query
+ *   structure's groups) or, when a32 is NULL, from a64 / b64 (int64 index lists).
+ * gn_rank_rows: q[i, 0:D] = x[a_i] .* y[b_i] (rows of x at stride ldx, of y at stride ldy), (a_i, b_i) taken as in
+ *   gn_rank_lookup.
+ * gn_rank_count: filtered rank of every entry of groups [0, n_groups) whose score rows are S[g] (lds >= n_cand;
+ *   q_rowptr and f_row point at the first group of the chunk); f_row[g] is the filter row of group g (from
+ *   gn_rank_lookup), f_row == NULL: no filter.  OGB rule: for an entry with target candidate t, with the negatives
+ *   N = {c != t : (a, b, c) not in the filter}, opt = #{c in N : S(c) > S(t)}, pess = #{c in N : S(c) >= S(t)},
+ *   rank[edge id] = 1 + (opt + pess) / 2 (float32).  S(t) is read from the same row as every S(c).
  * gn_rank_metrics: out (DEVICE double [1 + n_hits, n_rel]) = MRR = mean(1/rank) and Hits@k = mean(rank <= k) per
  *   relation over the edges rel_perm[rel_rowptr[r] : rel_rowptr[r+1]] (gn_index_prep of the edge types); NaN for a
  *   relation without edges.  hits_k is a HOST array of at most gn_rank_max_hits() entries (it travels in the
  *   kernel-parameter block: capturable).  Fixed-order float64 sums: repeated calls are bit-identical.
- * gn_rank_topk: the k (1 <= k <= 256) highest-scoring candidates c with (node[i], rel[i], c) not in the filter, for
- *   every query row i of S (overwritten: filtered entries are marked in place).  Order: descending pre-sigmoid
- *   score, ties by smaller id.  out_score / out_id [count, k]: score (sigmoid applied when `sigmoid`) and id; id -1
- *   and score NaN pad a query with fewer than k admissible candidates. */
-size_t gn_rank_csr_workspace_bytes(int64_t n_edges, int32_t n_nodes, int32_t n_rel);
-int gn_rank_csr(const int64_t* src, const int64_t* dst, const int64_t* etype, int64_t n_edges, int32_t n_nodes,
-                int32_t n_rel, int32_t* rowptr, int32_t* ent_dst, int32_t* ent_eid, int32_t* group_row /*or NULL*/,
-                int32_t* n_groups /*or NULL*/, void* ws, size_t ws_bytes, void* stream);
-int gn_rank_query_rows(const float* z, int64_t ldz, int32_t D, const float* w, int32_t n_rel, const int32_t* group_row,
-                       const int64_t* node, const int64_t* rel, int64_t count, float* q, int64_t ldq, void* stream);
-int gn_rank_count(const float* S, int64_t lds, int32_t n_nodes, const int32_t* group_row, int32_t n_groups,
-                  const int32_t* q_rowptr, const int32_t* q_dst, const int32_t* q_eid,
-                  const int32_t* f_rowptr /*or NULL*/, const int32_t* f_dst, float* rank, void* stream);
+ * gn_rank_topk: the k (1 <= k <= 256; k > n_cand is padded) highest-scoring candidates c of every query row i of S
+ *   (overwritten: filtered entries are marked in place), skipping the filter row f_row[i] (from gn_rank_lookup;
+ *   f_row == NULL: no filter).  Order: descending pre-sigmoid score, ties by smaller id.  out_score / out_id
+ *   [count, k]: score (sigmoid applied when `sigmoid`) and id; id -1 and score NaN pad a query with fewer than k
+ *   admissible candidates.
+ *
+ * gn_rank_csr: dense grouped structure of an edge list, the symmetrised filter view of pair queries (below) —
+ *   rowptr [n_nodes*n_rel + 1] (row s*n_rel + r), entries ent_dst / ent_eid [E] (candidate, edge id) sorted by
+ *   candidate inside a row (two stable counting sorts).  Requires n_nodes * n_rel < 2^31. */
+size_t gn_rank_group_workspace_bytes(int64_t n_edges);
+int gn_rank_group(const int64_t* a, const int64_t* b, const int64_t* c, int64_t n_edges, int32_t na, int32_t nb,
+                  int32_t nc, int32_t* rowptr, int32_t* group_a, int32_t* group_b, int32_t* ent_c, int32_t* ent_eid,
+                  int32_t* n_groups, void* ws, size_t ws_bytes, void* stream);
+int gn_rank_lookup(const int32_t* f_a, const int32_t* f_b, int32_t n_f, const int32_t* a32 /*or NULL*/,
+                   const int32_t* b32, const int64_t* a64, const int64_t* b64, int64_t count, int32_t* row,
+                   void* stream);
+int gn_rank_rows(const float* x, int64_t ldx, const float* y, int64_t ldy, int32_t D, const int32_t* a32 /*or NULL*/,
+                 const int32_t* b32, const int64_t* a64, const int64_t* b64, int64_t count, float* q, int64_t ldq,
+                 void* stream);
+int gn_rank_count(const float* S, int64_t lds, int32_t n_cand, int32_t n_groups, const int32_t* q_rowptr,
+                  const int32_t* q_c, const int32_t* q_eid, const int32_t* f_row /*or NULL*/, const int32_t* f_rowptr,
+                  const int32_t* f_c, float* rank, void* stream);
 int gn_rank_max_hits(void);
 int gn_rank_metrics(const float* rank, const int32_t* rel_rowptr, const int32_t* rel_perm, int32_t n_rel,
                     const int32_t* hits_k /*host*/, int32_t n_hits, double* out, void* stream);
-int gn_rank_topk(float* S, int64_t lds, int32_t n_nodes, int32_t n_rel, const int64_t* node, const int64_t* rel,
-                 int64_t count, const int32_t* f_rowptr /*or NULL*/, const int32_t* f_dst, int32_t k, int sigmoid,
-                 float* out_score, int64_t* out_id, void* stream);
-
-/* Relation queries (s, ?, t) of a directed pair: every relation r' in [0, n_rel) is a candidate, scored with the
- * PRE-sigmoid S(r') = sum_k z[s,k] z[t,k] w[r',k], one row of S = P . W^T with P[g] = z[s_g] .* z[t_g]
- * (gn_rank_pair_rows, then gn_sgemm / gn_tc_gemm with transB = 1; W the decoder weight [n_rel, D]).  P is bitwise
- * symmetric (fp32 products commute), so (s, t) and (t, s) give identical rows when both take the same product path.
- * Filter: the same set of directed known triples (s, r', t), duplicates counted once.  For a query triple (s, r, t):
- * N = {r' != r : (s, r', t) not in the filter}, opt = #{r' in N : S(r') > S(r)}, pess = #{r' in N : S(r') >= S(r)},
- * rank = 1 + (opt + pess) / 2, S(r) read from the same row as every S(r').  Metrics: gn_index_prep of the query
- * triples' relations, then gn_rank_metrics.
- *
- * gn_rank_pair_csr: pair-grouped structure of an edge list.  Three stable counting sorts (by rel, by dst, by src)
- *   order the entries by (src, dst, rel); rows are the distinct directed pairs in (src, dst) order, compacted (not
- *   s*n + t, which does not fit int32 for general n): rowptr [capacity n_edges + 1], pair_src / pair_dst [capacity
- *   n_edges], entries ent_rel / ent_eid [n_edges] (relation, edge id) sorted by relation inside a row; n_pairs
- *   (device int32) the row count.
- * gn_rank_pair_lookup: row[i] = the row of pair (s_i, t_i) in a pair-grouped filter of n_fpairs rows (binary search
- *   over its sorted pairs), or -1 when the filter holds no triple of that pair.  (s_i, t_i) from pair_src / pair_dst
- *   (int32, e.g. a query structure's pairs) or, when pair_src is NULL, from src / dst (int64).
- * gn_rank_pair_rows: p[i, 0:D] = z[s_i] .* z[t_i], (s_i, t_i) taken as in gn_rank_pair_lookup.
- * gn_rank_pair_count: filtered relation rank of every entry of pairs [0, n_pairs) whose score rows are S[g] (lds >=
- *   n_rel; q_rowptr and f_row point at the first pair of the chunk); f_row[g] is the filter row of pair g (from
- *   gn_rank_pair_lookup), f_row == NULL: no filter.  rank[edge id] as in gn_rank_count.
- * gn_rank_pair_topk: the k (1 <= k <= 256; k > n_rel is padded) highest-scoring relations r' with (s_i, r', t_i)
- *   not in the filter, for every row i of S (overwritten: filtered entries are marked in place); f_row[i] the
- *   filter row of query i, or f_row == NULL.  Order, padding and sigmoid as in gn_rank_topk. */
-size_t gn_rank_pair_csr_workspace_bytes(int64_t n_edges);
-int gn_rank_pair_csr(const int64_t* src, const int64_t* dst, const int64_t* etype, int64_t n_edges, int32_t n_nodes,
-                     int32_t n_rel, int32_t* rowptr, int32_t* pair_src, int32_t* pair_dst, int32_t* ent_rel,
-                     int32_t* ent_eid, int32_t* n_pairs, void* ws, size_t ws_bytes, void* stream);
-int gn_rank_pair_lookup(const int32_t* f_src, const int32_t* f_dst, int32_t n_fpairs,
-                        const int32_t* pair_src /*or NULL*/, const int32_t* pair_dst, const int64_t* src,
-                        const int64_t* dst, int64_t count, int32_t* row, void* stream);
-int gn_rank_pair_rows(const float* z, int64_t ldz, int32_t D, const int32_t* pair_src /*or NULL*/,
-                      const int32_t* pair_dst, const int64_t* src, const int64_t* dst, int64_t count, float* p,
-                      int64_t ldp, void* stream);
-int gn_rank_pair_count(const float* S, int64_t lds, int32_t n_rel, int32_t n_pairs, const int32_t* q_rowptr,
-                       const int32_t* q_rel, const int32_t* q_eid, const int32_t* f_row /*or NULL*/,
-                       const int32_t* f_rowptr, const int32_t* f_rel, float* rank, void* stream);
-int gn_rank_pair_topk(float* S, int64_t lds, int32_t n_rel, int64_t count, const int32_t* f_row /*or NULL*/,
-                      const int32_t* f_rowptr, const int32_t* f_rel, int32_t k, int sigmoid, float* out_score,
-                      int64_t* out_id, void* stream);
+int gn_rank_topk(float* S, int64_t lds, int32_t n_cand, int64_t count, const int32_t* f_row /*or NULL*/,
+                 const int32_t* f_rowptr, const int32_t* f_c, int32_t k, int sigmoid, float* out_score,
+                 int64_t* out_id, void* stream);
+size_t gn_rank_csr_workspace_bytes(int64_t n_edges);
+int gn_rank_csr(const int64_t* src, const int64_t* dst, const int64_t* etype, int64_t n_edges, int32_t n_nodes,
+                int32_t n_rel, int32_t* rowptr, int32_t* ent_dst, int32_t* ent_eid, void* ws, size_t ws_bytes,
+                void* stream);
 
 /* Top-k new pairs of a relation, queries (?, r, ?): the candidates are the UNORDERED pairs {s, t} with s < t (the
  * DistMult score is symmetric in s and t; a self-pair is not an interaction), scored with the PRE-sigmoid

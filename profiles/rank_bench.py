@@ -252,7 +252,7 @@ def run_relations(name, g, calls, dev):
     filt = gb.EdgeFilter([train, test], n, r)
     ranker = gb.RelationRanker(test[0], test[1], n, r, filter=filt)
     G, E = ranker.n_groups, test[0].size(1)
-    ps, pd = ranker._q.src[:G].long(), ranker._q.dst[:G].long()
+    ps, pd = ranker._q.a[:G].long(), ranker._q.b[:G].long()
     ref = TorchRelationRestatement(ps, pd, test, [train, test], n, r)
     rec = torch.empty((1 + len(HITS), r), dtype=torch.float64, device=dev)
 
@@ -354,7 +354,7 @@ def run(name, g, calls, dev):
     n, r = g["n_d"], g["n_rel"]
     filt = gb.EdgeFilter([train, test], n, r)
     ranker = gb.LinkRanker(test[0], test[1], n, r, filter=filt)
-    grp = ranker._q.group_row[: ranker.n_groups].long()
+    grp = ranker._q.a[: ranker.n_groups].long() * r + ranker._q.b[: ranker.n_groups].long()
     qn, qr = grp // r, grp % r
     ref = TorchRestatement(grp, test, [train, test], n, r)
     G, E = ranker.n_groups, test[0].size(1)

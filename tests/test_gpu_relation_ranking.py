@@ -200,8 +200,11 @@ def test_pose0_ranks_within_fp32_band(pose0):
     _check_shape(pose0, 4000, 0)
 
 
-def test_pose0_product_runs_on_tensor_cores(pose0):
+def test_pose0_ranks_run_on_tensor_cores_and_the_shared_count(pose0):
+    """One chunk of pair rows: one query-row launch, the product on gn_tc_gemm, one launch of the count kernel that
+    tail queries use too, and no filter lookup per call (each pair's filter row is found at construction)."""
     p = pose0
+    assert p["filt"] is p["ranker"].filter and p["ranker"].n_groups >= 4096
     p["ranker"].ranks(p["zt"], p["wt"])
     torch.cuda.synchronize()
     with torch.profiler.profile(activities=[torch.profiler.ProfilerActivity.CUDA]) as prof:
@@ -209,7 +212,9 @@ def test_pose0_product_runs_on_tensor_cores(pose0):
         torch.cuda.synchronize()
     names = [e.name for e in prof.events()]
     assert any("tc_gemm_kernel" in x for x in names), sorted(set(names))
-    assert any("rank_count_kernel" in x and "PairRows" in x for x in names), sorted(set(names))
+    assert sum("rank_rows_kernel" in x for x in names) == 1, sorted(set(names))
+    assert sum("rank_count_kernel" in x for x in names) == 1, sorted(set(names))
+    assert not any("rank_lookup_kernel" in x or "rank_rel_pairs" in x for x in names), sorted(set(names))
 
 
 def test_pose2_ranks_within_fp32_band(pose2):
