@@ -91,7 +91,7 @@ SIGNATURES = {
     "gn_pair_prep": (_INT, [_P, _P, _P, _I64, _I32, _I32, _P, _P, _P, _P, _SZ, _P]),
     "gn_distmult_bwd_pairs": (_INT, [_CSR, _P, _P, _P, _P, _I64, _I32, _P, _P, _P]),
     "gn_distmult_grads_workspace_bytes": (_SZ, [_I32, _I32, _I32]),
-    "gn_distmult_grads": (_INT, [_P, _P, _I32, _I32, _I32, _P, _I64, _P, _P, _I64, _P, _P, _SZ, _P]),
+    "gn_distmult_grads": (_INT, [_P, _P, _I32, _I32, _I32, _P, _I64, _P, _I64, _P, _I64, _P, _P, _SZ, _P]),
     "gn_softmax_fwd": (_INT, [_P, _I64, _I32, _P, _P]),
     "gn_softmax_bwd": (_INT, [_P, _P, _I64, _I32, _P, _P]),
     "gn_map2d": (_INT, [_INT, _P, _I64, _P, _I64, _I64, _I32, _P]),

@@ -196,9 +196,11 @@ __global__ void __launch_bounds__(256) pair_walk_kernel(const gn_csr csr, const 
       const int f = (v * LPE + fl) * VEC;
       if (f < D) {
         a0[v] = load_vec<VEC>(pa0 + f);
-        a1[v] = load_vec<VEC>(pa1 + f);
+        a1[v] = load_vec<VEC>(pa1 + f);      // (row 0 when the slot has no 2nd entry: read, not added)
       }
     }
+    // a slot without a 2nd entry adds nothing: predicated on position, not on a zero coefficient (0 * z[0] would
+    // carry a non-finite value of row 0 into this row)
 #pragma unroll
     for (int v = 0; v < NV; ++v) {
       const int f = (v * LPE + fl) * VEC;
@@ -206,7 +208,7 @@ __global__ void __launch_bounds__(256) pair_walk_kernel(const gn_csr csr, const 
 #pragma unroll
         for (int i = 0; i < VEC; ++i) {
           acc[v].v[i] = fmaf(g0, a0[v].v[i], acc[v].v[i]);
-          acc[v].v[i] = fmaf(g1, a1[v].v[i], acc[v].v[i]);     // g1 == 0 when the slot has no 2nd entry
+          if (has1) acc[v].v[i] = fmaf(g1, a1[v].v[i], acc[v].v[i]);
         }
       }
     }
@@ -245,15 +247,17 @@ __global__ void __launch_bounds__(256, 4) pair_walk_batch_kernel(const gn_csr cs
     for (int i = 0; i < 4; ++i) acc[v].v[i] = 0.f;
   for (int base = ci.beg; base < ci.end; base += 32) {
     const int mine = base + lane;
-    int o = 0;            // entries past the end of the chunk: row 0 with coefficient 0
+    int o = 0;
     float g = 0.f;
     if (mine < ci.end) {
       o = __ldg(ent_other + mine);
       g = __ldg(coef + __ldg(ent_eid + mine));
     }
-    const int steps = min(8, (ci.end - base + 3) >> 2);
-#pragma unroll 2
-    for (int t = 0; t < steps; ++t) {
+    // slot `slot` of step t takes entry base + 4t + slot.  The whole steps add every slot; the one partial step at a
+    // chunk's end (fewer than 4 entries left) adds only its live slots: predicated on position, not 0 * z[0]
+    const int rem = ci.end - base;
+    const int full = min(8, rem >> 2);
+    auto step = [&](int t, bool live) {
       const int from = t * 4 + slot;
       const int oo = __shfl_sync(kFull, o, from);
       const float gg = __shfl_sync(kFull, g, from);
@@ -261,14 +265,18 @@ __global__ void __launch_bounds__(256, 4) pair_walk_batch_kernel(const gn_csr cs
 #pragma unroll
       for (int v = 0; v < NV; ++v) {
         if (ok[v]) {
-          const float4 a = __ldg(za + v * 8);
+          float4 a = __ldg(za + v * 8);
+          if (!live) a = make_float4(0.f, 0.f, 0.f, 0.f);
           acc[v].v[0] = fmaf(gg, a.x, acc[v].v[0]);
           acc[v].v[1] = fmaf(gg, a.y, acc[v].v[1]);
           acc[v].v[2] = fmaf(gg, a.z, acc[v].v[2]);
           acc[v].v[3] = fmaf(gg, a.w, acc[v].v[3]);
         }
       }
-    }
+    };
+#pragma unroll 2
+    for (int t = 0; t < full; ++t) step(t, true);
+    if (full < 8 && (rem & 3)) step(full, slot < (rem & 3));
   }
 #pragma unroll
   for (int v = 0; v < NV; ++v) reduce_slots<8, 4>(acc[v]);
@@ -288,6 +296,15 @@ __global__ void __launch_bounds__(256, 4) pair_walk_batch_kernel(const gn_csr cs
 constexpr int kGradThreads = 1024;
 constexpr int kGradSlabNodes = 96;     // nodes per dw slab: 8 rounds of 12 groups at D = 80
 
+// acc + t * x, where a T element that is exactly 0 — a (node, relation) row no edge references — adds nothing (a
+// select, not 0 * x): a non-finite z row of an unreferenced node or w row of an unused relation then stays out of every
+// other row's sum, as in the autograd of the reference expression.  With finite factors this is plain fmaf.
+// (`x` is pinned first, so the select cannot turn the load of x into one that waits for t.)
+__device__ __forceinline__ float fma_t(float t, float x, float acc) {
+  asm volatile("" : "+f"(x));
+  return t != 0.f ? fmaf(t, x, acc) : acc;
+}
+
 __device__ __forceinline__ float grads_reduce_groups(float acc, int g, int G, int f, int D, float* red) {
   if (g < G && f < D) red[g * D + f] = acc;
   __syncthreads();
@@ -304,7 +321,7 @@ __global__ void __launch_bounds__(kGradThreads) distmult_grads_kernel(const floa
                                                                      const float* __restrict__ T2, int n_nodes,
                                                                      int n_rel, int D, const float* __restrict__ z,
                                                                      int64_t ldz, const float* __restrict__ w,
-                                                                     float* __restrict__ dz, int64_t lddz,
+                                                                     int64_t ldw, float* __restrict__ dz, int64_t lddz,
                                                                      float* __restrict__ dw, int n_slabs,
                                                                      float* __restrict__ slab_part,
                                                                      unsigned int* __restrict__ slab_count) {
@@ -330,11 +347,11 @@ __global__ void __launch_bounds__(kGradThreads) distmult_grads_kernel(const floa
             const int64_t t = (int64_t(row) * n_rel + i) * D + f;
             tv[u] = __ldg(T + t);
             if (T2) tv[u] += __ldg(T2 + t);
-            ov[u] = __ldg(w + int64_t(i) * D + f);
+            ov[u] = __ldg(w + int64_t(i) * ldw + f);
           }
         }
 #pragma unroll
-        for (int u = 0; u < kU; ++u) acc = fmaf(tv[u], ov[u], acc);
+        for (int u = 0; u < kU; ++u) acc = fma_t(tv[u], ov[u], acc);
       }
     }
     const float s = grads_reduce_groups(acc, g, G, f, D, red);
@@ -361,12 +378,12 @@ __global__ void __launch_bounds__(kGradThreads) distmult_grads_kernel(const floa
         }
       }
 #pragma unroll
-      for (int u = 0; u < kU; ++u) acc = fmaf(tv[u], ov[u], acc);
+      for (int u = 0; u < kU; ++u) acc = fma_t(tv[u], ov[u], acc);
     }
   }
   const float s = grads_reduce_groups(acc, g, G, f, D, red);
   if (n_slabs == 1) {
-    if (g == 0) dw[int64_t(rel) * D + f] = 0.5f * s;
+    if (g == 0) dw[int64_t(rel) * ldw + f] = 0.5f * s;
     return;
   }
   if (g == 0) slab_part[(int64_t(rel) * n_slabs + slab) * D + f] = s;
@@ -388,7 +405,7 @@ __global__ void __launch_bounds__(kGradThreads) distmult_grads_kernel(const floa
       for (int u = 0; u < 8; ++u) t += v[u];
     }
     for (; k < n_slabs; ++k) t += __ldcg(p + int64_t(k) * D);
-    dw[int64_t(rel) * D + f] = 0.5f * t;
+    dw[int64_t(rel) * ldw + f] = 0.5f * t;
   }
   if (threadIdx.x == 0) slab_count[rel] = 0;
 }
@@ -403,8 +420,9 @@ constexpr int kVSub = 16;
 constexpr int kVSlab = 128;
 constexpr int kVU = 4;
 
-__device__ __forceinline__ void f4_fma(float4& a, const float4& x, const float4& y) {
-  a.x = fmaf(x.x, y.x, a.x); a.y = fmaf(x.y, y.y, a.y); a.z = fmaf(x.z, y.z, a.z); a.w = fmaf(x.w, y.w, a.w);
+// a += t .* x, a zero element of t adding nothing (fma_t)
+__device__ __forceinline__ void f4_fma_t(float4& a, const float4& t, const float4& x) {
+  a.x = fma_t(t.x, x.x, a.x); a.y = fma_t(t.y, x.y, a.y); a.z = fma_t(t.z, x.z, a.z); a.w = fma_t(t.w, x.w, a.w);
 }
 __device__ __forceinline__ float4 f4_add(const float4& x, const float4& y) {
   return make_float4(x.x + y.x, x.y + y.y, x.z + y.z, x.w + y.w);
@@ -446,7 +464,7 @@ __global__ void __launch_bounds__(512) distmult_grads_vec_kernel(const float* __
           }
         }
 #pragma unroll
-        for (int u = 0; u < kVU; ++u) f4_fma(acc, tv[u], wv[u]);
+        for (int u = 0; u < kVU; ++u) f4_fma_t(acc, tv[u], wv[u]);
       }
     }
     if (GR > 1) {
@@ -477,7 +495,7 @@ __global__ void __launch_bounds__(512) distmult_grads_vec_kernel(const float* __
       }
     }
 #pragma unroll
-    for (int u = 0; u < kVU; ++u) f4_fma(acc, tv[u], zv[u]);
+    for (int u = 0; u < kVU; ++u) f4_fma_t(acc, tv[u], zv[u]);
   }
   red4[sub * C4 + c4] = acc;
   __syncthreads();
@@ -755,8 +773,8 @@ int gn_distmult_bwd_pairs(const gn_csr* pair_csr, const int32_t* ent_other, cons
 }
 
 static bool grads_vec_ok(int D, const float* T, const float* T2, const float* z, int64_t ldz, const float* w,
-                         const float* dz, int64_t lddz, const float* dw) {
-  return D % 4 == 0 && D <= 128 && ldz % 4 == 0 && lddz % 4 == 0 && aligned16(T) && (!T2 || aligned16(T2)) &&
+                         int64_t ldw, const float* dz, int64_t lddz, const float* dw) {
+  return D % 4 == 0 && D <= 128 && ldz % 4 == 0 && ldw == D && lddz % 4 == 0 && aligned16(T) && (!T2 || aligned16(T2)) &&
          aligned16(z) && aligned16(w) && (!dz || aligned16(dz)) && (!dw || aligned16(dw));
 }
 
@@ -766,11 +784,12 @@ size_t gn_distmult_grads_workspace_bytes(int32_t n_nodes, int32_t n_rel, int32_t
 }
 
 int gn_distmult_grads(const float* T, const float* T2, int32_t n_nodes, int32_t n_rel, int32_t D, const float* z,
-                      int64_t ldz, const float* w, float* dz, int64_t lddz, float* dw, void* ws, size_t ws_bytes,
-                      void* stream) {
-  if (n_nodes <= 0 || n_rel <= 0 || D <= 0 || D > kGradThreads || !T || !z || !w || (!dz && !dw)) return GN_ERR_ARG;
+                      int64_t ldz, const float* w, int64_t ldw, float* dz, int64_t lddz, float* dw, void* ws,
+                      size_t ws_bytes, void* stream) {
+  if (n_nodes <= 0 || n_rel <= 0 || D <= 0 || D > kGradThreads || ldw < D || !T || !z || !w || (!dz && !dw))
+    return GN_ERR_ARG;
   cudaStream_t st = as_stream(stream);
-  const bool vec = grads_vec_ok(D, T, T2, z, ldz, w, dz, lddz, dw);
+  const bool vec = grads_vec_ok(D, T, T2, z, ldz, w, ldw, dz, lddz, dw);
   const int n_slabs = int(ceil_div(n_nodes, vec ? kVSlab : kGradSlabNodes));
   unsigned int* count = nullptr;
   float* part = nullptr;
@@ -792,8 +811,8 @@ int gn_distmult_grads(const float* T, const float* T2, int32_t n_nodes, int32_t 
   const int G = kGradThreads / D;
   const size_t smem = size_t(G) * size_t(D) * sizeof(float);
   const int64_t blocks = int64_t(dw ? n_rel * n_slabs : 0) + (dz ? n_nodes : 0);
-  GN_LAUNCH(distmult_grads_kernel, (unsigned)blocks, kGradThreads, smem, st, T, T2, n_nodes, n_rel, D, z, ldz, w, dz,
-            lddz, dw, n_slabs, part, count);
+  GN_LAUNCH(distmult_grads_kernel, (unsigned)blocks, kGradThreads, smem, st, T, T2, n_nodes, n_rel, D, z, ldz, w, ldw,
+            dz, lddz, dw, n_slabs, part, count);
   return GN_OK;
 }
 

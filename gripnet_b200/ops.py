@@ -713,15 +713,35 @@ def _pair_walk(ps, coef, z):
     return t
 
 
-def _distmult_grads(t, t2, z, w, need_z, need_w):
-    n, d, r = z.size(0), z.size(1), w.size(0)
-    dz = torch.empty((n, d), dtype=torch.float32, device=z.device) if need_z else None
+def _col_blocks(z):
+    """Column ranges ``[c0, c1)`` of z that the backward kernels take in one pass each.
+
+    The walk takes rows of up to 1024 floats when they are float4 rows (width and row stride multiples of 4, 16-byte
+    aligned), 256 otherwise.  The backward is separable over feature columns (``T[:, :, f]``, ``dz[:, f]`` and
+    ``dw[:, f]`` depend on column f alone), so a wider row is handled in blocks of that width; every width up to it is
+    one block."""
+    d = z.size(1)
+    step = 1024 if (d % 4 == 0 and _ldz(z) % 4 == 0 and z.data_ptr() % 16 == 0) else 256
+    return [(c0, min(c0 + step, d)) for c0 in range(0, d, step)]
+
+
+def _distmult_grads(t, t2, z, w, dz, dw, c0=0):
+    """Columns ``[c0, c0 + t.size(1))`` of dz / dw (either may be None) from the walk(s) of those columns of z."""
+    if dz is None and dw is None:
+        return
+    n, d, r, full = z.size(0), t.size(1), w.size(0), w.size(1)      # w, dz, dw: contiguous, `full` columns
+    lib = _lib.load()
+    ws = _ws(lib.gn_distmult_grads_workspace_bytes(n, r, d), z.device)
+    off = 4 * c0
+    _lib.check(lib.gn_distmult_grads(t.data_ptr(), _ptr(t2), n, r, d, z.data_ptr() + off, _ldz(z), w.data_ptr() + off,
+                                     full, _ptr(dz) + off if dz is not None else None, full,
+                                     _ptr(dw) + off if dw is not None else None, _ptr(ws), ws.numel(), _stream()),
+               "gn_distmult_grads")
+
+
+def _grad_buffers(z, w, need_z, need_w):
+    dz = torch.empty((z.size(0), z.size(1)), dtype=torch.float32, device=z.device) if need_z else None
     dw = torch.empty_like(w) if need_w else None
-    if need_z or need_w:
-        lib = _lib.load()
-        ws = _ws(lib.gn_distmult_grads_workspace_bytes(n, r, d), z.device)
-        _lib.check(lib.gn_distmult_grads(t.data_ptr(), _ptr(t2), n, r, d, z.data_ptr(), _ldz(z), w.data_ptr(),
-                                         _ptr(dz), d, _ptr(dw), _ptr(ws), ws.numel(), _stream()), "gn_distmult_grads")
     return dz, dw
 
 
@@ -759,8 +779,10 @@ class DistMult(torch.autograd.Function):
         _check_versions(ctx.key_tensors, ctx.key_versions, "edge_index / edge_type")
         coef = _distmult_coef(grad.contiguous(), out, ctx.sigmoid)
         ps = pair_struct(ctx.key_tensors[0], ctx.key_tensors[1], z.size(0), w.size(0))
-        t = _pair_walk(ps, coef, z)
-        dz, dw = _distmult_grads(t, None, z, w, ctx.needs_input_grad[0], ctx.needs_input_grad[1])
+        dz, dw = _grad_buffers(z, w, ctx.needs_input_grad[0], ctx.needs_input_grad[1])
+        for c0, c1 in _col_blocks(z):
+            t = _pair_walk(ps, coef, z[:, c0:c1])
+            _distmult_grads(t, None, z, w, dz, dw, c0)
         return dz, dw, None, None, None
 
 
@@ -832,13 +854,19 @@ class DistMultPair(torch.autograd.Function):
         # one structure serves both lists when they are the same tensor: its arrival counters cannot be
         # shared by two concurrent walks, so that case runs on one stream
         br = streams.Branch(enabled=ps_p is not ps_n)
-        with br(g_neg, neg, z):
-            coef_n = _distmult_coef(g_neg, neg, ctx.sigmoid)
-            t_n = _pair_walk(ps_n, coef_n, z)
-        coef_p = _distmult_coef(g_pos, pos, ctx.sigmoid)
-        t_p = _pair_walk(ps_p, coef_p, z)
-        br.join()
-        dz, dw = _distmult_grads(t_p, t_n, z, w, ctx.needs_input_grad[0], ctx.needs_input_grad[1])
+        dz, dw = _grad_buffers(z, w, ctx.needs_input_grad[0], ctx.needs_input_grad[1])
+        coef_n = coef_p = None
+        for c0, c1 in _col_blocks(z):
+            zb = z[:, c0:c1]
+            with br(g_neg, neg, zb):
+                if coef_n is None:
+                    coef_n = _distmult_coef(g_neg, neg, ctx.sigmoid)
+                t_n = _pair_walk(ps_n, coef_n, zb)
+            if coef_p is None:
+                coef_p = _distmult_coef(g_pos, pos, ctx.sigmoid)
+            t_p = _pair_walk(ps_p, coef_p, zb)
+            br.join()
+            _distmult_grads(t_p, t_n, z, w, dz, dw, c0)
         if dw is not None and r != r_full:                    # relations outside this rank's slice: zero rows
             dw_full = torch.empty((r_full, w.size(1)), dtype=torch.float32, device=w.device)
             _lib.check(_lib.load().gn_zero(dw_full.data_ptr(), dw_full.numel() * 4, _stream()), "gn_zero")

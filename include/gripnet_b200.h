@@ -260,9 +260,12 @@ int gn_distmult_coef(const float* grad_out, const float* out, int64_t n_edges, i
  * and gn_distmult_grads finishes both gradients from T (plus an optional second T2 of another edge list,
  * e.g. the negatives of the same step) without touching the edges again:
  *   dz[n] = sum_r T[n,r] .* w[r],      dw[r] = 1/2 sum_n z[n] .* T[n,r]
- * (every edge sits in the pair rows of both of its endpoints, hence the 1/2; D <= 1024; `ws` holds
- * gn_distmult_grads_workspace_bytes: per-relation slab partials of dw + arrival counters).  Replaces the autograd of
- * gripnet/decoder.py:19-23 (three index_put scatters); atomic-free, fixed summation order. */
+ * (every edge sits in the pair rows of both of its endpoints, hence the 1/2; D <= 1024; rows of z, w / dw and dz are
+ * ldz, ldw and lddz floats apart; `ws` holds gn_distmult_grads_workspace_bytes: per-relation slab partials of dw +
+ * arrival counters).  A zero element of T adds nothing (no 0 * Inf from rows no edge references).  The walk takes
+ * D <= 256, or D <= 1024 for float4 rows (D, ldz multiples of 4, z 16-byte aligned).  Both gradients are separable
+ * over feature columns, so wider rows are handled in column blocks.  Replaces the autograd of gripnet/decoder.py:19-23
+ * (three index_put scatters); atomic-free, fixed summation order. */
 size_t gn_pair_prep_workspace_bytes(int64_t n_edges);
 int gn_pair_prep(const int64_t* src, const int64_t* dst, const int64_t* etype, int64_t n_edges, int32_t n_nodes,
                  int32_t n_rel, int32_t* pair_rowptr, int32_t* ent_other, int32_t* ent_eid /*[2E]*/,
@@ -272,7 +275,7 @@ int gn_distmult_bwd_pairs(const gn_csr* pair_csr, const int32_t* ent_other, cons
                           void* stream);
 size_t gn_distmult_grads_workspace_bytes(int32_t n_nodes, int32_t n_rel, int32_t D);
 int gn_distmult_grads(const float* T, const float* T2 /*or NULL*/, int32_t n_nodes, int32_t n_rel, int32_t D,
-                      const float* z, int64_t ldz, const float* w, float* dz /*or NULL*/, int64_t lddz,
+                      const float* z, int64_t ldz, const float* w, int64_t ldw, float* dz /*or NULL*/, int64_t lddz,
                       float* dw /*or NULL*/, void* ws, size_t ws_bytes, void* stream);
 
 /* ---- K11: multi-class decoder pieces  ------------------------------------ */
