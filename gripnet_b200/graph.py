@@ -8,6 +8,7 @@ All arrays live in HBM as int32 / fp32 tensors owned by these objects.
 """
 import ctypes as C
 import os
+import weakref
 from collections import OrderedDict
 
 import torch
@@ -554,7 +555,8 @@ def _capturing():
 # score[i*C + label[i]]  directly: an out-of-range id would be a silent out-of-bounds device read where
 # the reference raises IndexError).  One host check (min / max) per (tensor identity, version, bound),
 # remembered in an LRU; skipped while a CUDA graph is being captured (the eager warm-up iterations that
-# precede every capture have validated the same buffers).
+# precede every capture have validated the same buffers).  An entry lives only as long as the tensor it was
+# made for: a later tensor placed in the recycled storage with the same shape would have the same key.
 # --------------------------------------------------------------------------
 _validated = OrderedDict()
 _VALIDATED_CAPACITY = 256
@@ -564,7 +566,9 @@ def mark_valid(t, hi):
     """Record that every entry of ``t`` lies in ``[0, hi)`` (producers that guarantee it by construction,
     e.g. the device negative sampler, call this instead of paying the host check)."""
     key = (_Cache.tkey(t), int(hi))
-    _validated[key] = True
+    ref = _validated.get(key)
+    if ref is None or ref() is not t:
+        _validated[key] = weakref.ref(t, lambda r, k=key: _validated.pop(k) if _validated.get(k) is r else None)
     _validated.move_to_end(key)
     while len(_validated) > _VALIDATED_CAPACITY:
         _validated.popitem(last=False)
@@ -575,7 +579,8 @@ def validate_index(t, hi, name):
     if t is None or t.numel() == 0:
         return
     key = (_Cache.tkey(t), int(hi))
-    if key in _validated:
+    ref = _validated.get(key)
+    if ref is not None and ref() is not None:
         _validated.move_to_end(key)
         return
     if _capturing():

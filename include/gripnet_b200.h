@@ -177,7 +177,8 @@ int gn_index_prep(const int64_t* index, int64_t n, int32_t n_nodes,
  * addend) and the ReLU at :279/:305/:370.  Backward passes call it with the
  * transpose CSR.  Warp per chunk, 128-bit gathers, no atomics on data: rows split
  * over several chunks are combined in a fixed order by the last-arriving warp.
- * partial: [n_chunks, F] fp32 scratch (may be NULL when no row has > 1 chunk). */
+ * partial: fp32 scratch of 2 * (n_chunks - n_rows) rows of min(F, 128) floats (a row split over k
+ * chunks owns rows [2 * (first_chunk - row), +k)); may be NULL when no row has more than one chunk. */
 int gn_spmm(const gn_csr* csr, const float* x, int64_t ldx, int32_t F,
             const float* row_scale, const float* bias, const float* addend, int64_t ld_addend,
             int relu, float* out, int64_t ldo, float* partial, void* stream);
@@ -187,7 +188,9 @@ int gn_spmm(const gn_csr* csr, const float* x, int64_t ldx, int32_t F,
  *   op(A) is M x K (transA: stored K x M), op(B) is K x N (transB: stored N x K);
  *   batch_reduce != 0: a single C = sum_b op(A[b]) op(B[b]);
  *   a_rows != NULL: row r of the STORED A is fetched from A + a_rows[r]*lda (row gather);
- *   epilogue: (+ C if accumulate) (+ addend) then zero where relu_mask <= 0.
+ *   epilogue: (+ C if accumulate) (+ addend) then zero where relu_mask <= 0 (or NaN);
+ *   addend and relu_mask are [M, N] and NOT offset by the batch entry: every C[b] adds the same
+ *   addend and uses the same mask.
  *   split_k != 0: when the output tiles alone cannot fill the GPU, the flattened
  *   (batch-to-reduce, K) reduction is cut into slices whose partial products are
  *   summed in slice order from `ws` (deterministic, no atomics); `ws` must hold
